@@ -2,6 +2,7 @@
 """Benchmark of the MSDeformAttn hot path (BASELINE.json config 2) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dist init|trained|adversarial]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward + one backward of the op on one batch of synthetic input:
@@ -13,6 +14,9 @@ is weak and `value` = images all ranks processed / max-over-ranks device time.
 Output: ONE JSON line on rank 0 (see DESIGN.md "Measurement" for every key).
 `--impl reference` times the reference's own implementation (HF `multi_scale_deformable_attention`,
 M2F:798-837, fp32, autograd backward) on the host CPU with all threads, on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step computed (the op's output and the three input gradients) as
+DIR/<name>.npy in float32 (rank 0's batch; a fixed seeded sample of an array larger than DUMP_SAMPLE elements); the
+inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +37,8 @@ B_PER_GPU = 8
 H, D, L, P = 8, 32, 3, 4
 METRIC = "msda_fwd_bwd_throughput"
 UNIT = "images/s"
+OUTPUT_NAMES = ("output", "grad_value", "grad_sampling_locations", "grad_attention_weights")
+DUMP_SAMPLE = 1 << 21  # elements kept of a larger output: four float32 arrays of 8 MB, 32 MB in all
 
 
 def parse_args():
@@ -47,7 +53,25 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the other location distributions and fp32")
     ap.add_argument("--no-train", action="store_true", help="skip the `train` block (config 3 DDP fine-tune step)")
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip timing the reference function on the GPU")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+def dump_outputs(directory, tensors):
+    """Save each tensor as ``directory/<name>.npy`` in float32: whole when it has at most DUMP_SAMPLE elements, else
+    the same DUMP_SAMPLE elements of its flattened form on every run (seeded, ascending indices)."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in tensors.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(directory, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def algorithmic_bytes(B, S, dtype):
@@ -159,7 +183,7 @@ def reference_step_fn(n_images, q_fraction=1.0):
         v.grad = lo.grad = a.grad = None
         out = hf_forward_torch(v, SHAPES_C2, lo, a)
         out.backward(go)
-        return out
+        return out, v.grad, lo.grad, a.grad
 
     return step, nq
 
@@ -172,21 +196,16 @@ def run_reference(args, rank, world):
     torch.set_num_threads(cores)
     # one image (B=1 of the B=8 batch) with ALL its queries per step: the same per-image work as the b200 arm, fp32
     step, nq = reference_step_fn(1)
-    step()  # cold call (imports, allocator) -- never timed, never used for sizing
-    t0 = time.perf_counter()
-    step()
-    t1 = time.perf_counter() - t0
+    step()  # cold call (imports, allocator) -- never timed
     warmup, steps = args.warmup, args.steps
-    budget = 170.0  # keep the whole run within a few minutes: fewer steps, never fewer queries
-    if (warmup + steps) * t1 > budget:
-        warmup = min(warmup, 2)
-        steps = max(3, int((budget - warmup * t1) / t1))
     for _ in range(warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
-    dt = (time.perf_counter() - t0) / max(steps, 1)
+        res = step()
+    dt = (time.perf_counter() - t0) / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, res)))
     S = sum(h * w for h, w in SHAPES_C2)
     value = 1.0 / dt
     sample = (f"{steps} steps of 1 image each (B=1 of the B=8 batch, all {nq} of {S} queries), reference HF function "
@@ -442,6 +461,8 @@ def run_b200(args, rank, world, local_rank):
     launches = _cabi.launch_count() // max(args.steps + args.warmup, 1)
     ms_step = secs / args.steps * 1e3
     value = world * B_PER_GPU * args.steps / secs
+    if args.dump_outputs and rank == 0:  # before anything else reuses the problem's buffers
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, (prob.out, prob.gv, prob.gl, prob.ga))))
 
     # per-kernel times (library-recorded events), fwd-only and bwd-only call times
     kern = profile_kernels(prob, min(args.steps, 20))
