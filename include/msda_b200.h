@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define MSDA_B200_ABI_VERSION 11
+#define MSDA_B200_ABI_VERSION 12
 #define MSDA_B200_MAX_LEVELS 8
 
 /* dtype codes */
@@ -68,7 +68,6 @@ extern "C" {
                                          /* instead of the pixel-sorted kernel (v2, D=32 & P=4)  */
 #define MSDA_B200_FLAG_BWD_V2 32u        /* backward: force the CUDA-core pixel-sorted kernel (v2) instead of the  */
                                          /* group-sorted tensor-core kernel (v3, bf16 values, D=32 & P=4)          */
-#define MSDA_B200_FLAG_NO_WINDOW 8u      /* never use the window-staged (TMA) kernels of msda_win.cu */
 #define MSDA_B200_FLAG_STRICT_PADDING 16u /* forward: skip the FMA of every zero-weight corner, so a non-finite  */
                                          /* value in a pixel grid_sample's zeros padding never reads (M2F:823)  */
                                          /* cannot become 0 * Inf = NaN; 25-30 % slower (the backward kernels    */
@@ -88,17 +87,6 @@ typedef struct msda_b200_desc {
   uint32_t flags;      /* MSDA_B200_FLAG_*                                                       */
   const int32_t* spatial_shapes_hw;  /* host, L x 2 = (H_l, W_l); M2F:1312 spatial_shapes_list   */
   const int64_t* level_start_index;  /* host, L; M2F:1321                                        */
-  /* Optional tile schedule for `query_order` (scheduling only; results never depend on it).  With a schedule,
-   * tile t owns query_order[tile_start[t] .. tile_start[t+1]) -- queries whose sampling locations fall into the
-   * same small pixel windows (functional.pyramid_schedule: a tile_rows x tile_cols patch of the finest level plus
-   * the coarser-level queries whose reference point lies inside it).  Geometries the window-staged kernels
-   * (csrc/msda_win.cu: bf16, D = 32, P = 4, L <= 4) cover are then run by them; without a schedule
-   * (tile_start = NULL) thread blocks take fixed runs of query_order.                                         */
-  const int32_t* tile_start;  /* dev, num_tiles + 1 int32, or NULL                                       */
-  int32_t num_tiles;          /* tiles per batch element                                                 */
-  int32_t max_tile;           /* largest tile (queries); at most 192 for the window kernels              */
-  int32_t tile_rows;          /* patch of the finest level a tile was built from (0 = 8)                 */
-  int32_t tile_cols;          /* (0 = 16)                                                                */
 } msda_b200_desc;
 
 /* ABI version of the loaded library (== MSDA_B200_ABI_VERSION it was built with). */

@@ -36,12 +36,17 @@ def test_abi_version_and_error_string(lib):
     assert lib.msda_b200_last_error() is not None
 
 
-def test_desc_layout_matches_header():
+def test_desc_layout_matches_header_without_tile_schedule():
     from weed_instance_segmentation_b200 import _cabi
-    # 10 x int32, two host pointers, the tile-schedule pointer, 4 x int32: 40 + 16 + 8 + 16 bytes on LP64
-    assert ctypes.sizeof(_cabi.Desc) == 10 * 4 + 3 * ctypes.sizeof(ctypes.c_void_p) + 4 * 4
+    text = open(os.path.join(ROOT, "include", "msda_b200.h")).read()
+    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+    body = re.search(r"typedef struct msda_b200_desc \{(.*?)\} msda_b200_desc;", text, flags=re.S).group(1)
+    members = re.findall(r"(\w+)\s*;", body)
+    assert [name for name, _ in _cabi.Desc._fields_] == members
+    # 10 x int32, two host pointers: 40 + 16 bytes on LP64
+    assert ctypes.sizeof(_cabi.Desc) == 10 * 4 + 2 * ctypes.sizeof(ctypes.c_void_p)
     assert _cabi.Desc.spatial_shapes_hw.offset == 40
-    assert _cabi.Desc.tile_start.offset == 56 and _cabi.Desc.num_tiles.offset == 64 and _cabi.Desc.tile_cols.offset == 76
+    assert _cabi.Desc.level_start_index.offset == 48
 
 
 def test_validation_without_gpu(lib):

@@ -277,30 +277,53 @@ def test_nan_and_far_locations_are_safe(wis):
     _assert_close(got, want, FP32_BAR, "nan")
 
 
-WINDOW_CASES = [
-    ("c1_pyramid", 2, [(16, 16), (32, 32), (64, 64)]),
-    ("c3_odd", 1, [(31, 41), (61, 81), (121, 162)]),
-    ("two_levels", 2, [(5, 7), (9, 4)]),
-    ("one_pixel_levels", 2, [(1, 1), (1, 9), (7, 1), (4, 4)]),
+# bf16 values, D = 32, even H: the head-pair forward. L = 3, P = 4 takes its constant-index descriptor path; the odd
+# two-level geometry with three points per level takes the generic one.
+PAIR_CASES = [
+    ("c1_pyramid", 2, [(16, 16), (32, 32), (64, 64)], 8, 4),
+    ("odd_two_levels", 2, [(8, 9), (10, 6)], 2, 3),
 ]
 
 
-@pytest.mark.parametrize("kernel", ["0", "1"], ids=["cuda_core", "tensor_core"])
-@pytest.mark.parametrize("dist", ["init", "trained", "adversarial"])
-@pytest.mark.parametrize("case", WINDOW_CASES, ids=[c[0] for c in WINDOW_CASES])
-def test_window_staged_forward(wis, case, dist, kernel, monkeypatch):
-    """The opt-in window-staged forward kernels (csrc/msda_win.cu: TMA box loads into shared memory, gather from there,
-    on CUDA cores or through ldmatrix + mma.sync) against the oracle -- including samples that fall outside the
-    staged window (adversarial) and levels smaller than the window."""
-    from weed_instance_segmentation_b200.synth import msda_inputs
-    monkeypatch.setenv("MSDA_B200_WINDOW", "1")
-    monkeypatch.setenv("MSDA_B200_WIN_KERNEL", kernel)
-    tag, B, shapes = case
-    x = msda_inputs(B, shapes, dist=dist, seed=31, value_dtype=torch.bfloat16)
-    out = wis.ms_deform_attn(x["value"].cuda(), shapes, None, x["sampling_locations"].cuda(), x["attention_weights"].cuda())
-    want = oracle.c_forward(x["value"].float().numpy(), shapes, x["sampling_locations"].numpy(),
-                            x["attention_weights"].float().numpy(), dtype=np.float64)
-    assert rel_err(out.float().cpu().numpy(), want) <= BF16_BAR, f"{tag}/{dist}"
+@pytest.mark.parametrize("attn_dtype", [torch.bfloat16, torch.float32], ids=["attn_bf16", "attn_f32"])
+@pytest.mark.parametrize("case", PAIR_CASES, ids=[c[0] for c in PAIR_CASES])
+def test_head_pair_forward_matches_one_head_kernel(wis, case, attn_dtype):
+    """The head-pair forward (msda_fwd_pair_kernel) against the one-head kernel, which MSDA_B200_FLAG_STRICT_PADDING
+    routes the same problem to: plain, fused, and fused with implicit reference points (ref_points = NULL). With finite
+    inputs the results are bit-identical: strict mode only skips FMAs whose weight is exactly 0, which add +-0."""
+    from weed_instance_segmentation_b200 import _cabi, functional, synth
+    tag, B, shapes, H, P = case
+    D, L = 32, len(shapes)
+    lib = _cabi.load()
+    acode = _cabi.BF16 if attn_dtype == torch.bfloat16 else _cabi.F32
+    order = functional.query_order_2d(shapes, functional._TILE, "cuda")
+    ref = synth.reference_points(shapes, device="cuda")[None].expand(B, -1, -1, -1).contiguous()
+    stream = torch.cuda.current_stream().cuda_stream
+    for dist in ("init", "adversarial"):
+        x = synth.msda_inputs(B, shapes, num_heads=H, head_dim=D, num_points=P, dist=dist, seed=5, device="cuda",
+                              value_dtype=torch.bfloat16, attn_dtype=attn_dtype, with_grad_out=False)
+        value, loc, attn = x["value"], x["sampling_locations"], x["attention_weights"]
+        S = value.shape[1]
+        g = torch.Generator(device="cuda").manual_seed(1)
+        off = (synth.init_offsets(H, L, P).to("cuda")[None, None]
+               + 0.5 * torch.randn(B, S, H, L, P, 2, device="cuda", generator=g)).to(attn_dtype).contiguous()
+        logits = torch.randn(B, S, H, L * P, device="cuda", generator=g).to(attn_dtype)
+
+        def run(flags):
+            desc, keep = _cabi.make_desc(B, S, S, H, D, L, P, _cabi.BF16, acode, shapes, synth.level_start_index(shapes),
+                                         flags)
+            outs = [torch.empty(B, S, H * D, dtype=torch.bfloat16, device="cuda") for _ in range(3)]
+            _cabi.check(lib.msda_b200_forward(desc, value.data_ptr(), loc.data_ptr(), attn.data_ptr(), outs[0].data_ptr(),
+                                              order.data_ptr(), stream))
+            for out, r in ((outs[1], ref.data_ptr()), (outs[2], None)):
+                _cabi.check(lib.msda_b200_forward_fused(desc, value.data_ptr(), off.data_ptr(), logits.data_ptr(), r,
+                                                        out.data_ptr(), None, order.data_ptr(), stream))
+            torch.cuda.synchronize()
+            return outs
+
+        for name, pair, one in zip(("plain", "fused", "fused, implicit ref"), run(0), run(_cabi.FLAG_STRICT_PADDING)):
+            assert pair.abs().max() > 0, f"{tag}/{dist}: {name}"
+            assert torch.equal(pair, one), f"{tag}/{dist}: {name}"
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16], ids=["fp32", "bf16"])

@@ -11,13 +11,12 @@ import os
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "libmsda_b200.so")
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 MAX_LEVELS = 8
 F32, BF16, U8 = 0, 1, 2
 FLAG_PROFILE = 1
 FLAG_BF16_ATOMICS = 2
 FLAG_BWD_V1 = 4
-FLAG_NO_WINDOW = 8
 FLAG_STRICT_PADDING = 16
 FLAG_BWD_V2 = 32
 PROF_FWD, PROF_BWD_ZERO, PROF_BWD_MAIN, PROF_BWD_CONVERT = 0, 1, 2, 3
@@ -66,8 +65,6 @@ class Desc(ctypes.Structure):
         ("value_dtype", ctypes.c_int32), ("attn_dtype", ctypes.c_int32), ("flags", ctypes.c_uint32),
         ("spatial_shapes_hw", ctypes.POINTER(ctypes.c_int32)),
         ("level_start_index", ctypes.POINTER(ctypes.c_int64)),
-        ("tile_start", ctypes.c_void_p), ("num_tiles", ctypes.c_int32), ("max_tile", ctypes.c_int32),
-        ("tile_rows", ctypes.c_int32), ("tile_cols", ctypes.c_int32),
     ]
 
 
@@ -177,12 +174,11 @@ def check(rc: int) -> None:
 _desc_cache: dict = {}
 
 
-def make_desc(B, S, Q, H, D, L, P, value_dtype, attn_dtype, shapes_hw, level_start, flags=0, schedule=None):
+def make_desc(B, S, Q, H, D, L, P, value_dtype, attn_dtype, shapes_hw, level_start, flags=0):
     """Build a ``Desc`` plus the host arrays it points to (keep the returned tuple alive).
 
     Descriptors are immutable once built and the library only reads them during the call, so identical
-    problems share one cached instance (saves ~9 us of ctypes marshalling per call). ``schedule`` is a
-    ``functional.Schedule`` (device tile table) or None.
+    problems share one cached instance (saves ~9 us of ctypes marshalling per call).
     """
     key = (B, S, Q, H, D, L, P, value_dtype, attn_dtype, flags, tuple(tuple(hw) for hw in shapes_hw), tuple(level_start))
     hit = _desc_cache.get(key)
@@ -192,17 +188,12 @@ def make_desc(B, S, Q, H, D, L, P, value_dtype, attn_dtype, shapes_hw, level_sta
     else:
         shp = (ctypes.c_int32 * (2 * L))(*[int(v) for hw in shapes_hw for v in hw])
         lsi = (ctypes.c_int64 * L)(*[int(v) for v in level_start])
-        d0 = Desc(B, S, Q, H, D, L, P, value_dtype, attn_dtype, flags, shp, lsi, None, 0, 0, 0, 0)
+        d0 = Desc(B, S, Q, H, D, L, P, value_dtype, attn_dtype, flags, shp, lsi)
         if len(_desc_cache) > 256:
             _desc_cache.clear()
         keep = (shp, lsi)
         _desc_cache[key] = (d0, keep)
         d = Desc.from_buffer_copy(d0)
-    if schedule is not None:
-        d.tile_start = schedule.tile_start.data_ptr()
-        d.num_tiles = schedule.num_tiles
-        d.max_tile = schedule.max_tile
-        d.tile_rows, d.tile_cols = schedule.tile
     return d, keep
 
 

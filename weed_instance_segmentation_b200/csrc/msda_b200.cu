@@ -23,15 +23,10 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 
 #include "msda_b200.h"
-
-// msda_win.cu: window-staged (TMA) kernels for the pixel decoder's geometry
-extern "C" int msda_b200_internal_win_applicable(const msda_b200_desc* desc, const void* query_order);
-extern "C" int msda_b200_internal_win_forward(const msda_b200_desc* desc, const void* kparams, void* stream);
 
 namespace {
 
@@ -706,8 +701,6 @@ int validate(const msda_b200_desc* d) {
   const long long per_batch = (long long)d->S * d->H * d->D * (long long)dtype_size(d->value_dtype) / 16;
   if (per_batch >= (1ll << 31)) return fail(MSDA_B200_ERR_UNSUPPORTED, "S*H*D too large for 32-bit tile offsets");
   if ((long long)d->L * d->P > 64) return fail(MSDA_B200_ERR_UNSUPPORTED, "L*P=%d exceeds 64", d->L * d->P);
-  if (d->tile_start && (d->num_tiles <= 0 || d->max_tile <= 0))
-    return fail(MSDA_B200_ERR_INVALID, "tile schedule with num_tiles=%d, max_tile=%d", d->num_tiles, d->max_tile);
   return MSDA_B200_OK;
 }
 
@@ -737,11 +730,6 @@ int check_launch(const char* what) {
 constexpr int kFwdNT = 128, kFwdQPG = 1;  // measured on config 2: 0.332 ms (256/1: 0.347, 256/2: 0.332, 512/1: 0.410)
 constexpr int kBwdNT = 128, kBwdQPG = 1;
 
-int env_cfg(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v && *v ? atoi(v) : dflt;
-}
-
 template <typename VT, typename AT, int D, bool FUSED>
 int launch_fwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   constexpr int LPP = D / Vec16<VT>::N;
@@ -755,8 +743,6 @@ int launch_fwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   if (smem > 48 * 1024 &&
       cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return fail(MSDA_B200_ERR_CUDA, "forward: cannot reserve %zu bytes of shared memory", smem);
-  if (const int carve = env_cfg("MSDA_B200_FWD1_CARVEOUT", -1); carve >= 0)  // tuning runs (see launch_fwd_pair_cfg)
-    cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
   const long long blocks = (long long)p.B * p.num_tiles * p.H;
   if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "forward: grid too large");
   {
@@ -767,10 +753,12 @@ int launch_fwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   return check_launch("msda_b200_forward");
 }
 
-// Forward with two heads per block (see msda_fwd_pair_kernel). NT / QPG from the environment for tuning runs only.
-template <typename VT, typename AT, int D, int NT, int QPG, bool FUSED>
-int launch_fwd_pair_cfg(const msda_b200_desc* d, KParams p, cudaStream_t st) {
-  constexpr int HPB = 2;
+// Forward with two heads per block (see msda_fwd_pair_kernel). 128 threads, 2 (query, head) pairs per lane group
+// measured best on config 2 (ms): 128/2 0.294, 128/1 0.302, 256/2 0.297, 256/1 0.307, 128/4 0.407; one head per block
+// (msda_fwd_kernel) 0.313
+template <typename VT, typename AT, int D, bool FUSED>
+int launch_fwd_pair(const msda_b200_desc* d, KParams p, cudaStream_t st) {
+  constexpr int NT = 128, QPG = 2, HPB = 2;
   constexpr int LPP = D / Vec16<VT>::N, NG = NT / LPP, TV = NG * QPG, TQ = TV / HPB, ROW = TV + 1;
   fill_geometry(d, p, TQ);
   const size_t smem = (size_t)p.LP * ROW * (sizeof(float4) + sizeof(int)) + (FUSED ? (size_t)TV * p.LP * sizeof(float) + (size_t)TQ * sizeof(float2) : 0);
@@ -784,8 +772,7 @@ int launch_fwd_pair_cfg(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   // 124 KB of L1. Measured (profiles/r02_notes.md; config 2 init / trained, config 3 init / trained, ms): default
   // 0.286 / 0.306 / 0.661 / 0.717, 50 %: 0.282 / 0.301 / 0.655 / 0.696, 40 %: 0.313 / 0.337 / 0.697 / 0.747. The fused
   // prologue's blocks are 3 KB larger (softmax tile), 50 % holds only 6 of them: 0.407 vs 0.321 ms -> driver default.
-  cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout,
-                       env_cfg("MSDA_B200_FWD_CARVEOUT", FUSED ? -1 : 50));
+  cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, FUSED ? -1 : 50);
   const long long blocks = (long long)p.B * p.num_tiles * (p.H / HPB);
   if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "forward: grid too large");
   {
@@ -794,13 +781,6 @@ int launch_fwd_pair_cfg(const msda_b200_desc* d, KParams p, cudaStream_t st) {
     ++g_launches;
   }
   return check_launch("msda_b200_forward (head pairs)");
-}
-
-template <typename VT, typename AT, int D, bool FUSED>
-int launch_fwd_pair(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
-  // 128 threads, 2 (query, head) pairs per lane group measured best on config 2 (ms): 128/2 0.294, 128/1 0.302,
-  // 256/2 0.297, 256/1 0.307, 128/4 0.407; one head per block (msda_fwd_kernel) 0.313
-  return launch_fwd_pair_cfg<VT, AT, D, 128, 2, FUSED>(d, p, st);
 }
 
 template <typename VT, typename AT, int D, int ACC, bool FUSED>
@@ -816,8 +796,6 @@ int launch_bwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   if (smem > 48 * 1024 &&
       cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return fail(MSDA_B200_ERR_CUDA, "backward: cannot reserve %zu bytes of shared memory", smem);
-  if (const int carve = env_cfg("MSDA_B200_BWD1_CARVEOUT", -1); carve >= 0)  // tuning runs (see launch_fwd_pair_cfg)
-    cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
   const long long blocks = (long long)p.B * p.num_tiles * p.H;
   if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "backward: grid too large");
   {
@@ -832,7 +810,7 @@ template <typename VT, typename AT, bool FUSED>
 int dispatch_fwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
   if constexpr (std::is_same<VT, __nv_bfloat16>::value) {
     // 64-byte rows (bf16, D = 32): pair an even with an odd head (bank-conflict-free quarter-warps)
-    if (d->D == 32 && d->H % 2 == 0 && !(d->flags & MSDA_B200_FLAG_STRICT_PADDING) && !env_cfg("MSDA_B200_FWD_NO_PAIR", 0))
+    if (d->D == 32 && d->H % 2 == 0 && !(d->flags & MSDA_B200_FLAG_STRICT_PADDING))
       return launch_fwd_pair<VT, AT, 32, FUSED>(d, p, st);
   }
   switch (d->D) {
@@ -921,16 +899,6 @@ int dispatch_bwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
 
 template <bool FUSED>
 int run_forward(const msda_b200_desc* desc, const KParams& p, cudaStream_t st) {
-  if (!FUSED && msda_b200_internal_win_applicable(desc, p.q_order)) {
-    KParams w = p;
-    fill_geometry(desc, w, 1);
-    {
-      ProfScope ps((desc->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_FWD, st);
-      if (int rc = msda_b200_internal_win_forward(desc, &w, st)) return rc;
-      ++g_launches;
-    }
-    return check_launch("msda_b200_forward (window)");
-  }
   const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
   if (!vbf) return dispatch_fwd<float, float, FUSED>(desc, p, st);
   if (abf) return dispatch_fwd<__nv_bfloat16, __nv_bfloat16, FUSED>(desc, p, st);

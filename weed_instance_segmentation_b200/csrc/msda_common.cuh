@@ -1,5 +1,6 @@
-// msda_common.cuh -- structs and device helpers shared by the kernels of msda_b200.cu and msda_win.cu.
-// Included INSIDE each translation unit's anonymous namespace (after <cuda_bf16.h>, <cuda_runtime.h> and msda_b200.h).
+// msda_common.cuh -- structs and device helpers shared by the kernels of msda_b200.cu, msda_bwd_sorted.cuh and
+// msda_bwd_mma.cuh. Included INSIDE msda_b200.cu's anonymous namespace (after <cuda_bf16.h>, <cuda_runtime.h> and
+// msda_b200.h).
 #pragma once
 
 constexpr int kMaxL = MSDA_B200_MAX_LEVELS;

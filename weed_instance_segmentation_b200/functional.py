@@ -112,70 +112,6 @@ def query_order_2d(shapes: Sequence[tuple[int, int]], tile: int, device) -> torc
     return order
 
 
-class Schedule:
-    """Device-side tile schedule (``msda_b200_desc.tile_start`` & co): ``order`` is a permutation of the queries,
-    tile ``t`` owns ``order[tile_start[t]:tile_start[t+1]]``."""
-
-    __slots__ = ("order", "tile_start", "num_tiles", "max_tile", "tile")
-
-    def __init__(self, order, tile_start, num_tiles, max_tile, tile):
-        self.order, self.tile_start, self.num_tiles, self.max_tile, self.tile = order, tile_start, num_tiles, max_tile, tile
-
-
-_WIN_TILE = _parse_tile(os.environ.get("MSDA_B200_WIN_TILE", "8x16"))
-_WIN_MAX_TILE = 192  # kWinTQ of csrc/msda_win.cu
-_sched_cache: dict = {}
-
-
-def pyramid_schedule(shapes: Sequence[tuple[int, int]], tile=None, max_tile: int = _WIN_MAX_TILE, device="cpu") -> Schedule:
-    """Tiles for the window-staged kernels (csrc/msda_win.cu), for ``Q == S`` (query i sits on pixel i, M2F:1117-1123).
-
-    A tile is a ``tile`` = (rows, cols) patch of the finest level plus every coarser-level query whose reference
-    point (the centre of its own pixel, M2F:1095-1125) falls into that patch: all of a tile's queries then sample
-    around the same place in every level, so one small window per level covers them. Tiles larger than
-    ``max_tile`` are split. Scheduling only; results do not depend on it.
-    """
-    th, tw = _WIN_TILE if tile is None else tile
-    key = (tuple(shapes), th, tw, max_tile, str(device))
-    hit = _sched_cache.get(key)
-    if hit is not None:
-        return hit
-    anchor = max(range(len(shapes)), key=lambda l: shapes[l][0] * shapes[l][1])
-    ha, wa = shapes[anchor]
-    tiles_x = (wa + tw - 1) // tw
-    ids = []
-    for h, w in shapes:
-        y = torch.arange(h, dtype=torch.float64).view(h, 1).expand(h, w)
-        x = torch.arange(w, dtype=torch.float64).view(1, w).expand(h, w)
-        cy = ((y + 0.5) / h * ha).floor().clamp_(0, ha - 1).long()
-        cx = ((x + 0.5) / w * wa).floor().clamp_(0, wa - 1).long()
-        ids.append(((cy // th) * tiles_x + cx // tw).reshape(-1))
-    ids = torch.cat(ids)
-    order = torch.argsort(ids, stable=True)  # inside a tile: level-major, row-major
-    counts = torch.bincount(ids, minlength=1).tolist()
-    starts, acc = [0], 0
-    for c in counts:
-        done = 0
-        while done < c:
-            step = min(max_tile, c - done)
-            done += step
-            starts.append(acc + done)
-        acc += c
-    sizes = [b - a for a, b in zip(starts[:-1], starts[1:])]
-    sched = Schedule(order.to(torch.int32).to(device), torch.tensor(starts, dtype=torch.int32).to(device),
-                     len(sizes), max(sizes) if sizes else 0, (th, tw))
-    if len(_sched_cache) > 64:
-        _sched_cache.clear()
-    _sched_cache[key] = sched
-    return sched
-
-
-def _window_eligible(value, loc) -> bool:
-    """Geometries csrc/msda_win.cu covers (the library re-checks; everything else stays on msda_b200.cu)."""
-    return (value.dtype == torch.bfloat16 and value.shape[-1] == 32 and loc.shape[4] == 4 and loc.shape[3] <= 4
-            and os.environ.get("MSDA_B200_WINDOW", "0") == "1")
-
-
 def _check_inputs(value, shapes, loc, attn):
     if not (value.is_cuda and loc.is_cuda and attn.is_cuda):
         raise RuntimeError("ms_deform_attn: tensors must live on a CUDA device (this package has no CPU fallback)")
@@ -219,7 +155,7 @@ class MSDeformAttnFunction(torch.autograd.Function):
     """Forward / backward through ``msda_b200_forward`` / ``msda_b200_backward``."""
 
     @staticmethod
-    def forward(ctx, value, shapes, level_start, loc, attn, query_order, flags, schedule=None):
+    def forward(ctx, value, shapes, level_start, loc, attn, query_order, flags):
         lib = _cabi.load()
         in_dtypes = (loc.dtype, attn.dtype)
         value_c, loc_c, attn_c = _prepare(value, loc, attn)
@@ -227,12 +163,11 @@ class MSDeformAttnFunction(torch.autograd.Function):
         _, Q, _, L, P, _ = loc_c.shape
         out = torch.empty((B, Q, H * D), dtype=value_c.dtype, device=value_c.device)
         desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value_c.dtype], _DTYPE_CODE[attn_c.dtype],
-                                     shapes, level_start, flags, schedule)
-        fwd_order = schedule.order if schedule is not None else query_order
+                                     shapes, level_start, flags)
         with torch.cuda.device(value_c.device):
             stream = torch.cuda.current_stream().cuda_stream
             _cabi.check(lib.msda_b200_forward(desc, _ptr(value_c), _ptr(loc_c), _ptr(attn_c), _ptr(out),
-                                              _ptr(fwd_order), stream))
+                                              _ptr(query_order), stream))
         ctx.save_for_backward(value_c, loc_c, attn_c, query_order)
         ctx.geom = (shapes, level_start, flags, in_dtypes)
         del keep
@@ -270,7 +205,7 @@ class MSDeformAttnFunction(torch.autograd.Function):
             grad_loc = grad_loc.to(loc_dtype)
         if grad_attn.dtype != attn_dtype:
             grad_attn = grad_attn.to(attn_dtype)
-        return grad_value, None, None, grad_loc, grad_attn, None, None, None
+        return grad_value, None, None, grad_loc, grad_attn, None, None
 
 
 def ms_deform_attn(
@@ -296,16 +231,13 @@ def ms_deform_attn(
     shapes = _shapes_list(value_spatial_shapes)
     B, S, Q, H, D, L, P = _check_inputs(value, shapes, sampling_locations, attention_weights)
     level_start = _level_start(shapes, level_start_index)
-    order = sched = None
+    order = None
     if _USE_ORDER and Q == S and Q == sum(h * w for h, w in shapes) and level_start == _level_start(shapes, None):
         order = query_order_2d(shapes, _TILE, value.device)
-        if _window_eligible(value, sampling_locations):
-            sched = pyramid_schedule(shapes, device=value.device)
     flags = _cabi.FLAG_PROFILE if profile else 0
     if _STRICT_PADDING:
         flags |= _cabi.FLAG_STRICT_PADDING
-    return MSDeformAttnFunction.apply(value, shapes, level_start, sampling_locations, attention_weights, order, flags,
-                                      sched)
+    return MSDeformAttnFunction.apply(value, shapes, level_start, sampling_locations, attention_weights, order, flags)
 
 
 def multi_scale_deformable_attention(value, value_spatial_shapes, sampling_locations, attention_weights):
