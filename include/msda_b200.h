@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define MSDA_B200_ABI_VERSION 12
+#define MSDA_B200_ABI_VERSION 13
 #define MSDA_B200_MAX_LEVELS 8
 
 /* dtype codes */
@@ -72,6 +72,19 @@ extern "C" {
                                          /* value in a pixel grid_sample's zeros padding never reads (M2F:823)  */
                                          /* cannot become 0 * Inf = NaN; 25-30 % slower (the backward kernels    */
                                          /* always treat out-of-level corners as unread)                         */
+#define MSDA_B200_FLAG_DETERMINISTIC 64u /* backward: bit-identical grad_value, grad_loc / grad_offsets and         */
+                                         /* grad_attn / grad_logits for bit-identical inputs, whatever the stream,  */
+                                         /* query_order or host-pipeline chunking; takes precedence over BWD_V1,    */
+                                         /* BWD_V2 and BF16_ATOMICS.  No float atomics: the per-corner kernel       */
+                                         /* writes grad_loc / grad_attn and four (grad_value row, query, weight)    */
+                                         /* records per sample, a stable radix sort groups them by row in sample    */
+                                         /* order, and LPP lanes per (batch, row, head) sum their records in fp32   */
+                                         /* in that order and write grad_value once (every element, rows no sample  */
+                                         /* reads get 0).  Same dtypes and geometries as the default backward.      */
+                                         /* Needs a workspace (fp32 values too) of 24 bytes per record (4 per       */
+                                         /* sample: uint32 key + uint64 payload, double-buffered for the sort),     */
+                                         /* 8 bytes per (batch, row, head) bucket and the sort's scratch; problems  */
+                                         /* over 2^31 - 1 records or 2^32 - 1 buckets are MSDA_B200_ERR_UNSUPPORTED */
 
 /* Problem description: plain old data, filled by the caller on the host. */
 typedef struct msda_b200_desc {
@@ -106,13 +119,17 @@ int msda_b200_forward(const msda_b200_desc* desc, const void* value /*dev*/, con
                       const void* attn /*dev*/, void* out /*dev*/, const int32_t* query_order /*dev|NULL*/,
                       void* stream);
 
-/* Bytes of device scratch msda_b200_backward needs for this problem (0 if none). */
+/* Bytes of device scratch msda_b200_backward needs for this problem (0 if none).  bf16 values: B*S*H*D float32
+ * accumulators (none with MSDA_B200_FLAG_BF16_ATOMICS).  MSDA_B200_FLAG_DETERMINISTIC: the layout its comment
+ * describes, whatever the dtypes (0 for an invalid or unsupported descriptor). */
 size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc);
 
 /*
  * Backward.  Replaces autograd through M2F:798-837 (grid_sampler_2d_backward x L, etc.).
  * Writes every element of grad_value (B,S,H,D; the library zero-fills it first),
  * grad_loc (B,Q,H,L,P,2) float32 and grad_attn (B,Q,H,L,P).
+ * grad_value is summed with unordered float atomics, so its last bits vary from run to run; set
+ * MSDA_B200_FLAG_DETERMINISTIC for run-to-run identical gradients.
  */
 int msda_b200_backward(const msda_b200_desc* desc, const void* value /*dev*/, const float* loc /*dev*/,
                        const void* attn /*dev*/, const void* grad_out /*dev*/, void* grad_value /*dev*/,

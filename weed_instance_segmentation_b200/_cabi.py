@@ -11,7 +11,7 @@ import os
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "libmsda_b200.so")
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 MAX_LEVELS = 8
 F32, BF16, U8 = 0, 1, 2
 FLAG_PROFILE = 1
@@ -19,6 +19,7 @@ FLAG_BF16_ATOMICS = 2
 FLAG_BWD_V1 = 4
 FLAG_STRICT_PADDING = 16
 FLAG_BWD_V2 = 32
+FLAG_DETERMINISTIC = 64
 PROF_FWD, PROF_BWD_ZERO, PROF_BWD_MAIN, PROF_BWD_CONVERT = 0, 1, 2, 3
 
 # every symbol include/msda_b200.h declares

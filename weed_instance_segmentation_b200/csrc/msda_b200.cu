@@ -27,6 +27,12 @@
 #include <type_traits>
 
 #include "msda_b200.h"
+#include "msda_bwd_det.cuh"
+
+// msda_bwd_det.cu: the deterministic backward's sort and grad_value pull (CUB stays out of this file)
+extern "C" int msda_b200_internal_det_workspace_bytes(const msda_b200_desc* desc, size_t* bytes);
+extern "C" int msda_b200_internal_det_grad_value(const msda_b200_desc* desc, const void* grad_out, void* grad_value,
+                                                 void* workspace, cudaStream_t stream);
 
 namespace {
 
@@ -440,6 +446,8 @@ __global__ void __launch_bounds__(NT) msda_fwd_pair_kernel(const __grid_constant
 // ---------------------------------------------------------------------------------------------
 // ACC: 0 = fp32 accumulator with red.v4.f32 (grad_value itself for fp32 values, workspace for bf16)
 //      1 = bf16 grad_value accumulated in place with red.v4.bf16x2 (MSDA_B200_FLAG_BF16_ATOMICS)
+//      2 = no grad_value scatter: phase 1 writes each sample's grad_value records for msda_bwd_det.cu
+//          (MSDA_B200_FLAG_DETERMINISTIC); grad_loc / grad_attn as in the other modes
 template <typename VT, typename AT, int D, int NT, int QPG, int ACC, bool FUSED>
 __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KParams p) {
   constexpr int VEC = Vec16<VT>::N;
@@ -486,6 +494,27 @@ __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KP
     // that have one are flagged in the sign bit and take predicated loads in phase 2
     const bool all_alive = ok && ax.g0 != 0.f && ax.g1 != 0.f && ay.g0 != 0.f && ay.g1 != 0.f;
     soff[k] = (((lv.start + ay.base * lv.W + ax.base) * p.H + h) * LPP) | (all_alive ? 0 : (int)0x80000000);
+    if (ACC == 2) {
+      // grad_value records of the four slots (msda_bwd_det.cuh), with phase 2's liveness rule and weight expression
+      const float sx[2] = {ax.s0, ax.s1}, sy[2] = {ay.s0, ay.s1};
+      const bool gx[2] = {ax.g0 != 0.f, ax.g1 != 0.f}, gy[2] = {ay.g0 != 0.f, ay.g1 != 0.f};
+      const long long row0 = (long long)b * p.S + lv.start + ay.base * lv.W + ax.base;
+      unsigned key[4];
+      unsigned long long val[4];
+#pragma unroll
+      for (int cn = 0; cn < 4; ++cn) {
+        const int cy = cn >> 1, cx = cn & 1;
+        const float wc = a * sy[cy] * sx[cx];
+        const bool live = ok && gx[cx] && gy[cy] && wc != 0.f;
+        key[cn] = live ? (unsigned)((row0 + cy * lv.W + cx) * p.H + h) : p.det_sentinel;
+        val[cn] = ((unsigned long long)q << 32) | __float_as_uint(wc);
+      }
+      uint4* kd = reinterpret_cast<uint4*>(p.det_keys) + si;
+      *kd = make_uint4(key[0], key[1], key[2], key[3]);
+      ulonglong2* vd = reinterpret_cast<ulonglong2*>(p.det_vals) + 2 * si;
+      vd[0] = make_ulonglong2(val[0], val[1]);
+      vd[1] = make_ulonglong2(val[2], val[3]);
+    }
   }
   __syncthreads();
 
@@ -533,7 +562,7 @@ __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KP
 #pragma unroll
           for (int j = 0; j < VEC; ++j) d = fmaf(go[j], f[j], d);
           dot[cn] = d;
-          if (alive[cn] && wc[cn] != 0.f) {
+          if (ACC != 2 && alive[cn] && wc[cn] != 0.f) {
             // element offset of this lane's 16 bytes inside grad_value
             const long long e = ((long long)b * p.batch_stride16 + off + coff[cn] + c) * VEC;
             if (ACC == 0) {
@@ -879,7 +908,7 @@ int launch_bwd_mma(const msda_b200_desc* d, KParams p, cudaStream_t st) {
 
 template <typename VT, typename AT, int ACC, bool FUSED>
 int dispatch_bwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
-  if constexpr (std::is_same<VT, __nv_bfloat16>::value) {
+  if constexpr (std::is_same<VT, __nv_bfloat16>::value && ACC != 2) {
     if (sorted_applicable(d)) {
       if constexpr (ACC == 0) {
         if (!(d->flags & MSDA_B200_FLAG_BWD_V2)) return launch_bwd_mma<AT, FUSED>(d, p, st);
@@ -955,6 +984,35 @@ int run_backward(const msda_b200_desc* desc, KParams p, void* grad_value, void* 
   return MSDA_B200_OK;
 }
 
+// MSDA_B200_FLAG_DETERMINISTIC: the per-corner kernel without its scatter writes grad_loc / grad_attn and the records
+// of every sample; msda_bwd_det.cu orders the records and writes every element of grad_value from them. No float
+// atomics, so equal inputs give equal bits.
+template <bool FUSED>
+int run_backward_det(const msda_b200_desc* desc, KParams p, void* grad_value, void* workspace, size_t workspace_bytes,
+                     bool have_tensors, cudaStream_t st) {
+  if (desc->B == 0) return MSDA_B200_OK;
+  if (!grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
+  size_t need = 0;
+  if (int rc = msda_b200_internal_det_workspace_bytes(desc, &need)) return rc;
+  if (!workspace || workspace_bytes < need)
+    return fail(MSDA_B200_ERR_WORKSPACE, "backward: workspace of %zu bytes required, got %zu", need, workspace_bytes);
+  if (reinterpret_cast<uintptr_t>(workspace) & 15) return fail(MSDA_B200_ERR_INVALID, "backward: workspace must be 16-byte aligned");
+  if (desc->Q != 0) {
+    if (!have_tensors) return fail(MSDA_B200_ERR_INVALID, "backward: NULL tensor pointer");
+    const DetLayout lay = det_layout(desc);
+    p.det_keys = reinterpret_cast<unsigned*>(static_cast<char*>(workspace) + lay.keys_off[0]);
+    p.det_vals = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + lay.vals_off[0]);
+    p.det_sentinel = (unsigned)lay.keys;
+    const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
+    int rc;
+    if (!vbf) rc = dispatch_bwd<float, float, 2, FUSED>(desc, p, st);
+    else rc = abf ? dispatch_bwd<__nv_bfloat16, __nv_bfloat16, 2, FUSED>(desc, p, st)
+                  : dispatch_bwd<__nv_bfloat16, float, 2, FUSED>(desc, p, st);
+    if (rc) return rc;
+  }
+  return msda_b200_internal_det_grad_value(desc, p.grad_out, grad_value, workspace, st);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1000,6 +1058,11 @@ int msda_b200_forward_fused(const msda_b200_desc* desc, const void* value, const
 
 size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc) {
   if (!desc) return 0;
+  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC) {
+    size_t bytes = 0;
+    if (validate(desc) || msda_b200_internal_det_workspace_bytes(desc, &bytes)) return 0;
+    return bytes;
+  }
   if (desc->value_dtype == MSDA_B200_BF16 && !(desc->flags & MSDA_B200_FLAG_BF16_ATOMICS))
     return (size_t)desc->B * desc->S * desc->H * desc->D * sizeof(float);
   return 0;
@@ -1015,6 +1078,8 @@ int msda_b200_backward(const msda_b200_desc* desc, const void* value, const floa
   p.value = value; p.loc = loc; p.attn = attn; p.grad_out = grad_out;
   p.grad_loc = grad_loc; p.grad_attn = grad_attn; p.q_order = query_order;
   const bool have = value && loc && attn && grad_out && grad_loc && grad_attn;
+  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC)
+    return run_backward_det<false>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
   return run_backward<false>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -1031,6 +1096,8 @@ int msda_b200_backward_fused(const msda_b200_desc* desc, const void* value, cons
   if (!ref_points && desc->Q != desc->S)
     return fail(MSDA_B200_ERR_INVALID, "backward_fused: implicit reference points (ref_points = NULL) need Q == S");
   const bool have = value && offsets && logits && grad_out && grad_offsets && grad_logits;
+  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC)
+    return run_backward_det<true>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
   return run_backward<true>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
 }
 

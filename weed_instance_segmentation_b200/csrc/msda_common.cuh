@@ -33,6 +33,10 @@ struct KParams {
   int num_tiles;
   long long batch_stride16;  // S*H*D*sizeof(T)/16
   Level lv[kMaxL];
+  // deterministic backward (msda_bwd_kernel with ACC = 2): four grad_value records per sample, see msda_bwd_det.cuh
+  unsigned* det_keys;
+  unsigned long long* det_vals;
+  unsigned det_sentinel;
 };
 
 // ---------------------------------------------------------------------------------------------

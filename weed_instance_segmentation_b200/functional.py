@@ -50,6 +50,18 @@ _order_cache: dict = {}
 _lsi_checked: dict = {}
 
 
+def deterministic() -> bool:
+    """Whether the package computes gradients reproducibly: ``torch.use_deterministic_algorithms(True)`` is the switch.
+
+    Read at each backward (``HostPipeline`` reads it once, when it is built). When it is on, the op's backward runs
+    with ``FLAG_DETERMINISTIC`` (bit-identical gradients for identical inputs; the ``MSDA_B200_BWD_*`` and
+    ``MSDA_B200_BF16_ATOMICS`` selections are ignored), and the modules leave the B200 kernels whose backward reduces
+    with float atomics or atomic split-K (fused LayerNorm, bias-gradient column sums, the emulated float32 GEMMs, the
+    GroupNorm input assembly) for the torch path they otherwise fall back to.
+    """
+    return torch.are_deterministic_algorithms_enabled()
+
+
 def _shapes_list(value_spatial_shapes) -> list[tuple[int, int]]:
     """``spatial_shapes_list`` (M2F:1312) as host ints. A CUDA tensor costs one sync; pass a list."""
     if isinstance(value_spatial_shapes, torch.Tensor):
@@ -182,12 +194,15 @@ class MSDeformAttnFunction(torch.autograd.Function):
         B, S, H, D = value.shape
         _, Q, _, L, P, _ = loc.shape
         grad_out = grad_out.to(value.dtype).contiguous()
-        if _BF16_ATOMICS and value.dtype == torch.bfloat16:
-            flags |= _cabi.FLAG_BF16_ATOMICS
-        if _BWD_V1:
-            flags |= _cabi.FLAG_BWD_V1
-        if _BWD_V2:
-            flags |= _cabi.FLAG_BWD_V2
+        if deterministic():
+            flags |= _cabi.FLAG_DETERMINISTIC
+        else:
+            if _BF16_ATOMICS and value.dtype == torch.bfloat16:
+                flags |= _cabi.FLAG_BF16_ATOMICS
+            if _BWD_V1:
+                flags |= _cabi.FLAG_BWD_V1
+            if _BWD_V2:
+                flags |= _cabi.FLAG_BWD_V2
         desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value.dtype], _DTYPE_CODE[attn.dtype],
                                      shapes, level_start, flags)
         grad_value = torch.empty_like(value)

@@ -23,12 +23,14 @@ class HostPipeline:
 
     ``batch`` images per step, ``num_queries`` queries per image (``None``: one query per pixel),
     ``chunk_images`` images per staging chunk, ``slots`` staging slots (device memory: ``slots`` chunks).
+    ``deterministic``: run the backward with ``FLAG_DETERMINISTIC`` (bit-identical gradients for identical inputs,
+    whatever the chunking); ``None`` follows ``torch.use_deterministic_algorithms`` at construction.
     """
 
     def __init__(self, batch: int, spatial_shapes: Sequence[tuple[int, int]], num_heads: int, head_dim: int,
                  num_points: int, value_dtype: torch.dtype = torch.bfloat16, attn_dtype: torch.dtype | None = None,
                  num_queries: int | None = None, backward: bool = True, chunk_images: int = 1, slots: int = 3,
-                 device: torch.device | int | None = None):
+                 device: torch.device | int | None = None, deterministic: bool | None = None):
         if not torch.cuda.is_available():
             raise RuntimeError("HostPipeline needs a CUDA device (this package has no CPU fallback)")
         self._handle = None
@@ -43,11 +45,15 @@ class HostPipeline:
         if self.value_dtype not in _DTYPE_CODE or self.attn_dtype not in _DTYPE_CODE:
             raise TypeError("HostPipeline: float32 or bfloat16 tensors only")
         self.backward = bool(backward)
+        self.deterministic = functional.deterministic() if deterministic is None else bool(deterministic)
         flags = 0
-        if functional._BF16_ATOMICS and value_dtype == torch.bfloat16:
-            flags |= _cabi.FLAG_BF16_ATOMICS
-        if functional._BWD_V1:
-            flags |= _cabi.FLAG_BWD_V1
+        if self.deterministic:
+            flags |= _cabi.FLAG_DETERMINISTIC
+        else:
+            if functional._BF16_ATOMICS and value_dtype == torch.bfloat16:
+                flags |= _cabi.FLAG_BF16_ATOMICS
+            if functional._BWD_V1:
+                flags |= _cabi.FLAG_BWD_V1
         lsi = functional._level_start(self.shapes, None)
         desc, self._keep = _cabi.make_desc(self.B, self.S, self.Q, self.H, self.D, self.L, self.P,
                                            _DTYPE_CODE[self.value_dtype], _DTYPE_CODE[self.attn_dtype], self.shapes, lsi,

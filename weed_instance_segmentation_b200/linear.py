@@ -13,6 +13,7 @@ import torch
 import torch.nn.functional as F
 
 from . import _cabi
+from .functional import deterministic
 
 _DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
@@ -30,7 +31,7 @@ def f32_gemm_available() -> bool:
 
 def _use_f32_gemm(x, weight) -> bool:
     return (_F32_EMULATED and x.is_cuda and x.dtype == torch.float32 and weight.dtype == torch.float32
-            and not torch.is_autocast_enabled("cuda") and x.numel() > 0 and f32_gemm_available())
+            and not torch.is_autocast_enabled("cuda") and x.numel() > 0 and not deterministic() and f32_gemm_available())
 
 
 def _f32_workspace(device):

@@ -20,7 +20,7 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
-from .functional import ms_deform_attn
+from .functional import deterministic, ms_deform_attn
 from .fused import ms_deform_attn_fused
 from .layer_norm import add_layer_norm
 from .linear import linear as _fused_linear
@@ -73,7 +73,7 @@ class MSDeformAttn(nn.Module):
 
     def _proj(self, layer: nn.Linear, x):
         """``layer(x)``; with ``fused_linear`` the bias gradient is reduced by the B200 column-sum kernel."""
-        return _fused_linear(x, layer.weight, layer.bias) if self.fused_linear else layer(x)
+        return _fused_linear(x, layer.weight, layer.bias) if self.fused_linear and not deterministic() else layer(x)
 
     @staticmethod
     def with_pos_embed(tensor, position_embeddings):
@@ -189,14 +189,14 @@ class EncoderLayer(nn.Module):
         return new
 
     def _proj(self, layer: nn.Linear, x):
-        return _fused_linear(x, layer.weight, layer.bias) if self.fused_linear else layer(x)
+        return _fused_linear(x, layer.weight, layer.bias) if self.fused_linear and not deterministic() else layer(x)
 
     def _add_norm(self, branch, residual, norm, also_lowp=False, clamp=False):
         """``norm(residual + branch)`` (M2F:1049-1050, 1058-1059); one fused kernel when ``fused_norm`` is set.
         ``also_lowp``: return ``(y, y_bf16_or_None)`` -- the bfloat16 copy comes out of the same kernel.
         ``clamp``: also apply the layer's closing ``torch.clamp(y, -c, c)``, ``c = finfo(y.dtype).max - 1000``
         (M2F:1062-1065) -- inside the fused kernels when they run."""
-        ok = (self.fused_norm and branch.is_cuda and branch.shape[-1] % 128 == 0 and branch.shape[-1] <= 512
+        ok = (self.fused_norm and not deterministic() and branch.is_cuda and branch.shape[-1] % 128 == 0 and branch.shape[-1] <= 512
               and branch.dtype in (torch.float32, torch.bfloat16) and residual.dtype in (torch.float32, torch.bfloat16)
               and (torch.is_autocast_enabled() or (branch.dtype == residual.dtype == torch.float32)))
         if ok:
@@ -238,7 +238,7 @@ class EncoderLayer(nn.Module):
 
         residual = hidden_states
         fc1_in = lowp if lowp is not None else hidden_states
-        if self.fused_linear and self.activation_fn is F.relu:
+        if self.fused_linear and self.activation_fn is F.relu and not deterministic():
             hidden_states = _fused_linear_relu(fc1_in, self.fc1.weight, self.fc1.bias)  # bias + ReLU in the GEMM epilogue
         else:
             hidden_states = self.activation_fn(self._proj(self.fc1, fc1_in))

@@ -29,6 +29,7 @@ import torch
 from torch import nn
 
 from . import _cabi
+from .functional import deterministic
 
 _DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
@@ -141,7 +142,11 @@ def assemble_encoder_inputs(decoder, features) -> dict:
     norms = [decoder.input_projections[i][1] for i in range(len(levels))]
     projected = [conv(x) for conv, x in zip(convs, levels)]  # the 1x1 convolutions: dense GEMMs, left to the library
     shapes = [(int(x.shape[2]), int(x.shape[3])) for x in projected]
-    embeds = groupnorm_to_rows(projected, norms)
+    if deterministic():
+        # the fused kernels accumulate grad_gamma / grad_beta with float atomics: the reference's own sequence instead
+        embeds = torch.cat([norm(x).flatten(2).transpose(1, 2) for norm, x in zip(norms, projected)], 1)
+    else:
+        embeds = groupnorm_to_rows(projected, norms)
     const = decoder._b200_constants.get(decoder, shapes, embeds.shape[0], embeds.device, levels[0].dtype, embeds.dtype)
     # M2F:1315-1317: sine + level_embed[level]; (1, S, C), broadcasts over the batch
     pos = const["sine"] + decoder.level_embed.index_select(0, const["level_of_row"])[None].to(const["sine"].dtype)
