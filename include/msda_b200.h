@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define MSDA_B200_ABI_VERSION 13
+#define MSDA_B200_ABI_VERSION 14
 #define MSDA_B200_MAX_LEVELS 8
 
 /* dtype codes */
@@ -61,26 +61,25 @@ extern "C" {
 #define MSDA_B200_ERR_WORKSPACE 4   /* workspace missing or smaller than ..._workspace_bytes()   */
 
 /* flags (msda_b200_desc.flags) */
+/* Bits 2, 8 and 32 are retired (in-place bf16 atomics, no-window forward, pixel-sorted backward) and are not reused;
+ * every entry point that takes a descriptor returns MSDA_B200_ERR_INVALID for a bit not defined here. */
 #define MSDA_B200_FLAG_PROFILE 1u        /* record CUDA events around each kernel (see below)    */
-#define MSDA_B200_FLAG_BF16_ATOMICS 2u   /* backward, bf16: accumulate grad_value with packed    */
-                                         /* bf16x2 atomics in place (no fp32 workspace, lossy)   */
-#define MSDA_B200_FLAG_BWD_V1 4u         /* backward: force the per-corner reduction kernel (v1)  */
-                                         /* instead of the pixel-sorted kernel (v2, D=32 & P=4)  */
-#define MSDA_B200_FLAG_BWD_V2 32u        /* backward: force the CUDA-core pixel-sorted kernel (v2) instead of the  */
-                                         /* group-sorted tensor-core kernel (v3, bf16 values, D=32 & P=4)          */
+#define MSDA_B200_FLAG_BWD_V1 4u         /* backward: per-corner reduction kernel (v1) instead of */
+                                         /* the group-sorted tensor-core kernel (v3, bf16,        */
+                                         /* D=32 & P=4)                                           */
 #define MSDA_B200_FLAG_STRICT_PADDING 16u /* forward: skip the FMA of every zero-weight corner, so a non-finite  */
                                          /* value in a pixel grid_sample's zeros padding never reads (M2F:823)  */
                                          /* cannot become 0 * Inf = NaN; 25-30 % slower (the backward kernels    */
                                          /* always treat out-of-level corners as unread)                         */
 #define MSDA_B200_FLAG_DETERMINISTIC 64u /* backward: bit-identical grad_value, grad_loc / grad_offsets and         */
                                          /* grad_attn / grad_logits for bit-identical inputs, whatever the stream,  */
-                                         /* query_order or host-pipeline chunking; takes precedence over BWD_V1,    */
-                                         /* BWD_V2 and BF16_ATOMICS.  No float atomics: the per-corner kernel       */
-                                         /* writes grad_loc / grad_attn and four (grad_value row, query, weight)    */
-                                         /* records per sample, a stable radix sort groups them by row in sample    */
-                                         /* order, and LPP lanes per (batch, row, head) sum their records in fp32   */
-                                         /* in that order and write grad_value once (every element, rows no sample  */
-                                         /* reads get 0).  Same dtypes and geometries as the default backward.      */
+                                         /* query_order or host-pipeline chunking; takes precedence over BWD_V1. No */
+                                         /* float atomics: the per-corner kernel writes grad_loc / grad_attn and    */
+                                         /* four (grad_value row, query, weight) records per sample, a stable radix */
+                                         /* sort groups them by row in sample order, and LPP lanes per (batch, row, */
+                                         /* head) sum their records in fp32 in that order and write grad_value once */
+                                         /* (every element, rows no sample reads get 0).  Same dtypes and           */
+                                         /* geometries as the default backward.                                     */
                                          /* Needs a workspace (fp32 values too) of 24 bytes per record (4 per       */
                                          /* sample: uint32 key + uint64 payload, double-buffered for the sort),     */
                                          /* 8 bytes per (batch, row, head) bucket and the sort's scratch; problems  */
@@ -120,8 +119,8 @@ int msda_b200_forward(const msda_b200_desc* desc, const void* value /*dev*/, con
                       void* stream);
 
 /* Bytes of device scratch msda_b200_backward needs for this problem (0 if none).  bf16 values: B*S*H*D float32
- * accumulators (none with MSDA_B200_FLAG_BF16_ATOMICS).  MSDA_B200_FLAG_DETERMINISTIC: the layout its comment
- * describes, whatever the dtypes (0 for an invalid or unsupported descriptor). */
+ * accumulators.  MSDA_B200_FLAG_DETERMINISTIC: the layout its comment describes, whatever the dtypes (0 for an
+ * invalid or unsupported descriptor). */
 size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc);
 
 /*

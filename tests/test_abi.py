@@ -49,8 +49,8 @@ def test_desc_layout_matches_header_without_tile_schedule():
     assert _cabi.Desc.level_start_index.offset == 48
 
 
-def test_validation_without_gpu(lib):
-    """Argument validation happens before any CUDA call, so it is testable on the CPU box."""
+def test_validation_without_gpu_rejects_retired_flags(lib):
+    """Argument validation, retired flag bits included, happens before any CUDA call, so it is testable on the CPU."""
     from weed_instance_segmentation_b200 import _cabi
     d, keep = _cabi.make_desc(1, 4, 2, 1, 32, 1, 1, _cabi.F32, _cabi.F32, [(3, 3)], [0])
     rc = lib.msda_b200_forward(d, None, None, None, None, None, None)
@@ -61,8 +61,19 @@ def test_validation_without_gpu(lib):
     assert lib.msda_b200_forward(d, None, None, None, None, None, None) == 2  # fp32 value + bf16 attn
     d, keep = _cabi.make_desc(1, 9, 2, 1, 32, 1, 1, _cabi.BF16, _cabi.BF16, [(3, 3)], [0])
     assert lib.msda_b200_backward_workspace_bytes(d) == 9 * 32 * 4
-    d.flags = _cabi.FLAG_BF16_ATOMICS
-    assert lib.msda_b200_backward_workspace_bytes(d) == 0
+    # retired flag bits (2: bf16 atomics, 8: no-window forward, 32: pixel-sorted backward) and unknown ones are
+    # rejected, not ignored
+    for bit in (2, 8, 32, 128):
+        d.flags = bit
+        assert lib.msda_b200_forward(d, None, None, None, None, None, None) == 1
+        assert b"retired" in lib.msda_b200_last_error()
+        assert lib.msda_b200_backward(d, *([None] * 8 + [0, None, None])) == 1
+        assert b"retired" in lib.msda_b200_last_error()
+        assert lib.msda_b200_backward_fused(d, *([None] * 9 + [0, None, None])) == 1
+        assert b"retired" in lib.msda_b200_last_error()
+        handle = ctypes.c_void_p()
+        assert lib.msda_b200_host_pipeline_create(ctypes.byref(d), 1, 2, 1, None, ctypes.byref(handle)) == 1
+        assert b"retired" in lib.msda_b200_last_error() and not handle.value
     # empty problems succeed without touching the device
     d, keep = _cabi.make_desc(0, 9, 2, 1, 32, 1, 1, _cabi.F32, _cabi.F32, [(3, 3)], [0])
     assert lib.msda_b200_forward(d, None, None, None, None, None, None) == 0

@@ -20,13 +20,16 @@ def _header_define(name):
     return int(re.search(rf"#define {name} (\d+)u?\b", text).group(1))
 
 
-def test_flag_matches_header_and_abi_version_is_13(lib):
+def test_flag_matches_header_and_abi_version_is_14(lib):
     from weed_instance_segmentation_b200 import _cabi
     assert _header_define("MSDA_B200_FLAG_DETERMINISTIC") == _cabi.FLAG_DETERMINISTIC == 64
-    assert _header_define("MSDA_B200_ABI_VERSION") == _cabi.ABI_VERSION == lib.msda_b200_abi_version() == 13
-    others = [_cabi.FLAG_PROFILE, _cabi.FLAG_BF16_ATOMICS, _cabi.FLAG_BWD_V1, _cabi.FLAG_STRICT_PADDING, _cabi.FLAG_BWD_V2]
+    assert _header_define("MSDA_B200_ABI_VERSION") == _cabi.ABI_VERSION == lib.msda_b200_abi_version() == 14
+    others = [_cabi.FLAG_PROFILE, _cabi.FLAG_BWD_V1, _cabi.FLAG_STRICT_PADDING]
     assert all(f & _cabi.FLAG_DETERMINISTIC == 0 for f in others)
-    assert _cabi.FLAG_DETERMINISTIC != 8  # the bit of the removed FLAG_NO_WINDOW is not reused
+    assert _cabi.FLAG_DETERMINISTIC not in (2, 8, 32)  # the bits of the retired flags are not reused
+    text = open(os.path.join(ROOT, "include", "msda_b200.h")).read()
+    for retired in ("MSDA_B200_FLAG_BF16_ATOMICS", "MSDA_B200_FLAG_BWD_V2"):
+        assert not re.search(rf"#define {retired}\b", text)
 
 
 def test_deterministic_backward_validates_before_touching_the_device(lib):

@@ -66,7 +66,7 @@ def _kink_mask(off, ref, shapes, eps=1e-3):
 
 
 CASES = [
-    # (tag, B, shapes, H, D, P, Q)  -- D=32 & P=4 in bf16 takes the pixel-sorted backward, the rest v1
+    # (tag, B, shapes, H, D, P, Q)  -- D=32 & P=4 in bf16 takes the group-sorted backward, the rest v1
     ("m2f", 2, [(8, 8), (16, 16), (32, 32)], 8, 32, 4, None),
     ("odd", 1, [(7, 9), (13, 18), (25, 35)], 8, 32, 4, None),
     ("ragged_p3", 2, [(5, 7), (9, 4)], 4, 32, 3, 77),

@@ -141,9 +141,9 @@ def test_random_bf16(wis, case, dist, attn_dtype):
                   safe=_kink_safe(x["sampling_locations"].numpy(), shapes))
 
 
-# Geometries that stress the pixel-sorted backward's window logic (D=32, P=4, bf16 -> msda_bwd_sorted_kernel):
-# levels wider than the 256-pixel window edge, bounding boxes far larger than the 2048-pixel window capacity
-# (everything outside takes the fallback route), Q != S so queries arrive in no spatial order, one and five levels.
+# Geometries that stress the group-sorted backward's window logic (D=32, P=4, bf16 -> msda_bwd_mma_kernel): levels
+# wider than the window's 64 groups (256 pixels), bounding boxes far larger than its 256 4x2-pixel groups (everything
+# outside takes the fallback route), Q != S so queries arrive in no spatial order, one and five levels.
 SORTED_CASES = [
     ("wide_levels", 1, [(12, 300), (256, 20)], 8, 32, 4, 500),
     ("c5_like", 1, [(64, 64), (128, 128), (256, 256)], 2, 32, 4, 3000),
@@ -164,16 +164,15 @@ def test_sorted_backward_windows(wis, case, dist):
                   safe=_kink_safe(x["sampling_locations"].numpy(), shapes))
 
 
-@pytest.mark.parametrize("variant", ["v1", "v2", "v3"])
+@pytest.mark.parametrize("variant", ["v1", "v3"])
 @pytest.mark.parametrize("case", SORTED_CASES[:2] + [CASES[1]], ids=[c[0] for c in SORTED_CASES[:2] + [CASES[1]]])
 def test_every_backward_variant_matches_oracle(wis, monkeypatch, case, variant):
-    """The three selectable bf16 backward kernels -- v1 per-corner reductions (MSDA_B200_FLAG_BWD_V1), v2 pixel-sorted
-    CUDA-core pull (MSDA_B200_FLAG_BWD_V2), v3 group-sorted mma.sync (default) -- each against the oracle."""
+    """Both bf16 backward kernels -- v1 per-corner reductions (MSDA_B200_FLAG_BWD_V1) and v3 group-sorted mma.sync
+    (default) -- each against the oracle."""
     from weed_instance_segmentation_b200 import functional as F
     from weed_instance_segmentation_b200.synth import msda_inputs
     tag, B, shapes, H, D, P, Q = case
     monkeypatch.setattr(F, "_BWD_V1", variant == "v1")
-    monkeypatch.setattr(F, "_BWD_V2", variant == "v2")
     for dist in ("init", "adversarial"):
         x = msda_inputs(B, shapes, num_heads=H, head_dim=D, num_points=P, dist=dist, seed=31, num_queries=Q,
                         value_dtype=torch.bfloat16)
@@ -183,17 +182,17 @@ def test_every_backward_variant_matches_oracle(wis, monkeypatch, case, variant):
 
 
 def test_sorted_and_per_corner_backward_agree(wis, monkeypatch):
-    """v2 (pixel-sorted) and v1 (per-corner reductions) differ only in fp32 summation order."""
+    """The default v3 (group-sorted) and v1 (per-corner reductions) differ only in fp32 summation order."""
     from weed_instance_segmentation_b200 import functional as F
     from weed_instance_segmentation_b200.synth import msda_inputs
     shapes = [(16, 16), (32, 32), (64, 64)]
     x = msda_inputs(2, shapes, dist="trained", seed=13, value_dtype=torch.bfloat16)
     args = (x["value"], shapes, x["sampling_locations"], x["attention_weights"], x["grad_out"])
-    v2 = _run(wis, *args)
+    v3 = _run(wis, *args)
     monkeypatch.setattr(F, "_BWD_V1", True)
     v1 = _run(wis, *args)
-    assert np.array_equal(v1[0], v2[0])
-    for name, a, b in zip(("grad_value", "grad_loc", "grad_attn"), v1[1:], v2[1:]):
+    assert np.array_equal(v1[0], v3[0])
+    for name, a, b in zip(("grad_value", "grad_loc", "grad_attn"), v1[1:], v3[1:]):
         assert rel_err(a, b) <= 1e-2, name  # both carry one bf16 rounding of the output
 
 
@@ -436,7 +435,8 @@ def test_full_size_matches_reference_on_gpu_bf16(wis):
 
 
 def test_sorted_backward_fuzz(wis):
-    """40 random geometries / location patterns (tools/fuzz_sorted_backward.py): v2 and v1 agree to summation order."""
+    """40 random geometries / location patterns (tools/fuzz_sorted_backward.py): the default v3 and v1 agree to
+    summation order."""
     import importlib.util
     import os
     from weed_instance_segmentation_b200 import functional as F
@@ -450,11 +450,11 @@ def test_sorted_backward_fuzz(wis):
             B, shapes, H, Q, dist = fz.random_case(rng)
             value, loc, attn, go = fz.make_inputs(B, shapes, H, Q, dist, rng)
             F._BWD_V1 = False
-            v2 = fz.run(value, shapes, loc, attn, go)
+            v3 = fz.run(value, shapes, loc, attn, go)
             F._BWD_V1 = True
             v1 = fz.run(value, shapes, loc, attn, go)
-            assert torch.equal(v1[0], v2[0])
-            assert fz.rel(v2[1], v1[1]) <= 1.6e-2 and fz.rel(v2[3], v1[3]) <= 1.6e-2, (i, shapes, dist)
-            assert fz.rel(v2[2], v1[2]) <= 1e-4, (i, shapes, dist)
+            assert torch.equal(v1[0], v3[0])
+            assert fz.rel(v3[1], v1[1]) <= 1.6e-2 and fz.rel(v3[3], v1[3]) <= 1.6e-2, (i, shapes, dist)
+            assert fz.rel(v3[2], v1[2]) <= 1e-4, (i, shapes, dist)
     finally:
         F._BWD_V1 = False

@@ -1,5 +1,5 @@
-"""Development check of the backward kernels on a GPU box: v3 (group-sorted, mma.sync) and v2 (pixel-sorted, CUDA cores)
-against v1 (per-corner reductions) on a set of geometries, then their kernel times at BASELINE configs 2 and 3.
+"""Development check of the backward kernels on a GPU box: v3 (group-sorted, mma.sync) against v1 (per-corner
+reductions) on a set of geometries, then their kernel times at BASELINE configs 2 and 3.
 
     python tools/dev_bwd.py [--quick]
 """
@@ -65,20 +65,19 @@ def main():
             pr = Prob(B, shapes, dist, heads=heads, queries=Q, attn_dtype=adt)
             ref, _ = pr.run(_cabi.FLAG_BWD_V1)
             line = f"{tag:14s} attn={'bf16' if adt == torch.bfloat16 else 'f32 '}"
-            for name, flags in (("v2", _cabi.FLAG_BWD_V2), ("v3", 0)):
-                got, _ = pr.run(flags)
-                errs = [rel(g, r) for g, r in zip(got, ref)]
-                finite = all(torch.isfinite(g).all().item() for g in got)
-                bad = (not finite) or max(errs) > 1e-2
-                ok &= not bad
-                line += f" | {name} gv={errs[0]:.2e} gl={errs[1]:.2e} ga={errs[2]:.2e}{' BAD' if bad else ''}"
+            got, _ = pr.run(0)
+            errs = [rel(g, r) for g, r in zip(got, ref)]
+            finite = all(torch.isfinite(g).all().item() for g in got)
+            bad = (not finite) or max(errs) > 1e-2
+            ok &= not bad
+            line += f" | v3 gv={errs[0]:.2e} gl={errs[1]:.2e} ga={errs[2]:.2e}{' BAD' if bad else ''}"
             print(line, flush=True)
     if not quick:
         for tag, B, shapes in (("config2", 8, [(32, 32), (64, 64), (128, 128)]), ("config3", 16, [(31, 41), (61, 81), (121, 162)])):
             for dist in ("init", "trained", "adversarial"):
                 pr = Prob(B, shapes, dist)
                 line = f"{tag}/{dist:12s}"
-                for name, flags in (("v1", _cabi.FLAG_BWD_V1), ("v2", _cabi.FLAG_BWD_V2), ("v3", 0)):
+                for name, flags in (("v1", _cabi.FLAG_BWD_V1), ("v3", 0)):
                     ts = []
                     for _ in range(8):
                         _, ms = pr.run(flags, profile=True)

@@ -1,4 +1,4 @@
-"""Fuzz the pixel-sorted backward (v2) against the per-corner backward (v1) on random geometries.
+"""Fuzz the group-sorted backward (v3, the default) against the per-corner backward (v1) on random geometries.
 
 Both kernels compute the same sums in a different order, so bf16 outputs must agree to a couple of ulps
 and the fp32 grad_loc to ~1e-5. Run on a GPU box:  python tools/fuzz_sorted_backward.py [n_cases] [seed]
@@ -84,19 +84,19 @@ def main():
         B, shapes, H, Q, dist = random_case(rng)
         value, loc, attn, go = make_inputs(B, shapes, H, Q, dist, rng)
         F._BWD_V1 = False
-        v2 = run(value, shapes, loc, attn, go)
+        v3 = run(value, shapes, loc, attn, go)
         F._BWD_V1 = True
         v1 = run(value, shapes, loc, attn, go)
         F._BWD_V1 = False
-        assert torch.equal(v1[0], v2[0])
-        errs = {"grad_value": rel(v2[1], v1[1]), "grad_loc": rel(v2[2], v1[2]), "grad_attn": rel(v2[3], v1[3])}
+        assert torch.equal(v1[0], v3[0])
+        errs = {"grad_value": rel(v3[1], v1[1]), "grad_loc": rel(v3[2], v1[2]), "grad_attn": rel(v3[3], v1[3])}
         bars = {"grad_value": 1.6e-2, "grad_loc": 1e-4, "grad_attn": 1.6e-2}
         for k, e in errs.items():
             worst[k] = max(worst.get(k, 0.0), e)
-            if not (e <= bars[k]) or not all(torch.isfinite(t).all() for t in v2):
+            if not (e <= bars[k]) or not all(torch.isfinite(t).all() for t in v3):
                 print(f"MISMATCH case {i}: B={B} shapes={shapes} H={H} Q={Q} dist={dist}: {k} rel err {e:.3e}")
                 sys.exit(1)
-    print(f"fuzz ok: {n} cases, worst relative differences v2 vs v1: " + ", ".join(f"{k} {v:.2e}" for k, v in worst.items()))
+    print(f"fuzz ok: {n} cases, worst relative differences v3 vs v1: " + ", ".join(f"{k} {v:.2e}" for k, v in worst.items()))
 
 
 if __name__ == "__main__":

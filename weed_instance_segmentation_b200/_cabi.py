@@ -11,15 +11,16 @@ import os
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "libmsda_b200.so")
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 MAX_LEVELS = 8
 F32, BF16, U8 = 0, 1, 2
 FLAG_PROFILE = 1
-FLAG_BF16_ATOMICS = 2
 FLAG_BWD_V1 = 4
 FLAG_STRICT_PADDING = 16
-FLAG_BWD_V2 = 32
 FLAG_DETERMINISTIC = 64
+# retired bits (the library rejects 2 and 32): zero-valued names that bench.py still reads, so they select nothing
+FLAG_BF16_ATOMICS = 0
+FLAG_BWD_V2 = 0
 PROF_FWD, PROF_BWD_ZERO, PROF_BWD_MAIN, PROF_BWD_CONVERT = 0, 1, 2, 3
 
 # every symbol include/msda_b200.h declares

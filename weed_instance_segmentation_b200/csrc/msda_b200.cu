@@ -445,9 +445,9 @@ __global__ void __launch_bounds__(NT) msda_fwd_pair_kernel(const __grid_constant
 // Backward
 // ---------------------------------------------------------------------------------------------
 // ACC: 0 = fp32 accumulator with red.v4.f32 (grad_value itself for fp32 values, workspace for bf16)
-//      1 = bf16 grad_value accumulated in place with red.v4.bf16x2 (MSDA_B200_FLAG_BF16_ATOMICS)
 //      2 = no grad_value scatter: phase 1 writes each sample's grad_value records for msda_bwd_det.cu
-//          (MSDA_B200_FLAG_DETERMINISTIC); grad_loc / grad_attn as in the other modes
+//          (MSDA_B200_FLAG_DETERMINISTIC); grad_loc / grad_attn as with ACC = 0
+//      (1, in-place bf16 atomics, is retired; the values are kept so the kernels' names stay the same)
 template <typename VT, typename AT, int D, int NT, int QPG, int ACC, bool FUSED>
 __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KParams p) {
   constexpr int VEC = Vec16<VT>::N;
@@ -562,21 +562,13 @@ __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KP
 #pragma unroll
           for (int j = 0; j < VEC; ++j) d = fmaf(go[j], f[j], d);
           dot[cn] = d;
-          if (ACC != 2 && alive[cn] && wc[cn] != 0.f) {
+          if (ACC == 0 && alive[cn] && wc[cn] != 0.f) {
             // element offset of this lane's 16 bytes inside grad_value
             const long long e = ((long long)b * p.batch_stride16 + off + coff[cn] + c) * VEC;
-            if (ACC == 0) {
-              float* dst = reinterpret_cast<float*>(p.grad_value_acc) + e;
+            float* dst = reinterpret_cast<float*>(p.grad_value_acc) + e;
 #pragma unroll
-              for (int j = 0; j < VEC; j += 4)
-                red_add_f32x4(dst + j, wc[cn] * go[j], wc[cn] * go[j + 1], wc[cn] * go[j + 2], wc[cn] * go[j + 3]);
-            } else {
-              float t[VEC];
-#pragma unroll
-              for (int j = 0; j < VEC; ++j) t[j] = wc[cn] * go[j];
-              const uint4 pk = Vec16<VT>::pack(t);
-              red_add_bf16x8(reinterpret_cast<VT*>(p.grad_value_acc) + e, pk.x, pk.y, pk.z, pk.w);
-            }
+            for (int j = 0; j < VEC; j += 4)
+              red_add_f32x4(dst + j, wc[cn] * go[j], wc[cn] * go[j + 1], wc[cn] * go[j + 2], wc[cn] * go[j + 3]);
           }
         }
         sd[((size_t)s * T::TQ + ql) * LPP + c] = make_float4(dot[0], dot[1], dot[2], dot[3]);
@@ -630,7 +622,6 @@ __global__ void __launch_bounds__(NT) msda_bwd_kernel(const __grid_constant__ KP
   }
 }
 
-#include "msda_bwd_sorted.cuh"
 #include "msda_bwd_mma.cuh"
 
 // fp32 accumulator -> bf16 grad_value, 8 elements per thread
@@ -706,6 +697,12 @@ size_t dtype_size(int dt) { return dt == MSDA_B200_BF16 ? 2 : 4; }
 
 int validate(const msda_b200_desc* d) {
   if (!d) return fail(MSDA_B200_ERR_INVALID, "desc is NULL");
+  // a retired flag bit (2, 8, 32) selected a kernel that no longer exists: say so instead of ignoring it
+  constexpr uint32_t known = MSDA_B200_FLAG_PROFILE | MSDA_B200_FLAG_BWD_V1 | MSDA_B200_FLAG_STRICT_PADDING |
+                             MSDA_B200_FLAG_DETERMINISTIC;
+  if (d->flags & ~known)
+    return fail(MSDA_B200_ERR_INVALID, "flags 0x%x: bits 0x%x are unknown or retired", (unsigned)d->flags,
+                (unsigned)(d->flags & ~known));
   if (d->B < 0 || d->S < 0 || d->Q < 0) return fail(MSDA_B200_ERR_INVALID, "negative B/S/Q (%d, %d, %d)", d->B, d->S, d->Q);
   if (d->H <= 0 || d->D <= 0 || d->L <= 0 || d->P <= 0)
     return fail(MSDA_B200_ERR_INVALID, "H, D, L, P must be positive (%d, %d, %d, %d)", d->H, d->D, d->L, d->P);
@@ -852,41 +849,19 @@ int dispatch_fwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
   return fail(MSDA_B200_ERR_UNSUPPORTED, "head dim %d", d->D);
 }
 
-// Backward v2 (msda_bwd_sorted.cuh): instantiated for the model's geometry (D = 32, P = 4).
-// 128 queries / 256 threads per block measured best on config 2 (1.24 ms; 64/128: 1.35, 256/512: 1.29).
-constexpr int kSortNT = 256, kSortTQ = 128, kSortCAP = 2048;
+// Backward v3 (msda_bwd_mma.cuh): group-sorted rows + mma.sync, instantiated for the model's geometry (D = 32, P = 4)
+// with bf16 values; fp32 accumulator only.
+constexpr int kMmaNT = 256, kMmaTQ = 128, kMmaGCAP = 256, kMmaRCAP = 1024;
 
-bool sorted_applicable(const msda_b200_desc* d) {
+bool mma_applicable(const msda_b200_desc* d) {
   if (d->flags & MSDA_B200_FLAG_BWD_V1) return false;
   if (d->D != 32 || d->P != 4) return false;
-  // fp32 rows are 8 lanes wide: half as many entries per warp step, measured slower than v1 (2.35 vs 2.12 ms)
+  // fp32 values stay on v1: the mma.sync products take bf16 operands
   if (d->value_dtype != MSDA_B200_BF16) return false;
   for (int l = 0; l < d->L; ++l)  // pixel coordinates are packed into 12 bits each
     if (d->spatial_shapes_hw[2 * l] > 4095 || d->spatial_shapes_hw[2 * l + 1] > 4095) return false;
   return true;
 }
-
-template <typename VT, typename AT, int ACC, bool FUSED, int kNT, int kTQ, int kPL>
-int launch_bwd_sorted_cfg(const msda_b200_desc* d, KParams p, cudaStream_t st) {
-  constexpr int D = 32, P = 4;
-  constexpr int LPP = D / Vec16<VT>::N;
-  fill_geometry(d, p, kTQ);
-  const size_t smem = sorted_smem_layout<kNT, kTQ, P, kSortCAP, LPP>().total;
-  auto kern = msda_bwd_sorted_kernel<VT, AT, D, kNT, kTQ, P, kSortCAP, ACC, FUSED, kPL>;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "backward: cannot reserve %zu bytes of shared memory", smem);
-  const long long blocks = (long long)p.B * p.num_tiles * p.H;
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "backward: grid too large");
-  {
-    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_BWD_MAIN, st);
-    kern<<<(unsigned)blocks, kNT, smem, st>>>(p);
-    ++g_launches;
-  }
-  return check_launch("msda_b200_backward (sorted)");
-}
-
-// Backward v3 (msda_bwd_mma.cuh): group-sorted rows + mma.sync; same geometry as v2, fp32 accumulator only.
-constexpr int kMmaNT = 256, kMmaTQ = 128, kMmaGCAP = 256, kMmaRCAP = 1024;
 
 template <typename AT, bool FUSED>
 int launch_bwd_mma(const msda_b200_desc* d, KParams p, cudaStream_t st) {
@@ -908,13 +883,8 @@ int launch_bwd_mma(const msda_b200_desc* d, KParams p, cudaStream_t st) {
 
 template <typename VT, typename AT, int ACC, bool FUSED>
 int dispatch_bwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
-  if constexpr (std::is_same<VT, __nv_bfloat16>::value && ACC != 2) {
-    if (sorted_applicable(d)) {
-      if constexpr (ACC == 0) {
-        if (!(d->flags & MSDA_B200_FLAG_BWD_V2)) return launch_bwd_mma<AT, FUSED>(d, p, st);
-      }
-      return launch_bwd_sorted_cfg<VT, AT, ACC, FUSED, kSortNT, kSortTQ, 4>(d, p, st);
-    }
+  if constexpr (std::is_same<VT, __nv_bfloat16>::value && ACC == 0) {
+    if (mma_applicable(d)) return launch_bwd_mma<AT, FUSED>(d, p, st);
   }
   switch (d->D) {
     case 8: return launch_bwd<VT, AT, 8, ACC, FUSED>(d, p, st);
@@ -945,7 +915,6 @@ int run_backward(const msda_b200_desc* desc, KParams p, void* grad_value, void* 
                  bool have_tensors, cudaStream_t st) {
   const bool prof = (desc->flags & MSDA_B200_FLAG_PROFILE) != 0;
   const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
-  const bool bf16_atomics = vbf && (desc->flags & MSDA_B200_FLAG_BF16_ATOMICS);
   const size_t nvalue = (size_t)desc->B * desc->S * desc->H * desc->D;
   const size_t need = msda_b200_backward_workspace_bytes(desc);
   if (nvalue && !grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
@@ -966,8 +935,6 @@ int run_backward(const msda_b200_desc* desc, KParams p, void* grad_value, void* 
     p.grad_value_acc = acc;
     int rc;
     if (!vbf) rc = dispatch_bwd<float, float, 0, FUSED>(desc, p, st);
-    else if (bf16_atomics) rc = abf ? dispatch_bwd<__nv_bfloat16, __nv_bfloat16, 1, FUSED>(desc, p, st)
-                                    : dispatch_bwd<__nv_bfloat16, float, 1, FUSED>(desc, p, st);
     else rc = abf ? dispatch_bwd<__nv_bfloat16, __nv_bfloat16, 0, FUSED>(desc, p, st)
                   : dispatch_bwd<__nv_bfloat16, float, 0, FUSED>(desc, p, st);
     if (rc) return rc;
@@ -1063,7 +1030,7 @@ size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc) {
     if (validate(desc) || msda_b200_internal_det_workspace_bytes(desc, &bytes)) return 0;
     return bytes;
   }
-  if (desc->value_dtype == MSDA_B200_BF16 && !(desc->flags & MSDA_B200_FLAG_BF16_ATOMICS))
+  if (desc->value_dtype == MSDA_B200_BF16)
     return (size_t)desc->B * desc->S * desc->H * desc->D * sizeof(float);
   return 0;
 }

@@ -1,19 +1,21 @@
 // msda_bwd_mma.cuh -- backward v3: pixel-GROUP-sorted accumulation with warp-level tensor-core products.
-// Included by msda_b200.cu inside its anonymous namespace (after msda_bwd_sorted.cuh: uses Log2P, gdec, MI_*).
+// Included by msda_b200.cu inside its anonymous namespace (uses KParams, Level, Axis, Vec16, red_add_f32x4).
 //
-// Why: v2 (msda_bwd_sorted.cuh) sorts the 4 corner contributions of every sample by pixel and walks the list with
-// CUDA cores; its pull loop is bound by instruction issue (~9-13 warp instructions per contribution, half of them
-// the divergent run-boundary code).  Once contributions are grouped by target pixels the work IS two small matrix
-// products, so v3 groups SAMPLES by aligned 4x2-pixel groups (8 "slots") and lets mma.sync.m16n8k16 (bf16 in, fp32
-// accumulate) do both products for 16 list rows at a time:
+// Why: v1 issues one fp32 reduction per bilinear corner and is bound by L2 reduction throughput.  v2 (a pixel-sorted
+// CUDA-core pull, in git at commit 71afd7d) sorted the 4 corner contributions of every sample by pixel and was bound by
+// instruction issue (~9-13 warp instructions per contribution, half of them the divergent run-boundary code).  Once
+// contributions are grouped by target pixels the work IS two small matrix products, so v3 groups SAMPLES by aligned
+// 4x2-pixel groups (8 "slots") and lets mma.sync.m16n8k16 (bf16 in, fp32 accumulate) do both products for 16 list
+// rows at a time:
 //
 //   dots   D2[row, slot]   = sum_ch  GO[row, ch] * V[slot, ch]        (-> grad_attn / grad_loc, exact bf16 products)
 //   scatter GV[ch, slot]  += sum_row GO[row, ch] * Wt[row, slot]      (-> grad_value; Wt = attn * bilinear weight of
 //                                                                      the sample's corner that falls on the slot)
 //
 //   per thread block = (batch, head, tile of TQ queries), per level:
-//     a  sample descriptors + bounding box                                   (as v2)
-//     b  window of 4x2 pixel groups (<= GCAP groups; samples outside take the v1 route, as v2)
+//     a  sample descriptors (slot weights, derivative codes, clamped base pixel) + bounding box of the touched pixels
+//     b  window of 4x2 pixel groups (<= GCAP groups, around the mean position if the box is larger; samples outside
+//        take the v1 route)
 //     c  histogram of (sample, group) rows: a sample's 2x2 footprint meets 1, 2 or 4 groups (1.9 on average,
 //        against 4 corner entries in v2)
 //     d  one-counter-per-thread scan -> segment starts + a table of work items (group, <= 64 rows)
@@ -23,7 +25,7 @@
 //        the 16x8 dots go to shared memory per (sample, corner); one red.global.add.v4.f32 per lane and slot at the
 //        end of the item
 //     g  fallback contributions: direct reductions (v1 route)
-//     h  per-sample gradients from the four dots                              (as v2)
+//     h  one thread per sample folds its four dots into grad_attn / grad_loc
 //
 // grad_out rows are staged ONCE per block with their 32 channels permuted so that (i) the m16n8k16 fragments of both
 // products come straight out of ldmatrix and (ii) every lane ends up holding 4 consecutive channels of a slot, i.e.
@@ -97,7 +99,18 @@ __host__ __device__ inline MmaSmem mma_smem_layout() {
   return s;
 }
 
-enum { MI_NITEMS = 9 };  // next to MI_TOTAL (msda_bwd_sorted.cuh); MI_WSUM = 16 holds the per-warp scan totals
+template <int P>
+struct Log2P;
+template <> struct Log2P<1> { static constexpr int v = 0; };
+template <> struct Log2P<2> { static constexpr int v = 1; };
+template <> struct Log2P<4> { static constexpr int v = 2; };
+template <> struct Log2P<8> { static constexpr int v = 3; };
+
+// misc slots; MI_WSUM = 16 holds the per-warp scan totals
+enum { MI_MINX = 0, MI_MAXX, MI_MINY, MI_MAXY, MI_SUMX, MI_SUMY, MI_NACT, MI_FBN, MI_TOTAL, MI_NITEMS, MI_WSUM = 16 };
+
+// derivative code k of a sample's packed codes (2 bits each, value + 1) -> d(slot weight)/d(pixel coord)
+__device__ __forceinline__ float gdec(int code, int k) { return (float)(((code >> (2 * k)) & 3) - 1); }
 
 template <typename AT, int NT, int TQ, int P, int GCAP, int RCAP, bool FUSED>
 __global__ void __launch_bounds__(NT, 4) msda_bwd_mma_kernel(const __grid_constant__ KParams p) {

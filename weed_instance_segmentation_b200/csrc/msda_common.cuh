@@ -1,6 +1,5 @@
-// msda_common.cuh -- structs and device helpers shared by the kernels of msda_b200.cu, msda_bwd_sorted.cuh and
-// msda_bwd_mma.cuh. Included INSIDE msda_b200.cu's anonymous namespace (after <cuda_bf16.h>, <cuda_runtime.h> and
-// msda_b200.h).
+// msda_common.cuh -- structs and device helpers shared by the kernels of msda_b200.cu and msda_bwd_mma.cuh.
+// Included INSIDE msda_b200.cu's anonymous namespace (after <cuda_bf16.h>, <cuda_runtime.h> and msda_b200.h).
 #pragma once
 
 constexpr int kMaxL = MSDA_B200_MAX_LEVELS;
@@ -18,7 +17,7 @@ struct KParams {
   const void* attn;
   void* out;             // forward
   const void* grad_out;  // backward
-  void* grad_value_acc;  // backward: fp32 accumulator (grad_value itself for fp32) or bf16 grad_value
+  void* grad_value_acc;  // backward: fp32 accumulator (grad_value itself for fp32 values, the workspace for bf16)
   float* grad_loc;
   void* grad_attn;
   const int* q_order;
@@ -150,10 +149,5 @@ __device__ __forceinline__ void fma2_pair(float& a0, float& a1, float g0, float 
 // red.global.add.v4.f32 (sm_90+): one 16-byte reduction, no return value.
 __device__ __forceinline__ void red_add_f32x4(float* addr, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d)
-               : "memory");
-}
-// red.global.add.noftz.v4.bf16x2 (sm_90+): eight bf16 lanes in one 16-byte reduction.
-__device__ __forceinline__ void red_add_bf16x8(void* addr, unsigned a, unsigned b, unsigned c, unsigned d) {
-  asm volatile("red.global.add.noftz.v4.bf16x2 [%0], {%1, %2, %3, %4};" ::"l"(addr), "r"(a), "r"(b), "r"(c), "r"(d)
                : "memory");
 }

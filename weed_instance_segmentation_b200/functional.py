@@ -34,14 +34,16 @@ def _parse_tile(text):
     return (parts[0], parts[0]) if len(parts) == 1 else (parts[0], parts[1])
 
 
-# 2-D query tile (rows x cols) of the query order. The pixel-sorted backward (csrc/msda_bwd_sorted.cuh) owns 128
-# queries per block; an 8 x 16 patch keeps their samples inside a small pixel window, which is what lets it merge
+# 2-D query tile (rows x cols) of the query order. The group-sorted backward (csrc/msda_bwd_mma.cuh, kMmaTQ) owns
+# 128 queries per block; an 8 x 16 patch keeps their samples inside a small pixel window, which is what lets it merge
 # contributions before reducing. The forward does not care (measured: LSU-bound either way, profiles/r01_notes.md).
 _TILE = _parse_tile(os.environ.get("MSDA_B200_TILE", "8x16"))
 _USE_ORDER = os.environ.get("MSDA_B200_QUERY_ORDER", "1") != "0"
-_BF16_ATOMICS = os.environ.get("MSDA_B200_BF16_ATOMICS", "0") == "1"
+# Backward: the per-corner kernel (v1) everywhere instead of the group-sorted one; the reference the GPU tests use.
 _BWD_V1 = os.environ.get("MSDA_B200_BWD_V1", "0") == "1"
-_BWD_V2 = os.environ.get("MSDA_B200_BWD_V2", "0") == "1"  # CUDA-core pixel-sorted backward instead of the tensor-core one
+# Retired selections, always off; bench.py still reads the names.
+_BF16_ATOMICS = False
+_BWD_V2 = False
 # Forward: never multiply a zero-weight corner (exact zeros padding even when `value` holds NaN / Inf in pixels no
 # sample reads; 25-30 % slower, see include/msda_b200.h MSDA_B200_FLAG_STRICT_PADDING).
 _STRICT_PADDING = os.environ.get("MSDA_B200_STRICT_PADDING", "0") == "1"
@@ -54,12 +56,19 @@ def deterministic() -> bool:
     """Whether the package computes gradients reproducibly: ``torch.use_deterministic_algorithms(True)`` is the switch.
 
     Read at each backward (``HostPipeline`` reads it once, when it is built). When it is on, the op's backward runs
-    with ``FLAG_DETERMINISTIC`` (bit-identical gradients for identical inputs; the ``MSDA_B200_BWD_*`` and
-    ``MSDA_B200_BF16_ATOMICS`` selections are ignored), and the modules leave the B200 kernels whose backward reduces
-    with float atomics or atomic split-K (fused LayerNorm, bias-gradient column sums, the emulated float32 GEMMs, the
-    GroupNorm input assembly) for the torch path they otherwise fall back to.
+    with ``FLAG_DETERMINISTIC`` (bit-identical gradients for identical inputs; ``MSDA_B200_BWD_V1`` is ignored), and
+    the modules leave the B200 kernels whose backward reduces with float atomics or atomic split-K (fused LayerNorm,
+    bias-gradient column sums, the emulated float32 GEMMs, the GroupNorm input assembly) for the torch path they
+    otherwise fall back to.
     """
     return torch.are_deterministic_algorithms_enabled()
+
+
+def _backward_flags(deterministic: bool) -> int:
+    """Backward-kernel flags of the op, its fused form and ``HostPipeline``."""
+    if deterministic:
+        return _cabi.FLAG_DETERMINISTIC
+    return _cabi.FLAG_BWD_V1 if _BWD_V1 else 0
 
 
 def _shapes_list(value_spatial_shapes) -> list[tuple[int, int]]:
@@ -194,15 +203,7 @@ class MSDeformAttnFunction(torch.autograd.Function):
         B, S, H, D = value.shape
         _, Q, _, L, P, _ = loc.shape
         grad_out = grad_out.to(value.dtype).contiguous()
-        if deterministic():
-            flags |= _cabi.FLAG_DETERMINISTIC
-        else:
-            if _BF16_ATOMICS and value.dtype == torch.bfloat16:
-                flags |= _cabi.FLAG_BF16_ATOMICS
-            if _BWD_V1:
-                flags |= _cabi.FLAG_BWD_V1
-            if _BWD_V2:
-                flags |= _cabi.FLAG_BWD_V2
+        flags |= _backward_flags(deterministic())
         desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value.dtype], _DTYPE_CODE[attn.dtype],
                                      shapes, level_start, flags)
         grad_value = torch.empty_like(value)

@@ -70,14 +70,7 @@ class MSDeformAttnFusedFunction(torch.autograd.Function):
         shapes, level_start, (off_dtype, logit_dtype) = ctx.geom
         B, S, H, D = value.shape
         _, Q, _, L, P, _ = offsets.shape
-        flags = 0
-        if F.deterministic():
-            flags |= _cabi.FLAG_DETERMINISTIC
-        else:
-            if F._BF16_ATOMICS and value.dtype == torch.bfloat16:
-                flags |= _cabi.FLAG_BF16_ATOMICS
-            if F._BWD_V1:
-                flags |= _cabi.FLAG_BWD_V1
+        flags = F._backward_flags(F.deterministic())
         desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value.dtype], _DTYPE_CODE[offsets.dtype],
                                      shapes, level_start, flags)
         grad_out = grad_out.to(value.dtype).contiguous()

@@ -46,14 +46,7 @@ class HostPipeline:
             raise TypeError("HostPipeline: float32 or bfloat16 tensors only")
         self.backward = bool(backward)
         self.deterministic = functional.deterministic() if deterministic is None else bool(deterministic)
-        flags = 0
-        if self.deterministic:
-            flags |= _cabi.FLAG_DETERMINISTIC
-        else:
-            if functional._BF16_ATOMICS and value_dtype == torch.bfloat16:
-                flags |= _cabi.FLAG_BF16_ATOMICS
-            if functional._BWD_V1:
-                flags |= _cabi.FLAG_BWD_V1
+        flags = functional._backward_flags(self.deterministic)
         lsi = functional._level_start(self.shapes, None)
         desc, self._keep = _cabi.make_desc(self.B, self.S, self.Q, self.H, self.D, self.L, self.P,
                                            _DTYPE_CODE[self.value_dtype], _DTYPE_CODE[self.attn_dtype], self.shapes, lsi,
