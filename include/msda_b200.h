@@ -284,6 +284,40 @@ int msda_b200_point_sample_backward(float* const* grad_planes /*dev, R*/, const 
                                     int32_t K, void* stream);
 
 /*
+ * Deterministic form of msda_b200_point_sample_backward: bit-identical grad_planes for bit-identical inputs, whatever
+ * the stream or the order of the rows among different planes.  Same contract otherwise: it adds into zero-filled float32
+ * planes, NULL entries of grad_planes are skipped, corners outside the plane or with a NaN coordinate add nothing.
+ *   key_base[r] (dev, R int64)  destination keys of row r's plane: pixel y*w + x of it has the key key_base[r] + y*w + x.
+ *                               The caller numbers every pixel of every distinct gradient plane with one key in
+ *                               [0, keys): rows that write into the same plane have the same key_base, distinct planes
+ *                               have disjoint ranges [key_base, key_base + h*w).  A key outside [0, keys) adds nothing.
+ *   keys                        the number of keys.
+ * Each (row, point) writes four records, one per bilinear corner, at index 4*(r*K + k) + corner: a uint32 key and a
+ * uint64 payload (r << 32 | float32 bits of grad_out[r, k] * wx * wy -- the value the atomic form adds).  A stable
+ * radix sort over ceil(log2(keys + 1)) bits groups them by pixel in (row, point, corner) order; the thread at the start
+ * of each run sums it in fp32 in that order and adds the sum to its pixel once.  No float atomics.
+ * Workspace (device, at least ..._workspace_bytes(R, K, keys), 256-byte aligned): 24 bytes per record (key + payload,
+ * double-buffered for the sort) and the sort's scratch.  More than 2^31 - 1 records (4*R*K) or keys >= 2^32 - 1 is
+ * MSDA_B200_ERR_UNSUPPORTED.  The workspace size is 0 for invalid or unsupported arguments.
+ */
+size_t msda_b200_point_sample_backward_det_workspace_bytes(int64_t R, int32_t K, int64_t keys);
+int msda_b200_point_sample_backward_det(float* const* grad_planes /*dev, R*/, const msda_b200_ps_row* rows /*dev, R*/,
+                                        const int64_t* key_base /*dev, R*/, int64_t keys, const float* coords /*dev*/,
+                                        const float* grad_out /*dev, (R,K)*/, int64_t R, int32_t K,
+                                        void* workspace /*dev*/, size_t workspace_bytes, void* stream);
+
+/*
+ * Backward of bilinear resizing, F.interpolate(x, size=(Ho, Wo), mode="bilinear", align_corners=False) without a scale
+ * factor (the pixel decoder's FPN upsampling, M2F:1360-1371), for NC contiguous float32 planes:
+ *   grad_in (NC, Hi, Wi) = adjoint of the resize applied to grad_out (NC, Ho, Wo),
+ * with ATen's index arithmetic (scale = (float)in / out, src = max(scale * (dst + 0.5) - 0.5, 0), i0 = (int)src,
+ * i1 = i0 + (i0 < in - 1)).  A gather: every grad_in element is written once (no zero-fill needed) with the sum of the
+ * output pixels that read it, in a fixed order, in fp32 -- bit-identical results for bit-identical inputs.
+ */
+int msda_b200_resize_bilinear_backward(const float* grad_out /*dev*/, float* grad_in /*dev*/, int64_t NC, int32_t Hi,
+                                       int32_t Wi, int32_t Ho, int32_t Wo, void* stream);
+
+/*
  * Pixel-decoder input assembly (SURVEY.md section 8(f) rank 3; M2F:1301-1313): GroupNorm of a 1x1-conv output
  * x (B, C, HW; NCHW with the spatial dims flattened; float32 or bfloat16) fused with the flatten / transpose / concat
  * that feeds the encoder:   out[b, p, c] = (x[b, c, p] - mean[b, g]) * rstd[b, g] * gamma[c] + beta[c],   g = c / (C/G),

@@ -48,6 +48,9 @@ EXPORTS = (
     "msda_b200_groupnorm_to_rows_backward",
     "msda_b200_point_sample_forward",
     "msda_b200_point_sample_backward",
+    "msda_b200_point_sample_backward_det_workspace_bytes",
+    "msda_b200_point_sample_backward_det",
+    "msda_b200_resize_bilinear_backward",
     "msda_b200_host_pipeline_create",
     "msda_b200_host_pipeline_step",
     "msda_b200_host_pipeline_join",
@@ -146,6 +149,14 @@ def load() -> ctypes.CDLL:
     lib.msda_b200_point_sample_forward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
     lib.msda_b200_point_sample_backward.restype = ctypes.c_int
     lib.msda_b200_point_sample_backward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
+    lib.msda_b200_point_sample_backward_det_workspace_bytes.restype = ctypes.c_size_t
+    lib.msda_b200_point_sample_backward_det_workspace_bytes.argtypes = [ctypes.c_int64, ctypes.c_int32, ctypes.c_int64]
+    lib.msda_b200_point_sample_backward_det.restype = ctypes.c_int
+    lib.msda_b200_point_sample_backward_det.argtypes = [vp, vp, vp, ctypes.c_int64, vp, vp, ctypes.c_int64, ctypes.c_int32,
+                                                        vp, ctypes.c_size_t, vp]
+    lib.msda_b200_resize_bilinear_backward.restype = ctypes.c_int
+    lib.msda_b200_resize_bilinear_backward.argtypes = [vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
+                                                       ctypes.c_int32, ctypes.c_int32, vp]
     lib.msda_b200_host_pipeline_create.restype = ctypes.c_int
     lib.msda_b200_host_pipeline_create.argtypes = [dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp,
                                                    ctypes.POINTER(vp)]

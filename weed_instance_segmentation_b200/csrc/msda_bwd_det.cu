@@ -78,16 +78,6 @@ int check_supported(const DetLayout& lay) {
   return MSDA_B200_OK;
 }
 
-int sort_bytes(const DetLayout& lay, size_t* bytes, cudaStream_t st) {
-  *bytes = 0;
-  if (lay.records == 0) return MSDA_B200_OK;
-  cub::DoubleBuffer<unsigned> kb(nullptr, nullptr);
-  cub::DoubleBuffer<unsigned long long> vb(nullptr, nullptr);
-  const cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, *bytes, kb, vb, (int)lay.records, 0, lay.key_bits, st);
-  if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
-  return MSDA_B200_OK;
-}
-
 template <typename VT, int D>
 int launch_pull(const DetLayout& lay, const msda_b200_desc* d, const uint2* ranges, const unsigned long long* vals,
                 const void* grad_out, void* grad_value, cudaStream_t st) {
@@ -116,13 +106,41 @@ int dispatch_pull(const DetLayout& lay, const msda_b200_desc* d, const uint2* ra
 
 }  // namespace
 
+extern "C" int msda_b200_internal_det_sort_bytes(const DetLayout* lay, size_t* bytes) {
+  *bytes = 0;
+  if (lay->records == 0) return MSDA_B200_OK;
+  cub::DoubleBuffer<unsigned> kb(nullptr, nullptr);
+  cub::DoubleBuffer<unsigned long long> vb(nullptr, nullptr);
+  const cudaError_t e =
+      cub::DeviceRadixSort::SortPairs(nullptr, *bytes, kb, vb, (int)lay->records, 0, lay->key_bits, (cudaStream_t)0);
+  return e == cudaSuccess ? MSDA_B200_OK : fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+}
+
+extern "C" int msda_b200_internal_det_sort(const DetLayout* lay, void* workspace, const unsigned** keys,
+                                           const unsigned long long** vals, cudaStream_t st) {
+  char* ws = static_cast<char*>(workspace);
+  cub::DoubleBuffer<unsigned> kb(reinterpret_cast<unsigned*>(ws + lay->keys_off[0]),
+                                 reinterpret_cast<unsigned*>(ws + lay->keys_off[1]));
+  cub::DoubleBuffer<unsigned long long> vb(reinterpret_cast<unsigned long long*>(ws + lay->vals_off[0]),
+                                           reinterpret_cast<unsigned long long*>(ws + lay->vals_off[1]));
+  size_t sort = 0;
+  if (int rc = msda_b200_internal_det_sort_bytes(lay, &sort)) return rc;
+  const cudaError_t e =
+      cub::DeviceRadixSort::SortPairs(ws + lay->sort_off, sort, kb, vb, (int)lay->records, 0, lay->key_bits, st);
+  if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  msda_b200_internal_count_launch();  // the sort's kernels count as one launch
+  *keys = kb.Current();
+  *vals = vb.Current();
+  return MSDA_B200_OK;
+}
+
 // Workspace of the deterministic backward for a validated descriptor: the records, the bucket ranges and the sort's
 // scratch as CUB reports it (which reads the current device's attributes).
 extern "C" int msda_b200_internal_det_workspace_bytes(const msda_b200_desc* desc, size_t* bytes) {
   const DetLayout lay = det_layout(desc);
   if (int rc = check_supported(lay)) return rc;
   size_t sort = 0;
-  if (int rc = sort_bytes(lay, &sort, nullptr)) return rc;
+  if (int rc = msda_b200_internal_det_sort_bytes(&lay, &sort)) return rc;
   *bytes = lay.sort_off + sort;
   return MSDA_B200_OK;
 }
@@ -139,20 +157,12 @@ extern "C" int msda_b200_internal_det_grad_value(const msda_b200_desc* desc, con
   cudaError_t e = cudaMemsetAsync(ranges, 0, (size_t)lay.keys * sizeof(uint2), st);
   if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
   if (lay.records) {
-    cub::DoubleBuffer<unsigned> kb(reinterpret_cast<unsigned*>(ws + lay.keys_off[0]),
-                                   reinterpret_cast<unsigned*>(ws + lay.keys_off[1]));
-    cub::DoubleBuffer<unsigned long long> vb(reinterpret_cast<unsigned long long*>(ws + lay.vals_off[0]),
-                                             reinterpret_cast<unsigned long long*>(ws + lay.vals_off[1]));
-    size_t sort = 0;
-    if (int rc = sort_bytes(lay, &sort, st)) return rc;
-    e = cub::DeviceRadixSort::SortPairs(ws + lay.sort_off, sort, kb, vb, (int)lay.records, 0, lay.key_bits, st);
-    if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
-    msda_b200_internal_count_launch();  // the sort's kernels count as one launch
+    const unsigned* keys = nullptr;
+    if (int rc = msda_b200_internal_det_sort(&lay, workspace, &keys, &vals, st)) return rc;
     const int n = (int)lay.records;
-    msda_bwd_det_ranges_kernel<<<(n + kDetNT - 1) / kDetNT, kDetNT, 0, st>>>(kb.Current(), n, (unsigned)lay.keys, ranges);
+    msda_bwd_det_ranges_kernel<<<(n + kDetNT - 1) / kDetNT, kDetNT, 0, st>>>(keys, n, (unsigned)lay.keys, ranges);
     msda_b200_internal_count_launch();
     if ((e = cudaGetLastError()) != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
-    vals = vb.Current();
   }
   if (desc->value_dtype == MSDA_B200_BF16)
     return dispatch_pull<__nv_bfloat16>(lay, desc, ranges, vals, grad_out, grad_value, st);

@@ -59,7 +59,11 @@ def deterministic() -> bool:
     with ``FLAG_DETERMINISTIC`` (bit-identical gradients for identical inputs; ``MSDA_B200_BWD_V1`` is ignored), and
     the modules leave the B200 kernels whose backward reduces with float atomics or atomic split-K (fused LayerNorm,
     bias-gradient column sums, the emulated float32 GEMMs, the GroupNorm input assembly) for the torch path they
-    otherwise fall back to.
+    otherwise fall back to. ``point_sample`` (the converted criterion's mask logits) runs its sort-ordered backward
+    (``msda_b200_point_sample_backward_det``), and the converted pixel decoder upsamples its FPN tail with
+    ``pixel_decoder.resize_bilinear``, whose gather backward has one writer per element (torch's raises under the
+    switch). With the model converted by ``train.use_b200_path(model)`` (``"modules"`` mode, criterion included), a
+    whole fine-tuning step then has bit-identical gradients run to run.
     """
     return torch.are_deterministic_algorithms_enabled()
 

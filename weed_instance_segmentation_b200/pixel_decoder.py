@@ -155,6 +155,44 @@ def assemble_encoder_inputs(decoder, features) -> dict:
             "valid_ratios": const["valid_ratios"]}
 
 
+class _ResizeBilinear(torch.autograd.Function):
+    """``F.interpolate(x, size, mode="bilinear", align_corners=False)`` with a deterministic backward."""
+
+    @staticmethod
+    def forward(ctx, x, size):
+        ctx.meta = (tuple(x.shape), x.dtype)
+        # ATen's kernel itself: under the switch F.interpolate would take torch's decomposition instead, whose values
+        # differ in the last bits from the kernel this backward is the adjoint of
+        return torch.ops.aten.upsample_bilinear2d(x, list(size), False)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        lib = _cabi.load()
+        (n, c, hi, wi), dtype = ctx.meta
+        go = grad_out.float().contiguous()  # the kernel is fp32; other dtypes round-trip through it
+        grad_in = torch.empty((n, c, hi, wi), dtype=torch.float32, device=go.device)
+        with torch.cuda.device(go.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.check(lib.msda_b200_resize_bilinear_backward(go.data_ptr() if go.numel() else None,
+                                                               grad_in.data_ptr() if grad_in.numel() else None, n * c,
+                                                               hi, wi, go.shape[2], go.shape[3], stream))
+        return grad_in.to(dtype), None
+
+
+def resize_bilinear(x: torch.Tensor, size) -> torch.Tensor:
+    """``F.interpolate(x, size=size, mode="bilinear", align_corners=False)`` for an NCHW CUDA tensor, whose backward is
+    ``csrc/resize_bilinear.cu``: a gather with one writer per input element, so the gradient is bit-identical run to run.
+    torch's CUDA backward of the kernel scatters with atomics; under ``torch.use_deterministic_algorithms(True)``
+    ``F.interpolate`` switches to a decomposition whose backward accumulates with ``index_put``, and whose forward values
+    differ in the last bits from the switch-off path. Here the forward is the same kernel with the switch on or off."""
+    if not x.is_cuda:
+        raise RuntimeError("resize_bilinear: tensors must live on a CUDA device (this package has no CPU fallback)")
+    if x.dim() != 4:
+        raise ValueError(f"resize_bilinear: x must be (N, C, H, W), got {tuple(x.shape)}")
+    return _ResizeBilinear.apply(x, tuple(int(v) for v in size))
+
+
 def pixel_decoder_forward(self, features, encoder_outputs=None, output_attentions=None, output_hidden_states=None,
                           return_dict=None):
     """``Mask2FormerPixelDecoder.forward`` (M2F:1287-1385) with the input assembly above."""
@@ -178,8 +216,11 @@ def pixel_decoder_forward(self, features, encoder_outputs=None, output_attention
     # M2F:1360-1371: extra FPN levels, low to high resolution
     for idx, feature in enumerate(features[: self.num_fpn_levels][::-1]):
         current_fpn = self.lateral_convolutions[idx](feature)
-        out = current_fpn + nn.functional.interpolate(outputs[-1], size=current_fpn.shape[-2:], mode="bilinear",
-                                                      align_corners=False)
+        if deterministic():  # a gather backward instead of torch's index_put-based one
+            up = resize_bilinear(outputs[-1], current_fpn.shape[-2:])
+        else:
+            up = nn.functional.interpolate(outputs[-1], size=current_fpn.shape[-2:], mode="bilinear", align_corners=False)
+        out = current_fpn + up
         outputs.append(self.output_convolutions[idx](out))
     multi_scale_features = tuple(outputs[: self.num_feature_levels])  # M2F:1373-1379
     return Mask2FormerPixelDecoderOutput(mask_features=self.mask_projection(outputs[-1]),

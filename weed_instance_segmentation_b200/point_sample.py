@@ -7,7 +7,9 @@ the original tensors and a per-row address instead::
     out[r, k] = bilinear(sources[src_id[r]][plane_id[r]], coords[coord_row[r], k])        # (R, K) float32
 
 with ``grid_sample``'s conventions (bilinear, zeros padding, ``align_corners=False``, coordinates in [0, 1] as (x, y)).
-Gradients flow to the sources that require them (scatter with fp32 atomics); coordinates carry none.
+Gradients flow to the sources that require them (scatter with fp32 atomics; under
+``torch.use_deterministic_algorithms(True)`` a sort by destination pixel and ordered fp32 sums instead, so they are
+bit-identical run to run); coordinates carry none.
 CUDA only: ``csrc/point_sample.cu`` through the C ABI, no CPU path.
 """
 from __future__ import annotations
@@ -18,6 +20,7 @@ import numpy as np
 import torch
 
 from . import _cabi
+from .functional import deterministic
 
 _DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16, torch.uint8: _cabi.U8, torch.bool: _cabi.U8}
 
@@ -48,7 +51,8 @@ class _Rows:
         rows = np.stack([self.h[src_id], self.w[src_id], coord_row, code[src_id]], axis=1).astype(np.int32)
         self.device = device
         self.ptr = torch.from_numpy(ptr).to(device, non_blocking=True)
-        self.rows = torch.from_numpy(np.ascontiguousarray(rows)).to(device, non_blocking=True)
+        self.rows_host = np.ascontiguousarray(rows)
+        self.rows = torch.from_numpy(self.rows_host).to(device, non_blocking=True)
         self.max_coord_row = int(coord_row.max()) if self.R else -1
 
     def grad_pointers(self, grads: Sequence[torch.Tensor | None]) -> torch.Tensor:
@@ -56,6 +60,22 @@ class _Rows:
         live = base[self.src_id] != 0
         ptr = np.where(live, base[self.src_id] + self.plane_id * (self.h * self.w * 4)[self.src_id], 0)
         return torch.from_numpy(ptr).to(self.device, non_blocking=True)
+
+    def det_tables(self, grads: Sequence[torch.Tensor | None]):
+        """Tables of the deterministic backward: the rows whose source has a gradient (``live``, host indices), their
+        gradient-plane pointers, rows and destination keys (``key_base`` per row and the key count, see
+        ``msda_b200_point_sample_backward_det``). Every distinct (source, plane) gets its own key range."""
+        has = np.array([g is not None for g in grads])
+        live = np.nonzero(has[self.src_id])[0]
+        src, plane = self.src_id[live], self.plane_id[live]
+        pairs, inverse = np.unique(np.stack([src, plane], axis=1), axis=0, return_inverse=True)
+        size = (self.h * self.w)[pairs[:, 0]]
+        start = np.concatenate([[0], np.cumsum(size)[:-1]]).astype(np.int64)
+        key_base = start[inverse.reshape(-1)]
+        base = np.array([g.data_ptr() if g is not None else 0 for g in grads], dtype=np.int64)
+        ptr = base[src] + plane * (self.h * self.w * 4)[src]
+        to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(self.device, non_blocking=True)
+        return live, to_dev(ptr), to_dev(self.rows_host[live]), to_dev(key_base), int(size.sum())
 
 
 class PointSampleFunction(torch.autograd.Function):
@@ -91,13 +111,32 @@ class PointSampleFunction(torch.autograd.Function):
                  for (shape, _), need in zip(ctx.src_meta, needs)]
         if table.R and K and any(needs):
             go = grad_out.float().contiguous()
-            gptr = table.grad_pointers(grads)
             with torch.cuda.device(coords.device):
                 stream = torch.cuda.current_stream().cuda_stream
-                _cabi.check(lib.msda_b200_point_sample_backward(gptr.data_ptr(), table.rows.data_ptr(), coords.data_ptr(),
-                                                                go.data_ptr(), table.R, K, stream))
+                if deterministic():
+                    _backward_det(lib, table, grads, coords, go, K, stream)
+                else:
+                    gptr = table.grad_pointers(grads)
+                    _cabi.check(lib.msda_b200_point_sample_backward(gptr.data_ptr(), table.rows.data_ptr(),
+                                                                    coords.data_ptr(), go.data_ptr(), table.R, K, stream))
         outs = [g.to(dt) if g is not None else None for g, (_, dt) in zip(grads, ctx.src_meta)]
         return (None, None, *outs)
+
+
+def _backward_det(lib, table: _Rows, grads, coords, go, K, stream) -> None:
+    """``msda_b200_point_sample_backward_det`` over the rows that need a gradient (the criterion's target rows need
+    none, so compacting halves its sort)."""
+    live, gptr, rows, key_base, keys = table.det_tables(grads)
+    R = int(live.shape[0])
+    if R == 0:
+        return
+    if R != table.R:
+        go = go.index_select(0, torch.from_numpy(live).to(go.device, non_blocking=True))
+    nbytes = lib.msda_b200_point_sample_backward_det_workspace_bytes(R, K, keys)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=go.device) if nbytes else None  # 0: the call reports why
+    _cabi.check(lib.msda_b200_point_sample_backward_det(gptr.data_ptr(), rows.data_ptr(), key_base.data_ptr(), keys,
+                                                        coords.data_ptr(), go.data_ptr(), R, K,
+                                                        ws.data_ptr() if nbytes else None, nbytes, stream))
 
 
 def point_sample(sources: Sequence[torch.Tensor], src_id, plane_id, coords: torch.Tensor, coord_row) -> torch.Tensor:

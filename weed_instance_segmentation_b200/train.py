@@ -324,7 +324,13 @@ def main(argv=None):
     ap.add_argument("--infer", action="store_true",
                     help="inference replicas instead of training (the reference's run_inference call shape, "
                          "/root/reference/models/mask2former/inference.py:25-30): eval(), no_grad, no collective")
+    ap.add_argument("--deterministic", action="store_true",
+                    help="torch.use_deterministic_algorithms(True): bit-identical gradients run to run (with --impl b200, "
+                         "which converts the criterion); sets CUBLAS_WORKSPACE_CONFIG=:4096:8 unless it is set")
     args = ap.parse_args(argv)
+    if args.deterministic:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # read by cuBLAS when its first handle is made
+        torch.use_deterministic_algorithms(True)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
