@@ -318,6 +318,43 @@ int msda_b200_resize_bilinear_backward(const float* grad_out /*dev*/, float* gra
                                        int32_t Wi, int32_t Ho, int32_t Wo, void* stream);
 
 /*
+ * Instance post-processing (csrc/postprocess.cu): the mask side of Mask2FormerImageProcessor.
+ * post_process_instance_segmentation (transformers 5.5.0, image_processing_mask2former.py:605-724) for a whole batch,
+ * with no host round trip.  The caller keeps the class side in torch (softmax, per-image topk(Q, sorted=False) over the
+ * Q*C (query, class) scores, the label gather, pred_score = topk score * mask_score).
+ *   mask_logits (dev)  (B, Q, h, w) of `dtype` (MSDA_B200_F32 | MSDA_B200_BF16), contiguous
+ *   topk_index  (dev)  (B, Q) int64: selection j of image b picks query topk_index[b, j] / C (an index outside
+ *                      [0, Q*C) selects an empty mask)
+ *   target_hw   (dev)  (B, 2) int32 (H_i, W_i) > 0; (384, 384) for every image reproduces target_sizes=None
+ *   maps        (dev)  sum_i H_i*W_i float32: image i's (H_i, W_i) map follows image i-1's
+ *   table       (dev)  (B, Q, 3) int32: float32 bits of pred_score, label, segment id (-1 = not kept)
+ * scores: upsamples each selected plane to 384 x 384 with ATen's bilinear arithmetic (bf16: rounded to bf16), masks
+ *   it at logit > 0, writes mask_score (dev, (B, Q) float32) = sum(sigmoid * mask) / (sum(mask) + 1e-6), both sums in
+ *   fp32 in a fixed order (bf16: sigmoid rounded to bf16 first), and keeps in the workspace the mask bit-packed (18 KB
+ *   per selection) and whether it is non-empty after ATen's nearest resize to (H_i, W_i).
+ * paint: a selection is kept when it is non-empty there and (double)pred_score >= threshold; kept selections get ids
+ *   0, 1, ... in selection order; each target pixel gets the id of the last kept selection whose resized mask covers
+ *   it, else -1.  pred_score (dev, (B, Q) float32) and labels (dev, (B, Q) int64) are copied into the table.  max_h
+ *   (host) >= every H_i.  Run it after scores, on the same workspace.
+ * binary_maps: (n_inst, H, W) float32 0/1 maps of image `image`'s kept selections, in id order, from the table paint
+ *   wrote (n_inst = its kept count, H, W = its target size).
+ * Workspace (dev, at least _workspace_bytes(B, Q, C)): B*Q*(18432 + 4) bytes.  B <= 65535, Q <= 1024 and Q*C <= 2^31-1,
+ * else MSDA_B200_ERR_UNSUPPORTED; the workspace size is 0 for invalid or unsupported arguments.  No float atomics:
+ * bit-identical results for bit-identical inputs, whatever the stream.
+ */
+size_t msda_b200_postprocess_workspace_bytes(int32_t B, int32_t Q, int32_t C);
+int msda_b200_postprocess_scores(const void* mask_logits /*dev*/, int32_t dtype, const int64_t* topk_index /*dev*/,
+                                 int32_t C, const int32_t* target_hw /*dev*/, int32_t B, int32_t Q, int32_t h, int32_t w,
+                                 float* mask_score /*dev*/, void* workspace /*dev*/, size_t workspace_bytes, void* stream);
+int msda_b200_postprocess_paint(const void* workspace /*dev*/, size_t workspace_bytes, const float* pred_score /*dev*/,
+                                const int64_t* labels /*dev*/, double threshold, const int32_t* target_hw /*dev*/,
+                                int32_t B, int32_t Q, int32_t max_h, float* maps /*dev*/, int32_t* table /*dev*/,
+                                void* stream);
+int msda_b200_postprocess_binary_maps(const void* workspace /*dev*/, size_t workspace_bytes, const int32_t* table /*dev*/,
+                                      int32_t B, int32_t Q, int32_t image, int32_t H, int32_t W, int32_t n_inst,
+                                      float* out /*dev*/, void* stream);
+
+/*
  * Pixel-decoder input assembly (SURVEY.md section 8(f) rank 3; M2F:1301-1313): GroupNorm of a 1x1-conv output
  * x (B, C, HW; NCHW with the spatial dims flattened; float32 or bfloat16) fused with the flatten / transpose / concat
  * that feeds the encoder:   out[b, p, c] = (x[b, c, p] - mean[b, g]) * rstd[b, g] * gamma[c] + beta[c],   g = c / (C/G),

@@ -18,6 +18,7 @@ from .host import HostPipeline  # noqa: F401
 from .pixel_decoder import convert_pixel_decoder_inputs, groupnorm_to_rows  # noqa: F401
 from .point_sample import point_sample  # noqa: F401
 from .hf_patch import install, installed, is_installed, uninstall  # noqa: F401
+from .postprocess import post_process_instance_segmentation  # noqa: F401
 
 __all__ = [
     "HostPipeline",
@@ -36,4 +37,5 @@ __all__ = [
     "installed",
     "is_installed",
     "uninstall",
+    "post_process_instance_segmentation",
 ]

@@ -51,6 +51,10 @@ EXPORTS = (
     "msda_b200_point_sample_backward_det_workspace_bytes",
     "msda_b200_point_sample_backward_det",
     "msda_b200_resize_bilinear_backward",
+    "msda_b200_postprocess_workspace_bytes",
+    "msda_b200_postprocess_scores",
+    "msda_b200_postprocess_paint",
+    "msda_b200_postprocess_binary_maps",
     "msda_b200_host_pipeline_create",
     "msda_b200_host_pipeline_step",
     "msda_b200_host_pipeline_join",
@@ -157,6 +161,16 @@ def load() -> ctypes.CDLL:
     lib.msda_b200_resize_bilinear_backward.restype = ctypes.c_int
     lib.msda_b200_resize_bilinear_backward.argtypes = [vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
                                                        ctypes.c_int32, ctypes.c_int32, vp]
+    i32 = ctypes.c_int32
+    lib.msda_b200_postprocess_workspace_bytes.restype = ctypes.c_size_t
+    lib.msda_b200_postprocess_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.msda_b200_postprocess_scores.restype = ctypes.c_int
+    lib.msda_b200_postprocess_scores.argtypes = [vp, i32, vp, i32, vp, i32, i32, i32, i32, vp, vp, ctypes.c_size_t, vp]
+    lib.msda_b200_postprocess_paint.restype = ctypes.c_int
+    lib.msda_b200_postprocess_paint.argtypes = [vp, ctypes.c_size_t, vp, vp, ctypes.c_double, vp, i32, i32, i32, vp, vp,
+                                                vp]
+    lib.msda_b200_postprocess_binary_maps.restype = ctypes.c_int
+    lib.msda_b200_postprocess_binary_maps.argtypes = [vp, ctypes.c_size_t, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     lib.msda_b200_host_pipeline_create.restype = ctypes.c_int
     lib.msda_b200_host_pipeline_create.argtypes = [dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp,
                                                    ctypes.POINTER(vp)]

@@ -6,15 +6,14 @@
 // and writes the element once -- no zero-fill, no atomics. Zero weights are not skipped, so a non-finite grad_out
 // value reaches the same grad_in elements as in torch.
 //
-// Index arithmetic of ATen's upsample_bilinear2d (area_pixel_compute_scale / area_pixel_compute_source_index):
-//   scale = (float)in / out,  src = max(scale * (dst + 0.5) - 0.5, 0),  i0 = (int)src,  i1 = i0 + (i0 < in - 1),
-//   l1 = src - i0,  l0 = 1 - l1.
+// Index arithmetic of ATen's upsample_bilinear2d: bilinear_index.cuh.
 // i0 is non-decreasing in dst, so the outputs that read input index i (i0 == i or i1 == i, i.e. i0 in {i - 1, i}) are
-// one contiguous range; it is estimated from the inverse map with a margin and then settled with the formula above.
+// one contiguous range; it is estimated from the inverse map with a margin and then settled with that arithmetic.
 #include <cuda_runtime.h>
 
 #include <cstdint>
 
+#include "bilinear_index.cuh"
 #include "msda_b200.h"
 
 extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
@@ -24,23 +23,8 @@ namespace {
 
 constexpr int kRbThreads = 256;
 
-struct Src {
-  int i0, i1;
-  float l0, l1;
-};
-
-__device__ __forceinline__ Src source_index(float scale, int dst, int in) {
-  const float s = fmaxf(scale * (dst + 0.5f) - 0.5f, 0.f);
-  Src r;
-  r.i0 = (int)s;
-  r.i1 = r.i0 + (r.i0 < in - 1 ? 1 : 0);
-  r.l1 = s - r.i0;
-  r.l0 = 1.f - r.l1;
-  return r;
-}
-
 // Weight with which output index `dst` reads input index i (both taps when i0 == i1 at the last index).
-__device__ __forceinline__ float tap_weight(const Src& s, int i) {
+__device__ __forceinline__ float tap_weight(const BilinearSrc& s, int i) {
   return (s.i0 == i ? s.l0 : 0.f) + (s.i1 == i ? s.l1 : 0.f);
 }
 
@@ -49,10 +33,10 @@ __device__ __forceinline__ int2 output_range(float scale, int i, int in, int out
   const float inv = 1.f / scale;
   int lo = max((int)floorf((i - 0.5f) * inv - 0.5f) - 2, 0);
   int hi = min((int)ceilf((i + 1.5f) * inv - 0.5f) + 2, out - 1);
-  while (lo > 0 && source_index(scale, lo - 1, in).i0 >= i - 1) --lo;
-  while (lo <= hi && source_index(scale, lo, in).i0 < i - 1) ++lo;
-  while (hi + 1 < out && source_index(scale, hi + 1, in).i0 <= i) ++hi;
-  while (hi >= lo && source_index(scale, hi, in).i0 > i) --hi;
+  while (lo > 0 && bilinear_source_index(scale, lo - 1, in).i0 >= i - 1) --lo;
+  while (lo <= hi && bilinear_source_index(scale, lo, in).i0 < i - 1) ++lo;
+  while (hi + 1 < out && bilinear_source_index(scale, hi + 1, in).i0 <= i) ++hi;
+  while (hi >= lo && bilinear_source_index(scale, hi, in).i0 > i) --hi;
   return make_int2(lo, hi);
 }
 
@@ -68,9 +52,9 @@ resize_bilinear_bwd_kernel(const float* __restrict__ grad_out, float* __restrict
   const float* go = grad_out + nc * Ho * Wo;
   float acc = 0.f;
   for (int oy = ry.x; oy <= ry.y; ++oy) {
-    const float wy = tap_weight(source_index(scale_h, oy, Hi), y);
+    const float wy = tap_weight(bilinear_source_index(scale_h, oy, Hi), y);
     for (int ox = rx.x; ox <= rx.y; ++ox) {
-      const float wx = tap_weight(source_index(scale_w, ox, Wi), x);
+      const float wx = tap_weight(bilinear_source_index(scale_w, ox, Wi), x);
       acc = fmaf(__ldg(go + (long long)oy * Wo + ox), wy * wx, acc);
     }
   }
