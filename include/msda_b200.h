@@ -416,7 +416,8 @@ int msda_b200_host_pipeline_destroy(msda_b200_host_pipeline* pipeline);
 #define MSDA_B200_PROF_COUNT 4
 int msda_b200_profile_ms(int which, float* ms);
 
-/* Number of kernels the library launched in this process since the last reset (memsets not counted). */
+/* Number of kernels the library launched in this process since the last reset. Memsets are not counted, nor are
+ * the cuBLASLt GEMMs of msda_b200_linear_f32_*; the radix sort of a deterministic backward counts as one. */
 int64_t msda_b200_launch_count(int reset);
 
 #ifdef __cplusplus

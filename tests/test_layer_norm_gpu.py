@@ -101,3 +101,19 @@ def test_add_layer_norm_with_clamp_matches_torch(clamp, xdt):
     assert torch.equal(torch.isnan(got), torch.isnan(want))
     ok = ~torch.isnan(want)
     assert torch.allclose(got[ok], want[ok], rtol=1e-5, atol=1e-5)
+
+
+@pytest.mark.parametrize("clamp", [None, 1.0])
+def test_add_layer_norm_launches_are_counted(clamp):
+    """msda_b200_launch_count covers the layer-epilogue kernels: one launch forward, one backward."""
+    from weed_instance_segmentation_b200 import _cabi
+    from weed_instance_segmentation_b200.layer_norm import add_layer_norm
+    x = torch.randn(64, 256, device="cuda", requires_grad=True)
+    r = torch.randn(64, 256, device="cuda")
+    w, b = torch.ones(256, device="cuda", requires_grad=True), torch.zeros(256, device="cuda", requires_grad=True)
+    before = _cabi.launch_count()
+    y = add_layer_norm(x, r, w, b, 1e-5, clamp=clamp)
+    assert _cabi.launch_count() - before == 1
+    y.backward(torch.ones_like(y))
+    torch.cuda.synchronize()
+    assert _cabi.launch_count() - before == 2

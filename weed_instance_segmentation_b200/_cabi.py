@@ -8,6 +8,8 @@ from __future__ import annotations
 import ctypes
 import os
 
+import torch
+
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "libmsda_b200.so")
 
@@ -22,47 +24,12 @@ FLAG_DETERMINISTIC = 64
 FLAG_BF16_ATOMICS = 0
 FLAG_BWD_V2 = 0
 PROF_FWD, PROF_BWD_ZERO, PROF_BWD_MAIN, PROF_BWD_CONVERT = 0, 1, 2, 3
+DTYPE_CODE = {torch.float32: F32, torch.bfloat16: BF16}  # torch dtype -> the library's code (point sampling adds U8)
 
-# every symbol include/msda_b200.h declares
-EXPORTS = (
-    "msda_b200_abi_version",
-    "msda_b200_last_error",
-    "msda_b200_forward",
-    "msda_b200_backward_workspace_bytes",
-    "msda_b200_backward",
-    "msda_b200_forward_fused",
-    "msda_b200_backward_fused",
-    "msda_b200_add_layernorm_forward",
-    "msda_b200_add_layernorm_backward",
-    "msda_b200_add_layernorm_clamp_forward",
-    "msda_b200_add_layernorm_clamp_backward",
-    "msda_b200_query_value_cast_forward",
-    "msda_b200_query_value_cast_backward",
-    "msda_b200_relu_backward_column_sum",
-    "msda_b200_linear_f32_available",
-    "msda_b200_linear_f32_forward",
-    "msda_b200_linear_f32_grad_input",
-    "msda_b200_linear_f32_grad_weight",
-    "msda_b200_column_sum",
-    "msda_b200_groupnorm_to_rows_forward",
-    "msda_b200_groupnorm_to_rows_backward",
-    "msda_b200_point_sample_forward",
-    "msda_b200_point_sample_backward",
-    "msda_b200_point_sample_backward_det_workspace_bytes",
-    "msda_b200_point_sample_backward_det",
-    "msda_b200_resize_bilinear_backward",
-    "msda_b200_postprocess_workspace_bytes",
-    "msda_b200_postprocess_scores",
-    "msda_b200_postprocess_paint",
-    "msda_b200_postprocess_binary_maps",
-    "msda_b200_host_pipeline_create",
-    "msda_b200_host_pipeline_step",
-    "msda_b200_host_pipeline_join",
-    "msda_b200_host_pipeline_sync",
-    "msda_b200_host_pipeline_destroy",
-    "msda_b200_profile_ms",
-    "msda_b200_launch_count",
-)
+
+def ptr(t):
+    """The tensor's address, or None (NULL) for a missing or empty tensor."""
+    return t.data_ptr() if t is not None and t.numel() else None
 
 
 class Desc(ctypes.Structure):
@@ -75,6 +42,60 @@ class Desc(ctypes.Structure):
         ("spatial_shapes_hw", ctypes.POINTER(ctypes.c_int32)),
         ("level_start_index", ctypes.POINTER(ctypes.c_int64)),
     ]
+
+
+_vp, _i32, _i64, _size = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_size_t
+_int, _f32, _f64 = ctypes.c_int, ctypes.c_float, ctypes.c_double
+_desc = ctypes.POINTER(Desc)
+
+# name -> (restype, argtypes) of every function include/msda_b200.h declares (tests/test_abi_signatures.py checks
+# each entry against the header's prototype)
+SIGNATURES = {
+    "msda_b200_abi_version": (_int, []),
+    "msda_b200_last_error": (ctypes.c_char_p, []),
+    "msda_b200_forward": (_int, [_desc, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "msda_b200_backward_workspace_bytes": (_size, [_desc]),
+    "msda_b200_backward": (_int, [_desc, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _size, _vp, _vp]),
+    "msda_b200_forward_fused": (_int, [_desc, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "msda_b200_backward_fused": (_int, [_desc, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _size, _vp, _vp]),
+    "msda_b200_add_layernorm_forward": (_int, [_vp, _int, _vp, _int, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _i64, _i32,
+                                               _vp]),
+    "msda_b200_add_layernorm_backward": (_int, [_vp, _vp, _vp, _int, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64,
+                                                _i32, _vp]),
+    "msda_b200_add_layernorm_clamp_forward": (_int, [_vp, _int, _vp, _int, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp,
+                                                     _i64, _i32, _vp]),
+    "msda_b200_add_layernorm_clamp_backward": (_int, [_vp, _vp, _vp, _int, _vp, _int, _vp, _vp, _f32, _vp, _vp, _vp,
+                                                      _vp, _vp, _vp, _i64, _i32, _vp]),
+    "msda_b200_query_value_cast_forward": (_int, [_vp, _vp, _vp, _vp, _i64, _vp]),
+    "msda_b200_query_value_cast_backward": (_int, [_vp, _vp, _vp, _vp, _i64, _vp]),
+    "msda_b200_relu_backward_column_sum": (_int, [_vp, _vp, _int, _vp, _vp, _i64, _i32, _vp]),
+    "msda_b200_linear_f32_available": (_int, []),
+    "msda_b200_linear_f32_forward": (_int, [_vp, _vp, _vp, _int, _vp, _i64, _i32, _i32, _vp, _size, _vp]),
+    "msda_b200_linear_f32_grad_input": (_int, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _size, _vp]),
+    "msda_b200_linear_f32_grad_weight": (_int, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _size, _vp]),
+    "msda_b200_column_sum": (_int, [_vp, _int, _vp, _i64, _i32, _vp]),
+    "msda_b200_groupnorm_to_rows_forward": (_int, [_vp, _int, _vp, _vp, _f32, _vp, _i64, _vp, _i64, _i32, _i64, _i32,
+                                                   _vp]),
+    "msda_b200_groupnorm_to_rows_backward": (_int, [_vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32,
+                                                    _i64, _i32, _vp]),
+    "msda_b200_point_sample_forward": (_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp]),
+    "msda_b200_point_sample_backward": (_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp]),
+    "msda_b200_point_sample_backward_det_workspace_bytes": (_size, [_i64, _i32, _i64]),
+    "msda_b200_point_sample_backward_det": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _i32, _vp, _size, _vp]),
+    "msda_b200_resize_bilinear_backward": (_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp]),
+    "msda_b200_postprocess_workspace_bytes": (_size, [_i32, _i32, _i32]),
+    "msda_b200_postprocess_scores": (_int, [_vp, _i32, _vp, _i32, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _size, _vp]),
+    "msda_b200_postprocess_paint": (_int, [_vp, _size, _vp, _vp, _f64, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "msda_b200_postprocess_binary_maps": (_int, [_vp, _size, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "msda_b200_host_pipeline_create": (_int, [_desc, _i32, _i32, _i32, _vp, ctypes.POINTER(_vp)]),
+    "msda_b200_host_pipeline_step": (_int, [_vp] * 10),
+    "msda_b200_host_pipeline_join": (_int, [_vp, _vp]),
+    "msda_b200_host_pipeline_sync": (_int, [_vp]),
+    "msda_b200_host_pipeline_destroy": (_int, [_vp]),
+    "msda_b200_profile_ms": (_int, [_int, ctypes.POINTER(_f32)]),
+    "msda_b200_launch_count": (_i64, [_int]),
+}
+EXPORTS = tuple(SIGNATURES)
 
 
 class MSDAError(RuntimeError):
@@ -99,93 +120,9 @@ def load() -> ctypes.CDLL:
             "(needs nvcc). This package has no CPU fallback."
         )
     lib = ctypes.CDLL(LIB_PATH)
-    vp = ctypes.c_void_p
-    dp = ctypes.POINTER(Desc)
-    lib.msda_b200_abi_version.restype = ctypes.c_int
-    lib.msda_b200_abi_version.argtypes = []
-    lib.msda_b200_last_error.restype = ctypes.c_char_p
-    lib.msda_b200_last_error.argtypes = []
-    lib.msda_b200_forward.restype = ctypes.c_int
-    lib.msda_b200_forward.argtypes = [dp, vp, vp, vp, vp, vp, vp]
-    lib.msda_b200_backward_workspace_bytes.restype = ctypes.c_size_t
-    lib.msda_b200_backward_workspace_bytes.argtypes = [dp]
-    lib.msda_b200_backward.restype = ctypes.c_int
-    lib.msda_b200_backward.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_size_t, vp, vp]
-    lib.msda_b200_forward_fused.restype = ctypes.c_int
-    lib.msda_b200_forward_fused.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp, vp]
-    lib.msda_b200_backward_fused.restype = ctypes.c_int
-    lib.msda_b200_backward_fused.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_size_t, vp, vp]
-    lib.msda_b200_add_layernorm_forward.restype = ctypes.c_int
-    lib.msda_b200_add_layernorm_forward.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, vp, vp, ctypes.c_float, vp, vp, vp, vp,
-                                                    ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_add_layernorm_backward.restype = ctypes.c_int
-    lib.msda_b200_add_layernorm_backward.argtypes = [vp, vp, vp, ctypes.c_int, vp, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp,
-                                                     ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_add_layernorm_clamp_forward.restype = ctypes.c_int
-    lib.msda_b200_add_layernorm_clamp_forward.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, vp, vp, ctypes.c_float,
-                                                          ctypes.c_float, vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_add_layernorm_clamp_backward.restype = ctypes.c_int
-    lib.msda_b200_add_layernorm_clamp_backward.argtypes = [vp, vp, vp, ctypes.c_int, vp, ctypes.c_int, vp, vp, ctypes.c_float,
-                                                           vp, vp, vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_query_value_cast_forward.restype = ctypes.c_int
-    lib.msda_b200_query_value_cast_forward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, vp]
-    lib.msda_b200_query_value_cast_backward.restype = ctypes.c_int
-    lib.msda_b200_query_value_cast_backward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, vp]
-    lib.msda_b200_linear_f32_available.restype = ctypes.c_int
-    lib.msda_b200_linear_f32_available.argtypes = []
-    lib.msda_b200_linear_f32_forward.restype = ctypes.c_int
-    lib.msda_b200_linear_f32_forward.argtypes = [vp, vp, vp, ctypes.c_int, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
-                                                 vp, ctypes.c_size_t, vp]
-    for fn in (lib.msda_b200_linear_f32_grad_input, lib.msda_b200_linear_f32_grad_weight):
-        fn.restype = ctypes.c_int
-        fn.argtypes = [vp, vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, vp, ctypes.c_size_t, vp]
-    lib.msda_b200_relu_backward_column_sum.restype = ctypes.c_int
-    lib.msda_b200_relu_backward_column_sum.argtypes = [vp, vp, ctypes.c_int, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_column_sum.restype = ctypes.c_int
-    lib.msda_b200_column_sum.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_groupnorm_to_rows_forward.restype = ctypes.c_int
-    lib.msda_b200_groupnorm_to_rows_forward.argtypes = [vp, ctypes.c_int, vp, vp, ctypes.c_float, vp, ctypes.c_int64, vp,
-                                                        ctypes.c_int64, ctypes.c_int32, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_groupnorm_to_rows_backward.restype = ctypes.c_int
-    lib.msda_b200_groupnorm_to_rows_backward.argtypes = [vp, ctypes.c_int64, vp, ctypes.c_int, vp, vp, vp, vp, vp, vp,
-                                                         ctypes.c_int64, ctypes.c_int32, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_point_sample_forward.restype = ctypes.c_int
-    lib.msda_b200_point_sample_forward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_point_sample_backward.restype = ctypes.c_int
-    lib.msda_b200_point_sample_backward.argtypes = [vp, vp, vp, vp, ctypes.c_int64, ctypes.c_int32, vp]
-    lib.msda_b200_point_sample_backward_det_workspace_bytes.restype = ctypes.c_size_t
-    lib.msda_b200_point_sample_backward_det_workspace_bytes.argtypes = [ctypes.c_int64, ctypes.c_int32, ctypes.c_int64]
-    lib.msda_b200_point_sample_backward_det.restype = ctypes.c_int
-    lib.msda_b200_point_sample_backward_det.argtypes = [vp, vp, vp, ctypes.c_int64, vp, vp, ctypes.c_int64, ctypes.c_int32,
-                                                        vp, ctypes.c_size_t, vp]
-    lib.msda_b200_resize_bilinear_backward.restype = ctypes.c_int
-    lib.msda_b200_resize_bilinear_backward.argtypes = [vp, vp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
-                                                       ctypes.c_int32, ctypes.c_int32, vp]
-    i32 = ctypes.c_int32
-    lib.msda_b200_postprocess_workspace_bytes.restype = ctypes.c_size_t
-    lib.msda_b200_postprocess_workspace_bytes.argtypes = [i32, i32, i32]
-    lib.msda_b200_postprocess_scores.restype = ctypes.c_int
-    lib.msda_b200_postprocess_scores.argtypes = [vp, i32, vp, i32, vp, i32, i32, i32, i32, vp, vp, ctypes.c_size_t, vp]
-    lib.msda_b200_postprocess_paint.restype = ctypes.c_int
-    lib.msda_b200_postprocess_paint.argtypes = [vp, ctypes.c_size_t, vp, vp, ctypes.c_double, vp, i32, i32, i32, vp, vp,
-                                                vp]
-    lib.msda_b200_postprocess_binary_maps.restype = ctypes.c_int
-    lib.msda_b200_postprocess_binary_maps.argtypes = [vp, ctypes.c_size_t, vp, i32, i32, i32, i32, i32, i32, vp, vp]
-    lib.msda_b200_host_pipeline_create.restype = ctypes.c_int
-    lib.msda_b200_host_pipeline_create.argtypes = [dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp,
-                                                   ctypes.POINTER(vp)]
-    lib.msda_b200_host_pipeline_step.restype = ctypes.c_int
-    lib.msda_b200_host_pipeline_step.argtypes = [vp] * 10
-    lib.msda_b200_host_pipeline_join.restype = ctypes.c_int
-    lib.msda_b200_host_pipeline_join.argtypes = [vp, vp]
-    lib.msda_b200_host_pipeline_sync.restype = ctypes.c_int
-    lib.msda_b200_host_pipeline_sync.argtypes = [vp]
-    lib.msda_b200_host_pipeline_destroy.restype = ctypes.c_int
-    lib.msda_b200_host_pipeline_destroy.argtypes = [vp]
-    lib.msda_b200_profile_ms.restype = ctypes.c_int
-    lib.msda_b200_profile_ms.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_float)]
-    lib.msda_b200_launch_count.restype = ctypes.c_int64
-    lib.msda_b200_launch_count.argtypes = [ctypes.c_int]
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     got = lib.msda_b200_abi_version()
     if got != ABI_VERSION:
         raise ImportError(f"{LIB_PATH}: ABI version {got}, expected {ABI_VERSION}; rebuild the library")

@@ -29,8 +29,7 @@
 #include <mutex>
 
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
+#include "internal.h"
 
 namespace {
 

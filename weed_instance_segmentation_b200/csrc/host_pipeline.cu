@@ -17,9 +17,7 @@
 #include <vector>
 
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
-extern "C" int msda_b200_internal_validate(const msda_b200_desc* desc);  // msda_b200.cu: descriptor checks
+#include "internal.h"
 
 namespace {
 
@@ -58,12 +56,10 @@ struct msda_b200_host_pipeline {
 
 namespace {
 
-int cuda_fail(cudaError_t e) { return msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e)); }
-
-#define HP_CUDA(expr)                      \
-  do {                                     \
-    cudaError_t e_ = (expr);               \
-    if (e_ != cudaSuccess) return cuda_fail(e_); \
+#define HP_CUDA(expr)                                              \
+  do {                                                             \
+    cudaError_t e_ = (expr);                                       \
+    if (e_ != cudaSuccess) return cuda_error("host_pipeline", e_); \
   } while (0)
 
 struct DeviceGuard {
@@ -169,7 +165,7 @@ extern "C" int msda_b200_host_pipeline_create(const msda_b200_desc* desc, int32_
   }
   if (e != cudaSuccess) {
     release(p);
-    return cuda_fail(e);
+    return cuda_error("host_pipeline_create", e);
   }
   *pipeline = p;
   return MSDA_B200_OK;

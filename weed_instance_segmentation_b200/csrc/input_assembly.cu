@@ -14,12 +14,8 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
-#include <cstdio>
-
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);
-extern "C" void msda_b200_internal_count_launch(void);
+#include "internal.h"
 
 namespace {
 
@@ -170,16 +166,6 @@ __global__ void __launch_bounds__(256) gn_bwd_apply_transpose_kernel(const float
   }
 }
 
-int check(const char* what) {
-  const cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) {
-    char buf[256];
-    snprintf(buf, sizeof(buf), "%s: %s", what, cudaGetErrorString(e));
-    return msda_b200_internal_fail(MSDA_B200_ERR_CUDA, buf);
-  }
-  return MSDA_B200_OK;
-}
-
 int validate(int64_t B, int32_t C, int64_t HW, int32_t G, int dtype, const char* who) {
   if (B < 0 || HW < 0 || C <= 0 || G <= 0 || C % G != 0) return msda_b200_internal_fail(MSDA_B200_ERR_INVALID, who);
   if (C / G > 8) return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, who);  // at most 8 channels per group (256 / 32)
@@ -204,16 +190,16 @@ int msda_b200_groupnorm_to_rows_forward(const void* x, int x_dtype, const float*
   const dim3 grid((unsigned)((HW + 31) / 32), (unsigned)((C + 31) / 32), (unsigned)B);
   if (x_dtype == MSDA_B200_F32) {
     gn_stats_kernel<float><<<(unsigned)(B * G), 256, 0, st>>>(static_cast<const float*>(x), s2, C, (int)HW, G, eps);
+    if (int rc = launched("groupnorm_to_rows_forward: statistics")) return rc;
     gn_apply_transpose_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(x), s2, gamma, beta, out,
                                                           out_batch_stride, C, (int)HW, G);
   } else {
     gn_stats_kernel<__nv_bfloat16><<<(unsigned)(B * G), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), s2, C, (int)HW, G, eps);
+    if (int rc = launched("groupnorm_to_rows_forward: statistics")) return rc;
     gn_apply_transpose_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), s2, gamma, beta, out,
                                                                   out_batch_stride, C, (int)HW, G);
   }
-  msda_b200_internal_count_launch();
-  msda_b200_internal_count_launch();
-  return check("groupnorm_to_rows_forward");
+  return launched("groupnorm_to_rows_forward: normalise");
 }
 
 int msda_b200_groupnorm_to_rows_backward(const float* grad_out, int64_t grad_out_batch_stride, const void* x, int x_dtype,
@@ -231,18 +217,18 @@ int msda_b200_groupnorm_to_rows_backward(const float* grad_out, int64_t grad_out
   if (x_dtype == MSDA_B200_F32) {
     gn_bwd_reduce_kernel<float><<<(unsigned)(B * G), 256, 0, st>>>(grad_out, grad_out_batch_stride, static_cast<const float*>(x),
                                                                   s2, gamma, m12, grad_gamma, grad_beta, C, (int)HW, G);
+    if (int rc = launched("groupnorm_to_rows_backward: reduction")) return rc;
     gn_bwd_apply_transpose_kernel<float><<<grid, 256, 0, st>>>(grad_out, grad_out_batch_stride, static_cast<const float*>(x), s2,
                                                               m12, gamma, static_cast<float*>(grad_x), C, (int)HW, G);
   } else {
     gn_bwd_reduce_kernel<__nv_bfloat16><<<(unsigned)(B * G), 256, 0, st>>>(
         grad_out, grad_out_batch_stride, static_cast<const __nv_bfloat16*>(x), s2, gamma, m12, grad_gamma, grad_beta, C, (int)HW, G);
+    if (int rc = launched("groupnorm_to_rows_backward: reduction")) return rc;
     gn_bwd_apply_transpose_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(
         grad_out, grad_out_batch_stride, static_cast<const __nv_bfloat16*>(x), s2, m12, gamma,
         static_cast<__nv_bfloat16*>(grad_x), C, (int)HW, G);
   }
-  msda_b200_internal_count_launch();
-  msda_b200_internal_count_launch();
-  return check("groupnorm_to_rows_backward");
+  return launched("groupnorm_to_rows_backward: transpose");
 }
 
 }  // extern "C"

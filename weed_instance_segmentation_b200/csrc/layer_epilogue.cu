@@ -18,8 +18,7 @@
 #include <cstdint>
 
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
+#include "internal.h"
 
 namespace {
 
@@ -205,8 +204,7 @@ int launch_fwd_ch(int xd, int rd, const void* x, const void* r, const float* gam
     add_layernorm_fwd_kernel<bf, bf, CH><<<blocks, kThreads, 0, st>>>(x, r, gamma, beta, eps, y, y_lowp, mean, rstd, N, clamp);
   else
     add_layernorm_fwd_kernel<float, bf, CH><<<blocks, kThreads, 0, st>>>(x, r, gamma, beta, eps, y, y_lowp, mean, rstd, N, clamp);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("add_layernorm_forward");
 }
 
 template <int CH>
@@ -240,8 +238,7 @@ int launch_bwd_ch(int xd, int rd, const float* dy, const void* dy_lowp, const vo
   else MSDA_LN_BWD(float, bf);
 #undef MSDA_LN_BWD
 #undef MSDA_LN_BWD_LAUNCH
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("add_layernorm_backward");
 }
 
 bool bad_dtype(int d) { return d != MSDA_B200_F32 && d != MSDA_B200_BF16; }
@@ -463,8 +460,7 @@ static int column_sum_impl(const void* matrix, int dtype, float* out, int64_t ro
     colsum_kernel<__nv_bfloat16, false><<<(unsigned)blocks, threads, smem, st>>>(matrix, out, rows, cv, rl, rows_per_block);
   else
     colsum_kernel<float, false><<<(unsigned)blocks, threads, smem, st>>>(matrix, out, rows, cv, rl, rows_per_block);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("column_sum");
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -542,8 +538,7 @@ extern "C" int msda_b200_query_value_cast_forward(const float* hidden, const flo
   qv_cast_fwd_kernel<<<qv_blocks(n8), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const float4*>(hidden), reinterpret_cast<const float4*>(pos), reinterpret_cast<uint4*>(query_bf16),
       reinterpret_cast<uint4*>(value_bf16), n8);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("query_value_cast_forward");
 }
 
 extern "C" int msda_b200_query_value_cast_backward(const void* grad_query_bf16, const void* grad_value_bf16,
@@ -556,6 +551,5 @@ extern "C" int msda_b200_query_value_cast_backward(const void* grad_query_bf16, 
   qv_cast_bwd_kernel<<<qv_blocks(n8), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const uint4*>(grad_query_bf16), reinterpret_cast<const uint4*>(grad_value_bf16),
       reinterpret_cast<float4*>(grad_hidden), reinterpret_cast<float4*>(grad_pos), n8);
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("query_value_cast_backward");
 }

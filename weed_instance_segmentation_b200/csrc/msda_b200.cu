@@ -21,18 +21,14 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
-#include <cstring>
 #include <type_traits>
 
 #include "msda_b200.h"
+#include "internal.h"
 #include "msda_bwd_det.cuh"
-
-// msda_bwd_det.cu: the deterministic backward's sort and grad_value pull (CUB stays out of this file)
-extern "C" int msda_b200_internal_det_workspace_bytes(const msda_b200_desc* desc, size_t* bytes);
-extern "C" int msda_b200_internal_det_grad_value(const msda_b200_desc* desc, const void* grad_out, void* grad_value,
-                                                 void* workspace, cudaStream_t stream);
 
 namespace {
 
@@ -97,16 +93,6 @@ __device__ __forceinline__ float2 fused_loc(const KParams& p, long long si, long
   const float2 off = load_pair<AT>(p.offsets, si);
   const float2 r = p.ref ? __ldg(reinterpret_cast<const float2*>(p.ref) + ri) : implicit_reference_point(p, q);
   return make_float2(__fadd_rn(r.x, __fdiv_rn(off.x, (float)lv.W)), __fadd_rn(r.y, __fdiv_rn(off.y, (float)lv.H)));
-}
-
-// max and 1 / sum(exp(x - max)) of the LP logits of one (query, head)
-template <typename AT>
-__device__ __forceinline__ void softmax_stats(const AT* lg, int LP, float& mx, float& inv) {
-  mx = -INFINITY;
-  for (int s = 0; s < LP; ++s) mx = fmaxf(mx, to_float<AT>(lg[s]));
-  float sum = 0.f;
-  for (int s = 0; s < LP; ++s) sum += expf(to_float<AT>(lg[s]) - mx);
-  inv = 1.f / sum;
 }
 
 // max and 1/sum(exp(x - max)) of one (query, head) row, computed by four adjacent lanes (lane & 3 = sub) that each
@@ -746,10 +732,24 @@ void fill_geometry(const msda_b200_desc* d, KParams& p, int tq) {
   }
 }
 
-int check_launch(const char* what) {
-  const cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
-  return MSDA_B200_OK;
+// One launch of an MSDA kernel, timed into the profiling slot `prof` when the descriptor asks for it. Before it: the
+// dynamic shared-memory limit (raised above the 48 KB default, or always with `opt_in`), the carve-out unless it is
+// kKeepCarveout, and the grid limit.
+constexpr int kKeepCarveout = INT_MIN;
+
+template <typename... KA, typename... A>
+int launch(const msda_b200_desc* d, int prof, const char* what, void (*kern)(KA...), long long blocks, int threads,
+           size_t smem, bool opt_in, int carveout, cudaStream_t st, A... args) {
+  if ((opt_in || smem > 48 * 1024) &&
+      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    return fail(MSDA_B200_ERR_CUDA, "%s: cannot reserve %zu bytes of shared memory", what, smem);
+  if (carveout != kKeepCarveout) cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
+  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "%s: grid too large", what);
+  {
+    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, prof, st);
+    kern<<<(unsigned)blocks, threads, smem, st>>>(args...);
+  }
+  return launched(what);
 }
 
 // Launch geometry: NT threads per block, QPG queries per lane group.
@@ -766,17 +766,8 @@ int launch_fwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   const bool strict = (d->flags & MSDA_B200_FLAG_STRICT_PADDING) != 0;
   auto kern = strict ? msda_fwd_kernel<VT, AT, D, kFwdNT, kFwdQPG, FUSED, true>
                      : msda_fwd_kernel<VT, AT, D, kFwdNT, kFwdQPG, FUSED, false>;
-  if (smem > 48 * 1024 &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "forward: cannot reserve %zu bytes of shared memory", smem);
-  const long long blocks = (long long)p.B * p.num_tiles * p.H;
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "forward: grid too large");
-  {
-    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_FWD, st);
-    kern<<<(unsigned)blocks, kFwdNT, smem, st>>>(p);
-    ++g_launches;
-  }
-  return check_launch("msda_b200_forward");
+  return launch(d, MSDA_B200_PROF_FWD, "forward", kern, (long long)p.B * p.num_tiles * p.H, kFwdNT, smem, false,
+                kKeepCarveout, st, p);
 }
 
 // Forward with two heads per block (see msda_fwd_pair_kernel). 128 threads, 2 (query, head) pairs per lane group
@@ -790,23 +781,13 @@ int launch_fwd_pair(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   const size_t smem = (size_t)p.LP * ROW * (sizeof(float4) + sizeof(int)) + (FUSED ? (size_t)TV * p.LP * sizeof(float) + (size_t)TQ * sizeof(float2) : 0);
   auto kern = (d->L == 3 && d->P == 4) ? msda_fwd_pair_kernel<VT, AT, D, NT, QPG, HPB, FUSED, 3>
                                        : msda_fwd_pair_kernel<VT, AT, D, NT, QPG, HPB, FUSED, 0>;
-  if (smem > 48 * 1024 &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "forward: cannot reserve %zu bytes of shared memory", smem);
   // Shared-memory carve-out: what is left of the SM's 256 KB is the L1 the gather lives in. The driver's default makes
   // room for the register limit's 9 blocks; 50 % (132 KB) holds 7 blocks of the plain kernel and leaves the gather
   // 124 KB of L1. Measured (profiles/r02_notes.md; config 2 init / trained, config 3 init / trained, ms): default
   // 0.286 / 0.306 / 0.661 / 0.717, 50 %: 0.282 / 0.301 / 0.655 / 0.696, 40 %: 0.313 / 0.337 / 0.697 / 0.747. The fused
   // prologue's blocks are 3 KB larger (softmax tile), 50 % holds only 6 of them: 0.407 vs 0.321 ms -> driver default.
-  cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, FUSED ? -1 : 50);
-  const long long blocks = (long long)p.B * p.num_tiles * (p.H / HPB);
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "forward: grid too large");
-  {
-    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_FWD, st);
-    kern<<<(unsigned)blocks, NT, smem, st>>>(p);
-    ++g_launches;
-  }
-  return check_launch("msda_b200_forward (head pairs)");
+  return launch(d, MSDA_B200_PROF_FWD, "forward (head pairs)", kern, (long long)p.B * p.num_tiles * (p.H / HPB), NT,
+                smem, false, FUSED ? -1 : 50, st, p);
 }
 
 template <typename VT, typename AT, int D, int ACC, bool FUSED>
@@ -818,18 +799,8 @@ int launch_bwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   const size_t smem = n * (2 * sizeof(float4) + sizeof(float) + sizeof(int)) +
                       (size_t)p.LP * T::TQ * LPP * sizeof(float4) +
                       (FUSED ? 2 * (size_t)T::TQ * p.LP * sizeof(float) : 0);
-  auto kern = msda_bwd_kernel<VT, AT, D, kBwdNT, kBwdQPG, ACC, FUSED>;
-  if (smem > 48 * 1024 &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "backward: cannot reserve %zu bytes of shared memory", smem);
-  const long long blocks = (long long)p.B * p.num_tiles * p.H;
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "backward: grid too large");
-  {
-    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_BWD_MAIN, st);
-    kern<<<(unsigned)blocks, kBwdNT, smem, st>>>(p);
-    ++g_launches;
-  }
-  return check_launch("msda_b200_backward");
+  return launch(d, MSDA_B200_PROF_BWD_MAIN, "backward", msda_bwd_kernel<VT, AT, D, kBwdNT, kBwdQPG, ACC, FUSED>,
+                (long long)p.B * p.num_tiles * p.H, kBwdNT, smem, false, kKeepCarveout, st, p);
 }
 
 template <typename VT, typename AT, bool FUSED>
@@ -868,17 +839,9 @@ int launch_bwd_mma(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   constexpr int P = 4;
   fill_geometry(d, p, kMmaTQ);
   const size_t smem = mma_smem_layout<kMmaNT, kMmaTQ, P, kMmaGCAP, kMmaRCAP, FUSED>().total;
-  auto kern = msda_bwd_mma_kernel<AT, kMmaNT, kMmaTQ, P, kMmaGCAP, kMmaRCAP, FUSED>;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "backward: cannot reserve %zu bytes of shared memory", smem);
-  const long long blocks = (long long)p.B * p.num_tiles * p.H;
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "backward: grid too large");
-  {
-    ProfScope ps((d->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_BWD_MAIN, st);
-    kern<<<(unsigned)blocks, kMmaNT, smem, st>>>(p);
-    ++g_launches;
-  }
-  return check_launch("msda_b200_backward (group-sorted, mma)");
+  return launch(d, MSDA_B200_PROF_BWD_MAIN, "backward (group-sorted, mma)",
+                msda_bwd_mma_kernel<AT, kMmaNT, kMmaTQ, P, kMmaGCAP, kMmaRCAP, FUSED>,
+                (long long)p.B * p.num_tiles * p.H, kMmaNT, smem, true, kKeepCarveout, st, p);
 }
 
 template <typename VT, typename AT, int ACC, bool FUSED>
@@ -896,12 +859,48 @@ int dispatch_bwd(const msda_b200_desc* d, const KParams& p, cudaStream_t st) {
   return fail(MSDA_B200_ERR_UNSUPPORTED, "head dim %d", d->D);
 }
 
+// The (value, attention) dtype pairs that have kernels, as f(VT{}, AT{}): fp32 / fp32, bf16 / bf16 and bf16 / fp32.
+template <typename F>
+int with_dtypes(const msda_b200_desc* d, F f) {
+  if (d->value_dtype != MSDA_B200_BF16) return f(float{}, float{});
+  if (d->attn_dtype == MSDA_B200_BF16) return f(__nv_bfloat16{}, __nv_bfloat16{});
+  return f(__nv_bfloat16{}, float{});
+}
+
 template <bool FUSED>
 int run_forward(const msda_b200_desc* desc, const KParams& p, cudaStream_t st) {
-  const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
-  if (!vbf) return dispatch_fwd<float, float, FUSED>(desc, p, st);
-  if (abf) return dispatch_fwd<__nv_bfloat16, __nv_bfloat16, FUSED>(desc, p, st);
-  return dispatch_fwd<__nv_bfloat16, float, FUSED>(desc, p, st);
+  return with_dtypes(desc, [&](auto v, auto a) { return dispatch_fwd<decltype(v), decltype(a), FUSED>(desc, p, st); });
+}
+
+// The backward's argument checks, in this order, for a validated descriptor with B > 0. *need: the workspace bytes.
+int check_backward(const msda_b200_desc* d, const void* grad_value, const void* workspace, size_t workspace_bytes,
+                   bool have_tensors, size_t* need) {
+  if (!grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
+  if (!(d->flags & MSDA_B200_FLAG_DETERMINISTIC)) *need = msda_b200_backward_workspace_bytes(d);
+  else if (int rc = msda_b200_internal_det_workspace_bytes(d, need)) return rc;
+  if (*need && (!workspace || workspace_bytes < *need))
+    return fail(MSDA_B200_ERR_WORKSPACE, "backward: workspace of %zu bytes required, got %zu", *need, workspace_bytes);
+  if (*need && (reinterpret_cast<uintptr_t>(workspace) & 15))
+    return fail(MSDA_B200_ERR_INVALID, "backward: workspace must be 16-byte aligned");
+  if (d->Q != 0 && !have_tensors) return fail(MSDA_B200_ERR_INVALID, "backward: NULL tensor pointer");
+  return MSDA_B200_OK;
+}
+
+// MSDA_B200_FLAG_DETERMINISTIC: the per-corner kernel without its scatter writes grad_loc / grad_attn and the records
+// of every sample; msda_bwd_det.cu orders the records and writes every element of grad_value from them. No float
+// atomics, so equal inputs give equal bits.
+template <bool FUSED>
+int run_backward_det(const msda_b200_desc* desc, KParams p, void* grad_value, void* workspace, cudaStream_t st) {
+  if (desc->Q != 0) {
+    const DetLayout lay = det_layout(desc);
+    p.det_keys = reinterpret_cast<unsigned*>(static_cast<char*>(workspace) + lay.keys_off[0]);
+    p.det_vals = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + lay.vals_off[0]);
+    p.det_sentinel = (unsigned)lay.keys;
+    const int rc =
+        with_dtypes(desc, [&](auto v, auto a) { return dispatch_bwd<decltype(v), decltype(a), 2, FUSED>(desc, p, st); });
+    if (rc) return rc;
+  }
+  return msda_b200_internal_det_grad_value(desc, p.grad_out, grad_value, workspace, st);
 }
 
 // Shared by the plain and the fused backward: zero-fill, main kernel, bf16 conversion.
@@ -913,82 +912,42 @@ int run_forward(const msda_b200_desc* desc, const KParams& p, cudaStream_t st) {
 template <bool FUSED>
 int run_backward(const msda_b200_desc* desc, KParams p, void* grad_value, void* workspace, size_t workspace_bytes,
                  bool have_tensors, cudaStream_t st) {
-  const bool prof = (desc->flags & MSDA_B200_FLAG_PROFILE) != 0;
-  const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
-  const size_t nvalue = (size_t)desc->B * desc->S * desc->H * desc->D;
-  const size_t need = msda_b200_backward_workspace_bytes(desc);
-  if (nvalue && !grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
-  if (need && nvalue && (!workspace || workspace_bytes < need))
-    return fail(MSDA_B200_ERR_WORKSPACE, "backward: workspace of %zu bytes required, got %zu", need, workspace_bytes);
-  if (nvalue && need && (reinterpret_cast<uintptr_t>(workspace) & 15))
-    return fail(MSDA_B200_ERR_INVALID, "backward: workspace must be 16-byte aligned");
+  if (desc->B == 0) return MSDA_B200_OK;  // validate() makes S >= 1, so only an empty batch has no grad_value
+  size_t need = 0;
+  if (int rc = check_backward(desc, grad_value, workspace, workspace_bytes, have_tensors, &need)) return rc;
+  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC) return run_backward_det<FUSED>(desc, p, grad_value, workspace, st);
 
   // Zero-fill the accumulator (and grad_value): the scatter only touches sampled pixels.
+  const size_t nvalue = (size_t)desc->B * desc->S * desc->H * desc->D;
   void* acc = need ? workspace : grad_value;
-  if (nvalue) {
-    ProfScope ps(prof, MSDA_B200_PROF_BWD_ZERO, st);
-    const size_t acc_bytes = need ? need : nvalue * dtype_size(desc->value_dtype);
-    if (cudaMemsetAsync(acc, 0, acc_bytes, st) != cudaSuccess) return check_launch("backward: memset");
+  {
+    ProfScope ps((desc->flags & MSDA_B200_FLAG_PROFILE) != 0, MSDA_B200_PROF_BWD_ZERO, st);
+    const cudaError_t e = cudaMemsetAsync(acc, 0, need ? need : nvalue * dtype_size(desc->value_dtype), st);
+    if (e != cudaSuccess) return cuda_error("backward: memset", e);
   }
-  if ((long long)desc->B * desc->Q != 0) {
-    if (!have_tensors) return fail(MSDA_B200_ERR_INVALID, "backward: NULL tensor pointer");
+  if (desc->Q != 0) {
     p.grad_value_acc = acc;
-    int rc;
-    if (!vbf) rc = dispatch_bwd<float, float, 0, FUSED>(desc, p, st);
-    else rc = abf ? dispatch_bwd<__nv_bfloat16, __nv_bfloat16, 0, FUSED>(desc, p, st)
-                  : dispatch_bwd<__nv_bfloat16, float, 0, FUSED>(desc, p, st);
+    const int rc =
+        with_dtypes(desc, [&](auto v, auto a) { return dispatch_bwd<decltype(v), decltype(a), 0, FUSED>(desc, p, st); });
     if (rc) return rc;
   }
-  if (need && nvalue) {
-    ProfScope ps(prof, MSDA_B200_PROF_BWD_CONVERT, st);
+  if (need) {
     const long long n8 = (long long)(nvalue / 8);  // D is a multiple of 8, so nvalue % 8 == 0
-    const int blocks = (int)((n8 + 255) / 256 < 148 * 16 ? (n8 + 255) / 256 : 148 * 16);
-    msda_cvt_f32_bf16_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(workspace),
-                                                     reinterpret_cast<uint4*>(grad_value), n8);
-    ++g_launches;
-    if (int rc = check_launch("backward: convert")) return rc;
+    const long long blocks = (n8 + 255) / 256 < 148 * 16 ? (n8 + 255) / 256 : 148 * 16;
+    return launch(desc, MSDA_B200_PROF_BWD_CONVERT, "backward: convert", msda_cvt_f32_bf16_kernel, blocks, 256, 0,
+                  false, kKeepCarveout, st, reinterpret_cast<const float4*>(workspace),
+                  reinterpret_cast<uint4*>(grad_value), n8);
   }
   return MSDA_B200_OK;
-}
-
-// MSDA_B200_FLAG_DETERMINISTIC: the per-corner kernel without its scatter writes grad_loc / grad_attn and the records
-// of every sample; msda_bwd_det.cu orders the records and writes every element of grad_value from them. No float
-// atomics, so equal inputs give equal bits.
-template <bool FUSED>
-int run_backward_det(const msda_b200_desc* desc, KParams p, void* grad_value, void* workspace, size_t workspace_bytes,
-                     bool have_tensors, cudaStream_t st) {
-  if (desc->B == 0) return MSDA_B200_OK;
-  if (!grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
-  size_t need = 0;
-  if (int rc = msda_b200_internal_det_workspace_bytes(desc, &need)) return rc;
-  if (!workspace || workspace_bytes < need)
-    return fail(MSDA_B200_ERR_WORKSPACE, "backward: workspace of %zu bytes required, got %zu", need, workspace_bytes);
-  if (reinterpret_cast<uintptr_t>(workspace) & 15) return fail(MSDA_B200_ERR_INVALID, "backward: workspace must be 16-byte aligned");
-  if (desc->Q != 0) {
-    if (!have_tensors) return fail(MSDA_B200_ERR_INVALID, "backward: NULL tensor pointer");
-    const DetLayout lay = det_layout(desc);
-    p.det_keys = reinterpret_cast<unsigned*>(static_cast<char*>(workspace) + lay.keys_off[0]);
-    p.det_vals = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + lay.vals_off[0]);
-    p.det_sentinel = (unsigned)lay.keys;
-    const bool vbf = desc->value_dtype == MSDA_B200_BF16, abf = desc->attn_dtype == MSDA_B200_BF16;
-    int rc;
-    if (!vbf) rc = dispatch_bwd<float, float, 2, FUSED>(desc, p, st);
-    else rc = abf ? dispatch_bwd<__nv_bfloat16, __nv_bfloat16, 2, FUSED>(desc, p, st)
-                  : dispatch_bwd<__nv_bfloat16, float, 2, FUSED>(desc, p, st);
-    if (rc) return rc;
-  }
-  return msda_b200_internal_det_grad_value(desc, p.grad_out, grad_value, workspace, st);
 }
 
 }  // namespace
 
 extern "C" {
 
-// shared with layer_epilogue.cu (not part of the public header)
+// declared in internal.h for the library's other files
 int msda_b200_internal_fail(int code, const char* msg) { return fail(code, "%s", msg); }
-// shared with host_pipeline.cu: the descriptor checks of forward / backward
 int msda_b200_internal_validate(const msda_b200_desc* desc) { return validate(desc); }
-// shared with point_sample.cu: kernels launched outside this file count too
 void msda_b200_internal_count_launch(void) { ++g_launches; }
 
 int msda_b200_abi_version(void) { return MSDA_B200_ABI_VERSION; }
@@ -1001,8 +960,7 @@ int msda_b200_forward(const msda_b200_desc* desc, const void* value, const float
   if (int rc = validate(desc)) return rc;
   if ((long long)desc->B * desc->Q == 0) return MSDA_B200_OK;
   if (!value || !loc || !attn || !out) return fail(MSDA_B200_ERR_INVALID, "forward: NULL tensor pointer");
-  KParams p;
-  memset(&p, 0, sizeof(p));
+  KParams p{};
   p.value = value; p.loc = loc; p.attn = attn; p.out = out; p.q_order = query_order;
   return run_forward<false>(desc, p, reinterpret_cast<cudaStream_t>(stream));
 }
@@ -1016,8 +974,7 @@ int msda_b200_forward_fused(const msda_b200_desc* desc, const void* value, const
   if (!value || !offsets || !logits || !out) return fail(MSDA_B200_ERR_INVALID, "forward_fused: NULL tensor pointer");
   if (!ref_points && desc->Q != desc->S)
     return fail(MSDA_B200_ERR_INVALID, "forward_fused: implicit reference points (ref_points = NULL) need Q == S");
-  KParams p;
-  memset(&p, 0, sizeof(p));
+  KParams p{};
   p.value = value; p.offsets = offsets; p.logits = logits; p.ref = ref_points; p.out = out; p.attn_out = attn_out;
   p.q_order = query_order;
   return run_forward<true>(desc, p, reinterpret_cast<cudaStream_t>(stream));
@@ -1040,13 +997,10 @@ int msda_b200_backward(const msda_b200_desc* desc, const void* value, const floa
                        size_t workspace_bytes, const int32_t* query_order, void* stream) {
   g_err[0] = 0;
   if (int rc = validate(desc)) return rc;
-  KParams p;
-  memset(&p, 0, sizeof(p));
+  KParams p{};
   p.value = value; p.loc = loc; p.attn = attn; p.grad_out = grad_out;
   p.grad_loc = grad_loc; p.grad_attn = grad_attn; p.q_order = query_order;
   const bool have = value && loc && attn && grad_out && grad_loc && grad_attn;
-  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC)
-    return run_backward_det<false>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
   return run_backward<false>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -1056,15 +1010,12 @@ int msda_b200_backward_fused(const msda_b200_desc* desc, const void* value, cons
                              void* stream) {
   g_err[0] = 0;
   if (int rc = validate(desc)) return rc;
-  KParams p;
-  memset(&p, 0, sizeof(p));
+  KParams p{};
   p.value = value; p.offsets = offsets; p.logits = logits; p.ref = ref_points; p.grad_out = grad_out;
   p.grad_offsets = grad_offsets; p.grad_logits = grad_logits; p.q_order = query_order;
   if (!ref_points && desc->Q != desc->S)
     return fail(MSDA_B200_ERR_INVALID, "backward_fused: implicit reference points (ref_points = NULL) need Q == S");
   const bool have = value && offsets && logits && grad_out && grad_offsets && grad_logits;
-  if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC)
-    return run_backward_det<true>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
   return run_backward<true>(desc, p, grad_value, workspace, workspace_bytes, have, reinterpret_cast<cudaStream_t>(stream));
 }
 

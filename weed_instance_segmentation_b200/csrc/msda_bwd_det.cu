@@ -15,10 +15,8 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "msda_b200.h"
+#include "internal.h"
 #include "msda_bwd_det.cuh"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
-extern "C" void msda_b200_internal_count_launch(void);
 
 namespace {
 
@@ -68,13 +66,13 @@ __global__ void __launch_bounds__(kDetNT) msda_bwd_det_pull_kernel(const uint2* 
   grad_value[k * LPP + c] = Vec16<VT>::pack(acc);
 }
 
-int fail(int code, const char* msg) { return msda_b200_internal_fail(code, msg); }
-
 int check_supported(const DetLayout& lay) {
   if (lay.records > INT_MAX)
-    return fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: more than 2^31 - 1 records (4 per sample)");
+    return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED,
+                                   "deterministic backward: more than 2^31 - 1 records (4 per sample)");
   if (lay.keys > 0xffffffffll)
-    return fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: B*S*H does not fit a 32-bit sort key");
+    return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED,
+                                   "deterministic backward: B*S*H does not fit a 32-bit sort key");
   return MSDA_B200_OK;
 }
 
@@ -83,12 +81,11 @@ int launch_pull(const DetLayout& lay, const msda_b200_desc* d, const uint2* rang
                 const void* grad_out, void* grad_value, cudaStream_t st) {
   constexpr int LPP = D / Vec16<VT>::N;
   const long long blocks = (lay.keys * LPP + kDetNT - 1) / kDetNT;
-  if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: grid too large");
+  if (blocks > 0x7fffffffll)
+    return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: grid too large");
   msda_bwd_det_pull_kernel<VT, D><<<(unsigned)blocks, kDetNT, 0, st>>>(
       ranges, vals, static_cast<const uint4*>(grad_out), static_cast<uint4*>(grad_value), lay.keys, d->S, d->Q, d->H);
-  msda_b200_internal_count_launch();
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("deterministic backward: grad_value");
 }
 
 template <typename VT>
@@ -101,7 +98,7 @@ int dispatch_pull(const DetLayout& lay, const msda_b200_desc* d, const uint2* ra
     case 64: return launch_pull<VT, 64>(lay, d, ranges, vals, grad_out, grad_value, st);
     case 128: return launch_pull<VT, 128>(lay, d, ranges, vals, grad_out, grad_value, st);
   }
-  return fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: head dim");
+  return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "deterministic backward: head dim");
 }
 
 }  // namespace
@@ -113,7 +110,7 @@ extern "C" int msda_b200_internal_det_sort_bytes(const DetLayout* lay, size_t* b
   cub::DoubleBuffer<unsigned long long> vb(nullptr, nullptr);
   const cudaError_t e =
       cub::DeviceRadixSort::SortPairs(nullptr, *bytes, kb, vb, (int)lay->records, 0, lay->key_bits, (cudaStream_t)0);
-  return e == cudaSuccess ? MSDA_B200_OK : fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return e == cudaSuccess ? MSDA_B200_OK : cuda_error("deterministic sort: scratch size", e);
 }
 
 extern "C" int msda_b200_internal_det_sort(const DetLayout* lay, void* workspace, const unsigned** keys,
@@ -127,7 +124,7 @@ extern "C" int msda_b200_internal_det_sort(const DetLayout* lay, void* workspace
   if (int rc = msda_b200_internal_det_sort_bytes(lay, &sort)) return rc;
   const cudaError_t e =
       cub::DeviceRadixSort::SortPairs(ws + lay->sort_off, sort, kb, vb, (int)lay->records, 0, lay->key_bits, st);
-  if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  if (e != cudaSuccess) return cuda_error("deterministic sort", e);
   msda_b200_internal_count_launch();  // the sort's kernels count as one launch
   *keys = kb.Current();
   *vals = vb.Current();
@@ -154,15 +151,14 @@ extern "C" int msda_b200_internal_det_grad_value(const msda_b200_desc* desc, con
   char* ws = static_cast<char*>(workspace);
   uint2* ranges = reinterpret_cast<uint2*>(ws + lay.ranges_off);
   const unsigned long long* vals = reinterpret_cast<const unsigned long long*>(ws + lay.vals_off[0]);
-  cudaError_t e = cudaMemsetAsync(ranges, 0, (size_t)lay.keys * sizeof(uint2), st);
-  if (e != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  const cudaError_t e = cudaMemsetAsync(ranges, 0, (size_t)lay.keys * sizeof(uint2), st);
+  if (e != cudaSuccess) return cuda_error("deterministic backward: memset", e);
   if (lay.records) {
     const unsigned* keys = nullptr;
     if (int rc = msda_b200_internal_det_sort(&lay, workspace, &keys, &vals, st)) return rc;
     const int n = (int)lay.records;
     msda_bwd_det_ranges_kernel<<<(n + kDetNT - 1) / kDetNT, kDetNT, 0, st>>>(keys, n, (unsigned)lay.keys, ranges);
-    msda_b200_internal_count_launch();
-    if ((e = cudaGetLastError()) != cudaSuccess) return fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+    if (int rc = launched("deterministic backward: ranges")) return rc;
   }
   if (desc->value_dtype == MSDA_B200_BF16)
     return dispatch_pull<__nv_bfloat16>(lay, desc, ranges, vals, grad_out, grad_value, st);

@@ -4,7 +4,7 @@
 // msda_b200.h and cuda_runtime.h.
 //
 // Both write (uint32 key, uint64 payload) records into the first key / payload buffers of the layout; a stable CUB
-// radix sort over the key's bits (msda_b200_internal_det_sort) then groups them by key, each group in record order,
+// radix sort over the key's bits (msda_b200_internal_det_sort, internal.h) then groups them by key, each group in record order,
 // which depends on the inputs alone. The key `keys` (one past the last destination) marks a record that adds nothing
 // and sorts last.
 //
@@ -49,11 +49,3 @@ inline DetLayout det_sort_layout(long long records, long long keys, bool ranges)
 inline DetLayout det_layout(const msda_b200_desc* d) {
   return det_sort_layout(4ll * d->B * d->Q * d->H * d->L * d->P, (long long)d->B * d->S * d->H, true);
 }
-
-// msda_bwd_det.cu (CUB stays in that file). The caller has checked records <= INT_MAX and keys <= 2^32 - 1.
-// Bytes of the sort's scratch, as CUB reports them for the current device (0 without records):
-extern "C" int msda_b200_internal_det_sort_bytes(const DetLayout* lay, size_t* bytes);
-// The sort of the records in the first buffers of `workspace` (at least lay->sort_off + the bytes above); *keys and
-// *vals receive the buffers that hold the sorted records.
-extern "C" int msda_b200_internal_det_sort(const DetLayout* lay, void* workspace, const unsigned** keys,
-                                           const unsigned long long** vals, cudaStream_t stream);

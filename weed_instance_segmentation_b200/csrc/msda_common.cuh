@@ -123,8 +123,7 @@ struct Vec16<__nv_bfloat16> {
 
 __device__ __forceinline__ uint4 ldg16(const uint4* p) { return __ldg(p); }
 
-// Packed fp32 FMA (sm_100a FFMA2): (a0, a1) += w * (f0, f1) and (a0, a1) += (g0, g1) * (f0, f1), each element rounded
-// exactly like fmaf. One instruction for two FMAs: the kernels here are bound by instruction issue, not by the FMA pipe.
+// Packed fp32 FMA (sm_100a FFMA2): (a0, a1) += w * (f0, f1), each element rounded exactly like fmaf. One instruction for two FMAs: the kernels here are bound by instruction issue, not by the FMA pipe.
 __device__ __forceinline__ void fma2_scalar(float& a0, float& a1, float w, float f0, float f1) {
   asm("{ .reg .b64 ra, rw, rf;\n\t"
       "mov.b64 ra, {%0, %1};\n\t"
@@ -134,16 +133,6 @@ __device__ __forceinline__ void fma2_scalar(float& a0, float& a1, float w, float
       "mov.b64 {%0, %1}, ra; }"
       : "+f"(a0), "+f"(a1)
       : "f"(w), "f"(f0), "f"(f1));
-}
-__device__ __forceinline__ void fma2_pair(float& a0, float& a1, float g0, float g1, float f0, float f1) {
-  asm("{ .reg .b64 ra, rg, rf;\n\t"
-      "mov.b64 ra, {%0, %1};\n\t"
-      "mov.b64 rg, {%2, %3};\n\t"
-      "mov.b64 rf, {%4, %5};\n\t"
-      "fma.rn.f32x2 ra, rg, rf, ra;\n\t"
-      "mov.b64 {%0, %1}, ra; }"
-      : "+f"(a0), "+f"(a1)
-      : "f"(g0), "f"(g1), "f"(f0), "f"(f1));
 }
 
 // red.global.add.v4.f32 (sm_90+): one 16-byte reduction, no return value.

@@ -18,10 +18,8 @@
 #include <cstdint>
 
 #include "msda_b200.h"
+#include "internal.h"
 #include "msda_bwd_det.cuh"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
-extern "C" void msda_b200_internal_count_launch(void);               // msda_b200.cu: launch counter
 
 namespace {
 
@@ -151,14 +149,6 @@ point_sample_bwd_det_sum_kernel(float* const* __restrict__ grad_planes, const in
   grad_planes[r][key - key_base[r]] += acc;
 }
 
-int check(const char* what) {
-  const cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) return MSDA_B200_OK;
-  msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
-  (void)what;
-  return MSDA_B200_ERR_CUDA;
-}
-
 int check_args(const void* a, const void* b, const void* c, const void* d, int64_t R, int32_t K) {
   if (R < 0 || K < 0) return msda_b200_internal_fail(MSDA_B200_ERR_INVALID, "point_sample: negative row / point count");
   if (R > 0x7fffffffll) return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "point_sample: more than 2^31-1 rows");
@@ -194,8 +184,7 @@ extern "C" int msda_b200_point_sample_forward(const void* const* planes, const m
     return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "point_sample: rows x points exceeds the grid limit");
   point_sample_fwd_kernel<<<(unsigned)(R * chunks), kPsThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       planes, rows, reinterpret_cast<const float2*>(coords), out, K, chunks);
-  msda_b200_internal_count_launch();
-  return check("point_sample_forward");
+  return launched("point_sample_forward");
 }
 
 extern "C" int msda_b200_point_sample_backward(float* const* grad_planes, const msda_b200_ps_row* rows,
@@ -208,8 +197,7 @@ extern "C" int msda_b200_point_sample_backward(float* const* grad_planes, const 
     return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "point_sample: rows x points exceeds the grid limit");
   point_sample_bwd_kernel<<<(unsigned)(R * chunks), kPsThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       grad_planes, rows, reinterpret_cast<const float2*>(coords), grad_out, K, chunks);
-  msda_b200_internal_count_launch();
-  return check("point_sample_backward");
+  return launched("point_sample_backward");
 }
 
 extern "C" size_t msda_b200_point_sample_backward_det_workspace_bytes(int64_t R, int32_t K, int64_t keys) {
@@ -240,14 +228,12 @@ extern "C" int msda_b200_point_sample_backward_det(float* const* grad_planes, co
       grad_planes, rows, key_base, keys, reinterpret_cast<const float2*>(coords),
       grad_out, K, chunks, reinterpret_cast<unsigned*>(ws + lay.keys_off[0]),
       reinterpret_cast<unsigned long long*>(ws + lay.vals_off[0]));
-  msda_b200_internal_count_launch();
-  if (int rc = check("point_sample_backward_det")) return rc;
+  if (int rc = launched("point_sample_backward_det: records")) return rc;
   const unsigned* sorted_keys = nullptr;
   const unsigned long long* sorted_vals = nullptr;
   if (int rc = msda_b200_internal_det_sort(&lay, workspace, &sorted_keys, &sorted_vals, st)) return rc;
   const int n = (int)lay.records;
   point_sample_bwd_det_sum_kernel<<<(n + kPsThreads - 1) / kPsThreads, kPsThreads, 0, st>>>(
       grad_planes, key_base, sorted_keys, sorted_vals, n, (unsigned)keys);
-  msda_b200_internal_count_launch();
-  return check("point_sample_backward_det");
+  return launched("point_sample_backward_det: sums");
 }

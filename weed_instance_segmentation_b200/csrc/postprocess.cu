@@ -30,9 +30,7 @@
 
 #include "bilinear_index.cuh"
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
-extern "C" void msda_b200_internal_count_launch(void);               // msda_b200.cu: launch counter
+#include "internal.h"
 
 namespace {
 
@@ -211,12 +209,6 @@ pp_binary_maps_kernel(const uint32_t* __restrict__ bits, const int32_t* __restri
     out[i * plane + p] = s_sel[i] >= 0 && mask_bit(bits, b * Q + s_sel[i], r, c) ? 1.f : 0.f;
 }
 
-int launched() {
-  msda_b200_internal_count_launch();
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
-}
-
 // 0 when (B, Q) is valid, else the failure code (message set).
 int check_bq(int32_t B, int32_t Q) {
   if (B <= 0 || Q <= 0) return msda_b200_internal_fail(MSDA_B200_ERR_INVALID, "postprocess: B and Q must be positive");
@@ -258,7 +250,7 @@ extern "C" int msda_b200_postprocess_scores(const void* mask_logits, int32_t dty
     pp_score_kernel<__nv_bfloat16><<<blocks, kScoreThreads, 0, s>>>(static_cast<const __nv_bfloat16*>(mask_logits),
                                                                      topk_index, target_hw, Q, C, h, w, sh, sw,
                                                                      mask_score, bits, nonempty);
-  return launched();
+  return launched("postprocess_scores");
 }
 
 extern "C" int msda_b200_postprocess_paint(const void* workspace, size_t workspace_bytes, const float* pred_score,
@@ -275,7 +267,7 @@ extern "C" int msda_b200_postprocess_paint(const void* workspace, size_t workspa
   const int32_t* nonempty = reinterpret_cast<const int32_t*>(static_cast<const char*>(workspace) + bits_bytes(B, Q));
   pp_paint_kernel<<<dim3((unsigned)max_h, (unsigned)B), kPaintThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       bits, nonempty, pred_score, labels, threshold, target_hw, Q, maps, table);
-  return launched();
+  return launched("postprocess_paint");
 }
 
 extern "C" int msda_b200_postprocess_binary_maps(const void* workspace, size_t workspace_bytes, const int32_t* table,
@@ -296,5 +288,5 @@ extern "C" int msda_b200_postprocess_binary_maps(const void* workspace, size_t w
     return msda_b200_internal_fail(MSDA_B200_ERR_UNSUPPORTED, "postprocess_binary_maps: map too large");
   pp_binary_maps_kernel<<<(unsigned)blocks, kMapThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       static_cast<const uint32_t*>(workspace), table, image, Q, H, W, n_inst, out);
-  return launched();
+  return launched("postprocess_binary_maps");
 }

@@ -15,9 +15,7 @@
 
 #include "bilinear_index.cuh"
 #include "msda_b200.h"
-
-extern "C" int msda_b200_internal_fail(int code, const char* msg);  // msda_b200.cu: sets msda_b200_last_error()
-extern "C" void msda_b200_internal_count_launch(void);               // msda_b200.cu: launch counter
+#include "internal.h"
 
 namespace {
 
@@ -76,7 +74,5 @@ extern "C" int msda_b200_resize_bilinear_backward(const float* grad_out, float* 
   const long long blocks = (total + kRbThreads - 1) / kRbThreads;
   resize_bilinear_bwd_kernel<<<(unsigned)blocks, kRbThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       grad_out, grad_in, total, Hi, Wi, Ho, Wo, (float)Hi / Ho, (float)Wi / Wo);
-  msda_b200_internal_count_launch();
-  const cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MSDA_B200_OK : msda_b200_internal_fail(MSDA_B200_ERR_CUDA, cudaGetErrorString(e));
+  return launched("resize_bilinear_backward");
 }

@@ -24,9 +24,9 @@ from typing import Sequence
 import torch
 
 from . import _cabi
+from ._cabi import DTYPE_CODE, ptr
 from ._cabi import MSDAError  # noqa: F401  (re-export)
 
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
 # Scheduling knobs (results never depend on them).
 def _parse_tile(text):
@@ -156,7 +156,7 @@ def _check_inputs(value, shapes, loc, attn):
     if total > S:
         # M2F:942-945 ("Make sure to align the spatial shapes with the sequence length ...")
         raise ValueError(f"spatial shapes cover {total} rows but value has S={S}")
-    if value.dtype not in _DTYPE_CODE:
+    if value.dtype not in DTYPE_CODE:
         raise TypeError(f"value dtype {value.dtype} unsupported (float32 or bfloat16)")
     return B, S, Q, H, D, L, P
 
@@ -167,13 +167,9 @@ def _prepare(value, loc, attn):
     loc = loc.contiguous() if loc.dtype == torch.float32 else loc.float().contiguous()
     if value.dtype == torch.float32 and attn.dtype != torch.float32:
         attn = attn.float()
-    elif attn.dtype not in _DTYPE_CODE:
+    elif attn.dtype not in DTYPE_CODE:
         attn = attn.to(value.dtype)
     return value, loc, attn.contiguous()
-
-
-def _ptr(t):
-    return t.data_ptr() if t is not None and t.numel() else None
 
 
 class MSDeformAttnFunction(torch.autograd.Function):
@@ -187,12 +183,12 @@ class MSDeformAttnFunction(torch.autograd.Function):
         B, S, H, D = value_c.shape
         _, Q, _, L, P, _ = loc_c.shape
         out = torch.empty((B, Q, H * D), dtype=value_c.dtype, device=value_c.device)
-        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value_c.dtype], _DTYPE_CODE[attn_c.dtype],
+        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, DTYPE_CODE[value_c.dtype], DTYPE_CODE[attn_c.dtype],
                                      shapes, level_start, flags)
         with torch.cuda.device(value_c.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_forward(desc, _ptr(value_c), _ptr(loc_c), _ptr(attn_c), _ptr(out),
-                                              _ptr(query_order), stream))
+            _cabi.check(lib.msda_b200_forward(desc, ptr(value_c), ptr(loc_c), ptr(attn_c), ptr(out),
+                                              ptr(query_order), stream))
         ctx.save_for_backward(value_c, loc_c, attn_c, query_order)
         ctx.geom = (shapes, level_start, flags, in_dtypes)
         del keep
@@ -208,7 +204,7 @@ class MSDeformAttnFunction(torch.autograd.Function):
         _, Q, _, L, P, _ = loc.shape
         grad_out = grad_out.to(value.dtype).contiguous()
         flags |= _backward_flags(deterministic())
-        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value.dtype], _DTYPE_CODE[attn.dtype],
+        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, DTYPE_CODE[value.dtype], DTYPE_CODE[attn.dtype],
                                      shapes, level_start, flags)
         grad_value = torch.empty_like(value)
         grad_loc = torch.empty_like(loc)
@@ -217,9 +213,9 @@ class MSDeformAttnFunction(torch.autograd.Function):
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=value.device) if ws_bytes else None
         with torch.cuda.device(value.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_backward(desc, _ptr(value), _ptr(loc), _ptr(attn), _ptr(grad_out),
-                                               _ptr(grad_value), _ptr(grad_loc), _ptr(grad_attn),
-                                               _ptr(ws), ws_bytes, _ptr(query_order), stream))
+            _cabi.check(lib.msda_b200_backward(desc, ptr(value), ptr(loc), ptr(attn), ptr(grad_out),
+                                               ptr(grad_value), ptr(grad_loc), ptr(grad_attn),
+                                               ptr(ws), ws_bytes, ptr(query_order), stream))
         del keep
         if grad_loc.dtype != loc_dtype:
             grad_loc = grad_loc.to(loc_dtype)

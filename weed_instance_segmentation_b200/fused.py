@@ -21,9 +21,8 @@ from __future__ import annotations
 import torch
 
 from . import _cabi
+from ._cabi import DTYPE_CODE, ptr
 from . import functional as F
-
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
 
 def _aux_dtype(value, offsets, logits):
@@ -49,11 +48,11 @@ class MSDeformAttnFusedFunction(torch.autograd.Function):
         _, Q, _, L, P, _ = offsets_c.shape
         out = torch.empty((B, Q, H * D), dtype=value_c.dtype, device=value_c.device)
         attn = torch.empty((B, Q, H, L, P), dtype=torch.float32, device=value_c.device) if want_attn else None
-        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value_c.dtype], _DTYPE_CODE[aux], shapes, level_start)
+        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, DTYPE_CODE[value_c.dtype], DTYPE_CODE[aux], shapes, level_start)
         with torch.cuda.device(value_c.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_forward_fused(desc, F._ptr(value_c), F._ptr(offsets_c), F._ptr(logits_c),
-                                                    F._ptr(ref_c), F._ptr(out), F._ptr(attn), F._ptr(query_order), stream))
+            _cabi.check(lib.msda_b200_forward_fused(desc, ptr(value_c), ptr(offsets_c), ptr(logits_c),
+                                                    ptr(ref_c), ptr(out), ptr(attn), ptr(query_order), stream))
         ctx.save_for_backward(value_c, offsets_c, logits_c, ref_c, query_order)
         ctx.geom = (shapes, level_start, in_dtypes)
         del keep
@@ -71,7 +70,7 @@ class MSDeformAttnFusedFunction(torch.autograd.Function):
         B, S, H, D = value.shape
         _, Q, _, L, P, _ = offsets.shape
         flags = F._backward_flags(F.deterministic())
-        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, _DTYPE_CODE[value.dtype], _DTYPE_CODE[offsets.dtype],
+        desc, keep = _cabi.make_desc(B, S, Q, H, D, L, P, DTYPE_CODE[value.dtype], DTYPE_CODE[offsets.dtype],
                                      shapes, level_start, flags)
         grad_out = grad_out.to(value.dtype).contiguous()
         grad_value = torch.empty_like(value)
@@ -81,9 +80,9 @@ class MSDeformAttnFusedFunction(torch.autograd.Function):
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=value.device) if ws_bytes else None
         with torch.cuda.device(value.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_backward_fused(desc, F._ptr(value), F._ptr(offsets), F._ptr(logits), F._ptr(ref),
-                                                     F._ptr(grad_out), F._ptr(grad_value), F._ptr(grad_offsets),
-                                                     F._ptr(grad_logits), F._ptr(ws), ws_bytes, F._ptr(query_order), stream))
+            _cabi.check(lib.msda_b200_backward_fused(desc, ptr(value), ptr(offsets), ptr(logits), ptr(ref),
+                                                     ptr(grad_out), ptr(grad_value), ptr(grad_offsets),
+                                                     ptr(grad_logits), ptr(ws), ws_bytes, ptr(query_order), stream))
         del keep
         if grad_offsets.dtype != off_dtype:
             grad_offsets = grad_offsets.to(off_dtype)
@@ -135,7 +134,7 @@ def ms_deform_attn_fused(value, value_spatial_shapes, level_start_index, samplin
             raise ValueError("ms_deform_attn_fused does not differentiate with respect to reference_points")
     if sum(h * w for h, w in shapes) > S:
         raise ValueError(f"spatial shapes cover more rows than value has (S={S})")
-    if value.dtype not in _DTYPE_CODE:
+    if value.dtype not in DTYPE_CODE:
         raise TypeError(f"value dtype {value.dtype} unsupported (float32 or bfloat16)")
     level_start = F._level_start(shapes, level_start_index)
     order = None

@@ -14,8 +14,7 @@ from typing import Sequence
 import torch
 
 from . import _cabi, functional
-
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
+from ._cabi import DTYPE_CODE
 
 
 class HostPipeline:
@@ -42,14 +41,14 @@ class HostPipeline:
         self.Q = self.S if num_queries is None else int(num_queries)
         self.value_dtype = value_dtype
         self.attn_dtype = value_dtype if attn_dtype is None else attn_dtype
-        if self.value_dtype not in _DTYPE_CODE or self.attn_dtype not in _DTYPE_CODE:
+        if self.value_dtype not in DTYPE_CODE or self.attn_dtype not in DTYPE_CODE:
             raise TypeError("HostPipeline: float32 or bfloat16 tensors only")
         self.backward = bool(backward)
         self.deterministic = functional.deterministic() if deterministic is None else bool(deterministic)
         flags = functional._backward_flags(self.deterministic)
         lsi = functional._level_start(self.shapes, None)
         desc, self._keep = _cabi.make_desc(self.B, self.S, self.Q, self.H, self.D, self.L, self.P,
-                                           _DTYPE_CODE[self.value_dtype], _DTYPE_CODE[self.attn_dtype], self.shapes, lsi,
+                                           DTYPE_CODE[self.value_dtype], DTYPE_CODE[self.attn_dtype], self.shapes, lsi,
                                            flags)
         # the 2-D query order is a scheduling hint for one-query-per-pixel problems (functional.query_order_2d)
         self._order = (functional.query_order_2d(self.shapes, functional._TILE, self.device)

@@ -10,12 +10,7 @@ from __future__ import annotations
 import torch
 
 from . import _cabi
-
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
-
-
-def _ptr(t):
-    return t.data_ptr() if t is not None and t.numel() else None
+from ._cabi import DTYPE_CODE, ptr
 
 
 class AddLayerNormFunction(torch.autograd.Function):
@@ -34,14 +29,14 @@ class AddLayerNormFunction(torch.autograd.Function):
         with torch.cuda.device(xc.device):
             stream = torch.cuda.current_stream().cuda_stream
             if clamp is None:
-                _cabi.check(lib.msda_b200_add_layernorm_forward(_ptr(xc), _DTYPE_CODE[xc.dtype], _ptr(rc),
-                                                                _DTYPE_CODE[rc.dtype], _ptr(w), _ptr(b), float(eps), _ptr(y),
-                                                                _ptr(y_lowp), _ptr(mean), _ptr(rstd), rows, C, stream))
+                _cabi.check(lib.msda_b200_add_layernorm_forward(ptr(xc), DTYPE_CODE[xc.dtype], ptr(rc),
+                                                                DTYPE_CODE[rc.dtype], ptr(w), ptr(b), float(eps), ptr(y),
+                                                                ptr(y_lowp), ptr(mean), ptr(rstd), rows, C, stream))
             else:
-                _cabi.check(lib.msda_b200_add_layernorm_clamp_forward(_ptr(xc), _DTYPE_CODE[xc.dtype], _ptr(rc),
-                                                                      _DTYPE_CODE[rc.dtype], _ptr(w), _ptr(b), float(eps),
-                                                                      float(clamp), _ptr(y), _ptr(y_lowp), _ptr(mean),
-                                                                      _ptr(rstd), rows, C, stream))
+                _cabi.check(lib.msda_b200_add_layernorm_clamp_forward(ptr(xc), DTYPE_CODE[xc.dtype], ptr(rc),
+                                                                      DTYPE_CODE[rc.dtype], ptr(w), ptr(b), float(eps),
+                                                                      float(clamp), ptr(y), ptr(y_lowp), ptr(mean),
+                                                                      ptr(rstd), rows, C, stream))
         ctx.clamp = clamp
         ctx.save_for_backward(xc, rc, w, mean, rstd, *((b,) if clamp is not None else ()))
         ctx.param_dtypes = (weight.dtype, bias.dtype)
@@ -66,14 +61,14 @@ class AddLayerNormFunction(torch.autograd.Function):
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream().cuda_stream
             if ctx.clamp is None:
-                _cabi.check(lib.msda_b200_add_layernorm_backward(_ptr(gy), _ptr(gyl), _ptr(x), _DTYPE_CODE[x.dtype], _ptr(r),
-                                                                 _DTYPE_CODE[r.dtype], _ptr(w), _ptr(mean), _ptr(rstd),
-                                                                 _ptr(ds), _ptr(ds_lowp), _ptr(gw), _ptr(gb), rows, C, stream))
+                _cabi.check(lib.msda_b200_add_layernorm_backward(ptr(gy), ptr(gyl), ptr(x), DTYPE_CODE[x.dtype], ptr(r),
+                                                                 DTYPE_CODE[r.dtype], ptr(w), ptr(mean), ptr(rstd),
+                                                                 ptr(ds), ptr(ds_lowp), ptr(gw), ptr(gb), rows, C, stream))
             else:
                 _cabi.check(lib.msda_b200_add_layernorm_clamp_backward(
-                    _ptr(gy), _ptr(gyl), _ptr(x), _DTYPE_CODE[x.dtype], _ptr(r), _DTYPE_CODE[r.dtype], _ptr(w),
-                    _ptr(ctx.saved_tensors[5]), float(ctx.clamp), _ptr(mean), _ptr(rstd), _ptr(ds), _ptr(ds_lowp), _ptr(gw),
-                    _ptr(gb), rows, C, stream))
+                    ptr(gy), ptr(gyl), ptr(x), DTYPE_CODE[x.dtype], ptr(r), DTYPE_CODE[r.dtype], ptr(w),
+                    ptr(ctx.saved_tensors[5]), float(ctx.clamp), ptr(mean), ptr(rstd), ptr(ds), ptr(ds_lowp), ptr(gw),
+                    ptr(gb), rows, C, stream))
         gx = ds_lowp if x.dtype == torch.bfloat16 else ds
         gr = ds_lowp if r.dtype == torch.bfloat16 else ds
         wd, bd = ctx.param_dtypes
@@ -97,7 +92,7 @@ def add_layer_norm(x: torch.Tensor, residual: torch.Tensor, weight: torch.Tensor
         raise RuntimeError("add_layer_norm: tensors must live on a CUDA device (this package has no CPU fallback)")
     if x.shape != residual.shape:
         raise ValueError(f"add_layer_norm: x {tuple(x.shape)} and residual {tuple(residual.shape)} differ")
-    if x.dtype not in _DTYPE_CODE or residual.dtype not in _DTYPE_CODE:
+    if x.dtype not in DTYPE_CODE or residual.dtype not in DTYPE_CODE:
         raise TypeError("add_layer_norm: float32 or bfloat16 inputs only")
     C = x.shape[-1]
     if weight.numel() != C or bias.numel() != C:

@@ -13,9 +13,9 @@ import torch
 import torch.nn.functional as F
 
 from . import _cabi
+from ._cabi import DTYPE_CODE, ptr
 from .functional import deterministic
 
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
 # float32 projections on the bf16 tensor cores (csrc/gemm_f32.cu: cuBLASLt's CUBLAS_COMPUTE_32F_EMULATED_16BFX9, at least
 # SGEMM's accuracy at ~2x its speed). MSDA_B200_F32_GEMM=native keeps torch's SGEMM.
@@ -77,8 +77,8 @@ def column_sum(matrix: torch.Tensor) -> torch.Tensor:
     m = matrix.contiguous()
     out = torch.empty(C, dtype=torch.float32, device=m.device)
     with torch.cuda.device(m.device):
-        _cabi.check(lib.msda_b200_column_sum(m.data_ptr() if m.numel() else None, _DTYPE_CODE[m.dtype], out.data_ptr(),
-                                             m.numel() // C, C, torch.cuda.current_stream().cuda_stream))
+        _cabi.check(lib.msda_b200_column_sum(ptr(m), DTYPE_CODE[m.dtype], out.data_ptr(), m.numel() // C, C,
+                                             torch.cuda.current_stream().cuda_stream))
     return out
 
 
@@ -91,9 +91,8 @@ def relu_backward_column_sum(grad_y: torch.Tensor, y: torch.Tensor):
     out = torch.empty_like(g)
     col = torch.empty(C, dtype=torch.float32, device=g.device)
     with torch.cuda.device(g.device):
-        _cabi.check(lib.msda_b200_relu_backward_column_sum(g.data_ptr() if g.numel() else None, a.data_ptr() if a.numel() else None,
-                                                           _DTYPE_CODE[g.dtype], out.data_ptr() if out.numel() else None,
-                                                           col.data_ptr(), g.numel() // C, C,
+        _cabi.check(lib.msda_b200_relu_backward_column_sum(ptr(g), ptr(a), DTYPE_CODE[g.dtype],
+                                                           ptr(out), col.data_ptr(), g.numel() // C, C,
                                                            torch.cuda.current_stream().cuda_stream))
     return out, col
 
@@ -184,7 +183,7 @@ class LinearReLUFunction(torch.autograd.Function):
 def _kernel_ok(x, weight, bias) -> bool:
     dt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
     C = weight.shape[0]
-    return (x.is_cuda and bias is not None and dt in _DTYPE_CODE and C % (8 if dt == torch.bfloat16 else 4) == 0
+    return (x.is_cuda and bias is not None and dt in DTYPE_CODE and C % (8 if dt == torch.bfloat16 else 4) == 0
             and C <= (2048 if dt == torch.bfloat16 else 1024))
 
 
@@ -203,7 +202,7 @@ def linear(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor) -> torch.T
     """
     dt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
     C = weight.shape[0]
-    ok = (x.is_cuda and bias is not None and dt in _DTYPE_CODE and C % (8 if dt == torch.bfloat16 else 4) == 0
+    ok = (x.is_cuda and bias is not None and dt in DTYPE_CODE and C % (8 if dt == torch.bfloat16 else 4) == 0
           and C <= (2048 if dt == torch.bfloat16 else 1024))
     if not ok:
         return F.linear(x, weight, bias)
@@ -221,11 +220,8 @@ class QueryValueCastFunction(torch.autograd.Function):
         q = torch.empty(h.shape, dtype=torch.bfloat16, device=h.device)
         v = torch.empty(h.shape, dtype=torch.bfloat16, device=h.device)
         with torch.cuda.device(h.device):
-            _cabi.check(lib.msda_b200_query_value_cast_forward(h.data_ptr() if h.numel() else None,
-                                                               p.data_ptr() if p.numel() else None,
-                                                               q.data_ptr() if q.numel() else None,
-                                                               v.data_ptr() if v.numel() else None, h.numel(),
-                                                               torch.cuda.current_stream().cuda_stream))
+            _cabi.check(lib.msda_b200_query_value_cast_forward(ptr(h), ptr(p), ptr(q), ptr(v),
+                                                               h.numel(), torch.cuda.current_stream().cuda_stream))
         ctx.shape, ctx.device = h.shape, h.device
         return q, v
 
@@ -240,7 +236,6 @@ class QueryValueCastFunction(torch.autograd.Function):
         gv = grad_v.to(torch.bfloat16).contiguous() if grad_v is not None else None
         gh = torch.empty(ctx.shape, dtype=torch.float32, device=ctx.device)
         gp = torch.empty(ctx.shape, dtype=torch.float32, device=ctx.device) if need_p else None
-        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
         with torch.cuda.device(ctx.device):
             _cabi.check(lib.msda_b200_query_value_cast_backward(ptr(gq), ptr(gv), ptr(gh), ptr(gp), gh.numel(),
                                                                 torch.cuda.current_stream().cuda_stream))

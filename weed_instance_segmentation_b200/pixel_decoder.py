@@ -29,9 +29,8 @@ import torch
 from torch import nn
 
 from . import _cabi
+from ._cabi import DTYPE_CODE, ptr
 from .functional import deterministic
-
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
 
 
 class _GroupNormToRows(torch.autograd.Function):
@@ -54,7 +53,7 @@ class _GroupNormToRows(torch.autograd.Function):
             start = 0
             for x, g, b, st, hw in zip(xs, gammas, betas, stats, hws):
                 _cabi.check(lib.msda_b200_groupnorm_to_rows_forward(
-                    x.data_ptr(), _DTYPE_CODE[x.dtype], g.data_ptr(), b.data_ptr(), float(eps),
+                    x.data_ptr(), DTYPE_CODE[x.dtype], g.data_ptr(), b.data_ptr(), float(eps),
                     out.data_ptr() + start * C * 4, S * C, st.data_ptr(), B, C, hw, groups, stream))
                 start += hw
         ctx.save_for_backward(*xs, *gammas, *stats)
@@ -80,7 +79,7 @@ class _GroupNormToRows(torch.autograd.Function):
                 gb = torch.zeros(C, dtype=torch.float32, device=x.device)
                 scratch = torch.empty(B * groups * 2, dtype=torch.float32, device=x.device)
                 _cabi.check(lib.msda_b200_groupnorm_to_rows_backward(
-                    grad_out.data_ptr() + start * C * 4, S * C, x.data_ptr(), _DTYPE_CODE[x.dtype], g.data_ptr(),
+                    grad_out.data_ptr() + start * C * 4, S * C, x.data_ptr(), DTYPE_CODE[x.dtype], g.data_ptr(),
                     st.data_ptr(), gx.data_ptr(), gg.data_ptr(), gb.data_ptr(), scratch.data_ptr(), B, C, hw, groups, stream))
                 start += hw
                 gxs.append(gx)
@@ -97,7 +96,7 @@ def groupnorm_to_rows(xs, norms) -> torch.Tensor:
     groups, eps = norms[0].num_groups, norms[0].eps
     if any(n.num_groups != groups or n.eps != eps or not n.affine for n in norms):
         raise ValueError("groupnorm_to_rows: the levels must share num_groups / eps and be affine")
-    if any(x.dtype not in _DTYPE_CODE for x in xs):
+    if any(x.dtype not in DTYPE_CODE for x in xs):
         raise TypeError("groupnorm_to_rows: float32 or bfloat16 inputs")
     return _GroupNormToRows.apply(eps, groups, *xs, *[n.weight for n in norms], *[n.bias for n in norms])
 
@@ -174,8 +173,7 @@ class _ResizeBilinear(torch.autograd.Function):
         grad_in = torch.empty((n, c, hi, wi), dtype=torch.float32, device=go.device)
         with torch.cuda.device(go.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_resize_bilinear_backward(go.data_ptr() if go.numel() else None,
-                                                               grad_in.data_ptr() if grad_in.numel() else None, n * c,
+            _cabi.check(lib.msda_b200_resize_bilinear_backward(ptr(go), ptr(grad_in), n * c,
                                                                hi, wi, go.shape[2], go.shape[3], stream))
         return grad_in.to(dtype), None
 

@@ -22,7 +22,7 @@ import torch
 from . import _cabi
 from .functional import deterministic
 
-_DTYPE_CODE = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16, torch.uint8: _cabi.U8, torch.bool: _cabi.U8}
+_DTYPE_CODE = {**_cabi.DTYPE_CODE, torch.uint8: _cabi.U8, torch.bool: _cabi.U8}
 
 
 class _Rows:
@@ -86,10 +86,8 @@ class PointSampleFunction(torch.autograd.Function):
         out = torch.empty((table.R, K), dtype=torch.float32, device=coords.device)
         with torch.cuda.device(coords.device):
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(lib.msda_b200_point_sample_forward(table.ptr.data_ptr() if table.R else None,
-                                                           table.rows.data_ptr() if table.R else None,
-                                                           coords.data_ptr() if coords.numel() else None,
-                                                           out.data_ptr() if out.numel() else None, table.R, K, stream))
+            _cabi.check(lib.msda_b200_point_sample_forward(_cabi.ptr(table.ptr), _cabi.ptr(table.rows),
+                                                           _cabi.ptr(coords), _cabi.ptr(out), table.R, K, stream))
         ctx.table = table
         ctx.save_for_backward(coords)
         ctx.src_meta = [(s.shape, s.dtype) for s in sources]
@@ -136,7 +134,7 @@ def _backward_det(lib, table: _Rows, grads, coords, go, K, stream) -> None:
     ws = torch.empty(nbytes, dtype=torch.uint8, device=go.device) if nbytes else None  # 0: the call reports why
     _cabi.check(lib.msda_b200_point_sample_backward_det(gptr.data_ptr(), rows.data_ptr(), key_base.data_ptr(), keys,
                                                         coords.data_ptr(), go.data_ptr(), R, K,
-                                                        ws.data_ptr() if nbytes else None, nbytes, stream))
+                                                        _cabi.ptr(ws), nbytes, stream))
 
 
 def point_sample(sources: Sequence[torch.Tensor], src_id, plane_id, coords: torch.Tensor, coord_row) -> torch.Tensor:

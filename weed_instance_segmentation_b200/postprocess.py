@@ -18,8 +18,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-
-_DTYPES = {torch.float32: _cabi.F32, torch.bfloat16: _cabi.BF16}
+from ._cabi import DTYPE_CODE
 
 
 def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_threshold: float = 0.5,
@@ -43,7 +42,7 @@ def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_thr
         raise RuntimeError("post_process_instance_segmentation: outputs must live on one CUDA device "
                            "(this package has no CPU fallback)")
     for name, t in (("class_queries_logits", cls), ("masks_queries_logits", masks)):
-        if t.dtype not in _DTYPES:
+        if t.dtype not in DTYPE_CODE:
             raise TypeError(f"post_process_instance_segmentation: {name} has dtype {t.dtype}; float32 or bfloat16 only")
     if cls.dim() != 3 or masks.dim() != 4 or masks.shape[:2] != cls.shape[:2] or cls.shape[-1] < 2:
         raise ValueError(f"post_process_instance_segmentation: class logits {tuple(cls.shape)} (B, Q, C+1 >= 2) and "
@@ -81,7 +80,7 @@ def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_thr
         workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         mask_score = torch.empty((B, Q), dtype=torch.float32, device=dev)
         _cabi.check(lib.msda_b200_postprocess_scores(
-            masks.data_ptr(), _DTYPES[masks.dtype], topk_index.data_ptr(), C, hw.data_ptr(), B, Q, masks.shape[2],
+            masks.data_ptr(), DTYPE_CODE[masks.dtype], topk_index.data_ptr(), C, hw.data_ptr(), B, Q, masks.shape[2],
             masks.shape[3], mask_score.data_ptr(), workspace.data_ptr(), ws_bytes, stream))
         pred_scores = (scores_per_image * mask_score).contiguous()  # float32 for either class-logit dtype
         n_map = sum(h * w for h, w in sizes)
