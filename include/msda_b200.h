@@ -93,7 +93,7 @@ typedef struct msda_b200_desc {
   int32_t H;           /* heads                                                                  */
   int32_t D;           /* channels per head: 8, 16, 32, 64, 128                                  */
   int32_t L;           /* levels, 1..MSDA_B200_MAX_LEVELS                                        */
-  int32_t P;           /* points per level                                                       */
+  int32_t P;           /* points per level; L*P <= 64 (backward: see below)                      */
   int32_t value_dtype; /* MSDA_B200_F32 | MSDA_B200_BF16: value, out, grad_out, grad_value       */
   int32_t attn_dtype;  /* MSDA_B200_F32 | MSDA_B200_BF16: attn, grad_attn                        */
   uint32_t flags;      /* MSDA_B200_FLAG_*                                                       */
@@ -129,6 +129,12 @@ size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc);
  * grad_loc (B,Q,H,L,P,2) float32 and grad_attn (B,Q,H,L,P).
  * grad_value is summed with unordered float atomics, so its last bits vary from run to run; set
  * MSDA_B200_FLAG_DETERMINISTIC for run-to-run identical gradients.
+ * Geometry: the forward takes every L*P <= 64.  The backward's per-corner kernel holds the L*P samples of 128 / LPP
+ * queries (LPP = D * sizeof(value) / 16) in shared memory, at most 227 KB per block, so small head dims allow less:
+ *   fp32 D = 8: L*P <= 50 (fused backward: 45);  bf16 D = 8: L*P <= 32 (28);  bf16 D = 16: L*P <= 50 (45);
+ *   every other (dtype, D): L*P <= 64.
+ * Past its limit msda_b200_backward and msda_b200_backward_fused return MSDA_B200_ERR_UNSUPPORTED before any CUDA
+ * call, as does msda_b200_host_pipeline_create with a backward; msda_b200_backward_workspace_bytes returns 0.
  */
 int msda_b200_backward(const msda_b200_desc* desc, const void* value /*dev*/, const float* loc /*dev*/,
                        const void* attn /*dev*/, const void* grad_out /*dev*/, void* grad_value /*dev*/,

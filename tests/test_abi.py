@@ -79,6 +79,47 @@ def test_validation_without_gpu_rejects_retired_flags(lib):
     assert lib.msda_b200_forward(d, None, None, None, None, None, None) == 0
 
 
+# (value dtype, D, largest L*P of the backward, of the fused backward): the per-corner backward kernel keeps the L*P
+# samples of 128 / LPP queries in shared memory, at most 227 KB per block
+BACKWARD_LIMITS = [("f32", 8, 50, 45), ("bf16", 8, 32, 28), ("bf16", 16, 50, 45)]
+
+
+@pytest.mark.parametrize("vdt,D,plain,fused", BACKWARD_LIMITS, ids=[f"{v}_d{D}" for v, D, _, _ in BACKWARD_LIMITS])
+def test_backward_shared_memory_limit_is_checked_before_the_device(lib, vdt, D, plain, fused):
+    """One L*P past the backward's limit is refused as unsupported, naming the limit, before any CUDA call -- by the
+    backward, the fused backward, the deterministic backward, the workspace query and a host pipeline with a backward;
+    at the limit the geometry passes the check (the calls fail later, on their NULL tensors)."""
+    from weed_instance_segmentation_b200 import _cabi
+    code = _cabi.BF16 if vdt == "bf16" else _cabi.F32
+    for flags in (0, _cabi.FLAG_DETERMINISTIC):
+        for lp, fused_entry in ((plain, False), (fused, True)):
+            for p, refused in ((lp + 1, True), (lp, False)):
+                d, keep = _cabi.make_desc(1, 16, 16, 1, D, 1, p, code, code, [(4, 4)], [0], flags)
+                if fused_entry:
+                    rc = lib.msda_b200_backward_fused(d, *([None] * 9 + [0, None, None]))
+                else:
+                    rc = lib.msda_b200_backward(d, *([None] * 8 + [0, None, None]))
+                msg = lib.msda_b200_last_error()
+                tag = f"flags={flags} fused={fused_entry} L*P={p}"
+                if refused:
+                    assert rc == 2, (tag, msg)
+                    assert b"227 KB" in msg and f"at most L*P={lp} ".encode() in msg, (tag, msg)
+                else:
+                    assert rc == 1 and b"grad_value is NULL" in msg, (tag, msg)
+    d, keep = _cabi.make_desc(1, 16, 16, 1, D, 1, plain + 1, code, code, [(4, 4)], [0])
+    assert lib.msda_b200_backward_workspace_bytes(d) == 0
+    d.flags = _cabi.FLAG_DETERMINISTIC
+    assert lib.msda_b200_backward_workspace_bytes(d) == 0
+    assert b"227 KB" in lib.msda_b200_last_error()
+    d.flags = 0
+    handle = ctypes.c_void_p()
+    assert lib.msda_b200_host_pipeline_create(ctypes.byref(d), 1, 2, 1, None, ctypes.byref(handle)) == 2
+    assert b"227 KB" in lib.msda_b200_last_error() and not handle.value
+    if code == _cabi.BF16:
+        d, keep = _cabi.make_desc(1, 16, 16, 1, D, 1, plain, code, code, [(4, 4)], [0])
+        assert lib.msda_b200_backward_workspace_bytes(d) == 16 * D * 4
+
+
 def test_no_cpu_fallback():
     import torch
     import weed_instance_segmentation_b200 as wis

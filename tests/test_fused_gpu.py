@@ -65,13 +65,23 @@ def _kink_mask(off, ref, shapes, eps=1e-3):
     return ((pix - pix.round()).abs() > eps).all(-1).numpy()
 
 
+FIVE_LEVELS = [(3, 3), (5, 5), (9, 9), (17, 17), (33, 33)]
+EIGHT_LEVELS = [(2, 2), (3, 3), (4, 4), (5, 5), (6, 7), (8, 8), (11, 9), (16, 16)]
+
 CASES = [
     # (tag, B, shapes, H, D, P, Q)  -- D=32 & P=4 in bf16 takes the group-sorted backward, the rest v1
     ("m2f", 2, [(8, 8), (16, 16), (32, 32)], 8, 32, 4, None),
     ("odd", 1, [(7, 9), (13, 18), (25, 35)], 8, 32, 4, None),
     ("ragged_p3", 2, [(5, 7), (9, 4)], 4, 32, 3, 77),
     ("d64", 1, [(6, 6), (12, 12)], 4, 64, 2, 50),
+    # L*P > 16: the forward's three-pass softmax; L >= 5 levels in the group-sorted backward's closing loop
+    ("l5p4", 1, FIVE_LEVELS, 4, 32, 4, None),
+    ("l8p4", 1, EIGHT_LEVELS, 2, 32, 4, None),
+    ("l8p8", 1, EIGHT_LEVELS, 2, 32, 8, 90),  # L*P = 64, the most validate() takes
+    ("d16", 2, [(6, 6), (12, 12)], 8, 16, 4, None),
+    ("d128", 1, [(6, 6), (12, 12)], 2, 128, 4, 50),
 ]
+BF16_CASES = CASES[:3] + [c for c in CASES if c[0] in ("d64", "l5p4", "l8p4", "l8p8", "d128")]
 
 
 @pytest.fixture(scope="module")
@@ -100,7 +110,7 @@ def test_fused_fp32(wis, case, dist):
         assert e <= 4e-5, f"{tag}/{dist}: {name} rel err {e:.3e}"
 
 
-@pytest.mark.parametrize("case", CASES[:3], ids=[c[0] for c in CASES[:3]])
+@pytest.mark.parametrize("case", BF16_CASES, ids=[c[0] for c in BF16_CASES])
 def test_fused_bf16(wis, case):
     tag, B, shapes, H, D, P, Q = case
     value, off, logits, ref, go = _inputs(B, shapes, H, D, P, Q, seed=4)
@@ -113,6 +123,71 @@ def test_fused_bf16(wis, case):
             g, w = g * safe, w * safe
         e = rel_err(g.reshape(w.shape), w)
         assert e <= 2e-2, f"{tag}: {name} rel err {e:.3e}"
+
+
+# bf16, D = 32, P = 4: the group-sorted backward by default; three and five levels
+COMMON_MODE_GEOMS = [
+    ("l3", 1, [(8, 8), (16, 16), (32, 32)], 8, 32, 4, None),
+    ("l5", 1, FIVE_LEVELS, 4, 32, 4, None),
+]
+COMMON_MODE_PARAMS = [(g, mu, peaked, torch.bfloat16) for g in COMMON_MODE_GEOMS for mu in (0.0, 3.0, 10.0)
+                      for peaked in (False, True)] + [(COMMON_MODE_GEOMS[1], 10.0, True, torch.float32)]
+
+
+def _common_mode_inputs(case, mu, peaked, seed=17):
+    """value = mu + randn; with `peaked`, one logit of every (query, head) row raised by 8 (its weight close to 1)."""
+    tag, B, shapes, H, D, P, Q = case
+    value, off, logits, ref, go = _inputs(B, shapes, H, D, P, Q, seed=seed)
+    if peaked:
+        j = torch.randint(0, logits.shape[-1], logits.shape[:-1] + (1,), generator=torch.Generator().manual_seed(seed))
+        logits = logits.scatter_add(-1, j, torch.full(j.shape, 8.0))
+    return value + mu, off, logits, ref, go
+
+
+@pytest.mark.parametrize("case,mu,peaked,dtype", COMMON_MODE_PARAMS,
+                         ids=[f"{g[0]}-mu{mu:g}-{'peaked' if pk else 'spread'}-{'fp32' if dt == torch.float32 else 'bf16'}"
+                              for g, mu, pk, dt in COMMON_MODE_PARAMS])
+def test_fused_softmax_backward_common_mode(wis, monkeypatch, case, mu, peaked, dtype):
+    """grad_logits = a_j * (ga_j - sum_k a_k ga_k) cancels whenever the L*P attention gradients ga of a row share a
+    common part: value rows with a non-zero mean (ga ~ mu * <grad_out, 1>) or one dominant logit. The result must come
+    from fp32 ga (one rounding to the logits' dtype) in every backward the fused entry point runs: the default (the
+    group-sorted kernel in bf16), the per-corner kernel and the deterministic one."""
+    from weed_instance_segmentation_b200 import functional as F
+    tag, B, shapes, H, D, P, Q = case
+    value, off, logits, ref, go = _common_mode_inputs(case, mu, peaked)
+    value, off, logits, go = (t.to(dtype) for t in (value, off, logits, go))  # reference points stay fp32
+    want = _reference_chain(value.float(), off.float(), logits.float(), ref, go.float(), shapes)
+    safe = _kink_mask(off.float(), ref, shapes)[..., None]
+    bars = {"grad_logits": 1e-2} if dtype == torch.bfloat16 else {}
+    for mode in ("default", "per_corner", "deterministic"):
+        monkeypatch.setattr(F, "_BWD_V1", mode == "per_corner")
+        prev = torch.are_deterministic_algorithms_enabled()
+        torch.use_deterministic_algorithms(mode == "deterministic")
+        try:
+            got = _run_fused(wis, value, off, logits, ref, go, shapes)
+        finally:
+            torch.use_deterministic_algorithms(prev)
+        for name, g, w in zip(("out", "grad_value", "grad_offsets", "grad_logits"), got, want):
+            if name == "grad_offsets":
+                g, w = g * safe, w * safe
+            e = rel_err(g.reshape(w.shape), w)
+            bar = bars.get(name, 2e-2 if dtype == torch.bfloat16 else 4e-5)
+            assert e <= bar, f"{mode}: {name} rel err {e:.3e} > {bar:g}"
+
+
+def test_fused_softmax_backward_common_mode_full_size(wis, monkeypatch):
+    """BASELINE config 2 geometry (B = 2) in bf16 with value = 10 + randn: grad_logits of the default (group-sorted)
+    backward against the per-corner one, which keeps ga in fp32; each carries one bf16 rounding of the result."""
+    from weed_instance_segmentation_b200 import functional as F
+    shapes = [(32, 32), (64, 64), (128, 128)]
+    value, off, logits, ref, go = _inputs(2, shapes, 8, 32, 4, None, seed=23)
+    args = ((value + 10.0).bfloat16(), off.bfloat16(), logits.bfloat16(), ref, go.bfloat16(), shapes)
+    grad_logits = []
+    for per_corner in (False, True):
+        monkeypatch.setattr(F, "_BWD_V1", per_corner)
+        grad_logits.append(_run_fused(wis, *args)[3])
+    e = rel_err(grad_logits[0], grad_logits[1])
+    assert e <= 1e-2, f"grad_logits: group-sorted vs per-corner rel err {e:.3e}"
 
 
 def test_fused_matches_unfused_bitwise_forward(wis):

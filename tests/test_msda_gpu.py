@@ -112,7 +112,11 @@ CASES = [
     ("d64", 2, [(6, 6), (12, 12)], 4, 64, 2, 50),
     ("one_pixel_levels", 2, [(1, 1), (1, 9), (7, 1), (4, 4)], 2, 32, 2, 33),
     ("many_points", 1, [(8, 8)], 2, 32, 16, None),
+    ("d128", 1, [(6, 6), (12, 12)], 2, 128, 4, 40),
+    ("d8", 2, [(6, 6), (12, 12)], 4, 8, 4, None),
 ]
+# bf16: the model's geometry, and every head dim besides 32 (the per-corner backward at D = 8, 16, 64, 128)
+BF16_CASES = CASES[:4] + [c for c in CASES if c[0] in ("d64", "d128", "d8")]
 
 
 @pytest.mark.parametrize("dist", ["init", "trained", "adversarial"])
@@ -130,7 +134,7 @@ def test_random_fp32(wis, case, dist):
 
 @pytest.mark.parametrize("attn_dtype", [torch.bfloat16, torch.float32], ids=["attn_bf16", "attn_f32"])
 @pytest.mark.parametrize("dist", ["init", "trained", "adversarial"])
-@pytest.mark.parametrize("case", CASES[:4], ids=[c[0] for c in CASES[:4]])
+@pytest.mark.parametrize("case", BF16_CASES, ids=[c[0] for c in BF16_CASES])
 def test_random_bf16(wis, case, dist, attn_dtype):
     from weed_instance_segmentation_b200.synth import msda_inputs
     tag, B, shapes, H, D, P, Q = case
@@ -164,11 +168,14 @@ def test_sorted_backward_windows(wis, case, dist):
                   safe=_kink_safe(x["sampling_locations"].numpy(), shapes))
 
 
+VARIANT_CASES = SORTED_CASES[:2] + [CASES[1]] + [c for c in CASES if c[0] in ("d64", "d128")]
+
+
 @pytest.mark.parametrize("variant", ["v1", "v3"])
-@pytest.mark.parametrize("case", SORTED_CASES[:2] + [CASES[1]], ids=[c[0] for c in SORTED_CASES[:2] + [CASES[1]]])
+@pytest.mark.parametrize("case", VARIANT_CASES, ids=[c[0] for c in VARIANT_CASES])
 def test_every_backward_variant_matches_oracle(wis, monkeypatch, case, variant):
     """Both bf16 backward kernels -- v1 per-corner reductions (MSDA_B200_FLAG_BWD_V1) and v3 group-sorted mma.sync
-    (default) -- each against the oracle."""
+    (default) -- each against the oracle. At D = 64 and 128 the default is the per-corner kernel as well."""
     from weed_instance_segmentation_b200 import functional as F
     from weed_instance_segmentation_b200.synth import msda_inputs
     tag, B, shapes, H, D, P, Q = case
@@ -258,6 +265,24 @@ def test_error_behaviour(wis):
         wis.ms_deform_attn(v.half(), [(4, 4)], None, loc, attn)
     with pytest.raises(wis.MSDAError):  # head dim without a kernel: reported by the library, not swallowed
         wis.ms_deform_attn(torch.zeros(1, 16, 8, 24, device="cuda"), [(4, 4)], None, loc, attn)
+
+
+def test_refused_backward_does_not_fail_the_next_calls(wis):
+    """bf16 values with D = 8 take L*P <= 32 in the backward (shared memory; include/msda_b200.h), while the forward
+    takes 64: at L*P = 33 the forward runs and the backward is refused as unsupported. The refusal is an argument
+    error and must not resurface as an error of the next, valid, forward and backward on the same thread."""
+    from weed_instance_segmentation_b200.synth import msda_inputs
+    shapes = [(4, 4), (2, 3), (3, 2)]
+    x = msda_inputs(1, shapes, num_heads=2, head_dim=8, num_points=11, dist="init", seed=3, num_queries=10,
+                    value_dtype=torch.bfloat16)
+    v = x["value"].cuda().requires_grad_(True)
+    out = wis.ms_deform_attn(v, shapes, None, x["sampling_locations"].cuda(), x["attention_weights"].cuda())
+    with pytest.raises(RuntimeError, match="shared memory") as refused:
+        out.backward(x["grad_out"].cuda().reshape(out.shape))
+    x = msda_inputs(1, [(6, 6), (12, 12)], num_heads=4, head_dim=8, num_points=4, dist="init", seed=3)
+    args = (x["value"], [(6, 6), (12, 12)], x["sampling_locations"], x["attention_weights"], x["grad_out"])
+    _assert_close(_run(wis, *args), _oracle(*args, dtype=np.float32), FP32_BAR, "after a refused backward")
+    assert "error 2" in str(refused.value) and "227 KB" in str(refused.value)
 
 
 def test_nan_and_far_locations_are_safe(wis):

@@ -106,6 +106,8 @@ extern "C" int msda_b200_host_pipeline_create(const msda_b200_desc* desc, int32_
   // The library's own descriptor checks FIRST (L <= MSDA_B200_MAX_LEVELS, positive sizes, level table inside S):
   // only a validated descriptor says how many entries of the caller's arrays may be read.
   if (int rc = msda_b200_internal_validate(desc)) return rc;  // last_error set by validate
+  if (with_backward)
+    if (int rc = msda_b200_internal_check_backward(desc)) return rc;
   msda_b200_host_pipeline* p = new (std::nothrow) msda_b200_host_pipeline();
   if (!p) return msda_b200_internal_fail(MSDA_B200_ERR_INVALID, "host_pipeline_create: out of host memory");
   p->desc = *desc;

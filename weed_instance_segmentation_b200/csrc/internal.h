@@ -12,6 +12,8 @@ extern "C" {
 int msda_b200_internal_fail(int code, const char* msg);
 // msda_b200.cu: the descriptor checks of forward / backward
 int msda_b200_internal_validate(const msda_b200_desc* desc);
+// msda_b200.cu: the geometry limit of msda_b200_backward (shared memory per block) for a validated descriptor
+int msda_b200_internal_check_backward(const msda_b200_desc* desc);
 // msda_b200.cu: one more launch for msda_b200_launch_count()
 void msda_b200_internal_count_launch(void);
 

@@ -740,9 +740,14 @@ constexpr int kKeepCarveout = INT_MIN;
 template <typename... KA, typename... A>
 int launch(const msda_b200_desc* d, int prof, const char* what, void (*kern)(KA...), long long blocks, int threads,
            size_t smem, bool opt_in, int carveout, cudaStream_t st, A... args) {
-  if ((opt_in || smem > 48 * 1024) &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-    return fail(MSDA_B200_ERR_CUDA, "%s: cannot reserve %zu bytes of shared memory", what, smem);
+  if (opt_in || smem > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) {
+      char msg[128];
+      snprintf(msg, sizeof(msg), "%s: cannot reserve %zu bytes of shared memory", what, smem);
+      return cuda_error(msg, e);
+    }
+  }
   if (carveout != kKeepCarveout) cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
   if (blocks > 0x7fffffffll) return fail(MSDA_B200_ERR_UNSUPPORTED, "%s: grid too large", what);
   {
@@ -755,6 +760,30 @@ int launch(const msda_b200_desc* d, int prof, const char* what, void (*kern)(KA.
 // Launch geometry: NT threads per block, QPG queries per lane group.
 constexpr int kFwdNT = 128, kFwdQPG = 1;  // measured on config 2: 0.332 ms (256/1: 0.347, 256/2: 0.332, 512/1: 0.410)
 constexpr int kBwdNT = 128, kBwdQPG = 1;
+constexpr size_t kMaxBlockSmem = 227 * 1024;  // opt-in dynamic shared memory per block on sm_100
+
+// Dynamic shared memory of msda_bwd_kernel (the per-corner backward) for a validated descriptor and lp = L*P samples
+// per (query, head). It grows with L*P and with the queries per block (128 / LPP), so small head dims reach
+// kMaxBlockSmem below L*P = 64.
+size_t bwd_smem(const msda_b200_desc* d, int lp, bool fused) {
+  const size_t lpp = (size_t)d->D * dtype_size(d->value_dtype) / 16, tq = kBwdNT / lpp * kBwdQPG, row = tq + 1;
+  return lp * row * (2 * sizeof(float4) + sizeof(float) + sizeof(int)) + lp * tq * lpp * sizeof(float4) +
+         (fused ? 2 * tq * lp * sizeof(float) : 0);
+}
+
+// The backward's geometry limit, checked before any CUDA call (a launch past it fails in cudaFuncSetAttribute). The
+// group-sorted kernel's shared memory is fixed (mma_smem_layout, about 65 KB), so the per-corner kernel's is the bound
+// that can refuse a geometry.
+int check_backward_smem(const msda_b200_desc* d, bool fused) {
+  const int lp = d->L * d->P;
+  if (bwd_smem(d, lp, fused) <= kMaxBlockSmem) return MSDA_B200_OK;
+  int max_lp = lp - 1;
+  while (max_lp > 0 && bwd_smem(d, max_lp, fused) > kMaxBlockSmem) --max_lp;
+  return fail(MSDA_B200_ERR_UNSUPPORTED,
+              "%s: L*P=%d needs %zu bytes of shared memory per block with D=%d %s values, over the 227 KB limit "
+              "(at most L*P=%d here)", fused ? "backward_fused" : "backward", lp, bwd_smem(d, lp, fused), d->D,
+              d->value_dtype == MSDA_B200_BF16 ? "bf16" : "fp32", max_lp);
+}
 
 template <typename VT, typename AT, int D, bool FUSED>
 int launch_fwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
@@ -795,12 +824,8 @@ int launch_bwd(const msda_b200_desc* d, KParams p, cudaStream_t st) {
   constexpr int LPP = D / Vec16<VT>::N;
   using T = Tile<kBwdNT, LPP, kBwdQPG>;
   fill_geometry(d, p, T::TQ);
-  const size_t n = (size_t)p.LP * T::ROW;
-  const size_t smem = n * (2 * sizeof(float4) + sizeof(float) + sizeof(int)) +
-                      (size_t)p.LP * T::TQ * LPP * sizeof(float4) +
-                      (FUSED ? 2 * (size_t)T::TQ * p.LP * sizeof(float) : 0);
   return launch(d, MSDA_B200_PROF_BWD_MAIN, "backward", msda_bwd_kernel<VT, AT, D, kBwdNT, kBwdQPG, ACC, FUSED>,
-                (long long)p.B * p.num_tiles * p.H, kBwdNT, smem, false, kKeepCarveout, st, p);
+                (long long)p.B * p.num_tiles * p.H, kBwdNT, bwd_smem(d, p.LP, FUSED), false, kKeepCarveout, st, p);
 }
 
 template <typename VT, typename AT, bool FUSED>
@@ -873,8 +898,9 @@ int run_forward(const msda_b200_desc* desc, const KParams& p, cudaStream_t st) {
 }
 
 // The backward's argument checks, in this order, for a validated descriptor with B > 0. *need: the workspace bytes.
-int check_backward(const msda_b200_desc* d, const void* grad_value, const void* workspace, size_t workspace_bytes,
-                   bool have_tensors, size_t* need) {
+int check_backward(const msda_b200_desc* d, bool fused, const void* grad_value, const void* workspace,
+                   size_t workspace_bytes, bool have_tensors, size_t* need) {
+  if (int rc = check_backward_smem(d, fused)) return rc;
   if (!grad_value) return fail(MSDA_B200_ERR_INVALID, "backward: grad_value is NULL");
   if (!(d->flags & MSDA_B200_FLAG_DETERMINISTIC)) *need = msda_b200_backward_workspace_bytes(d);
   else if (int rc = msda_b200_internal_det_workspace_bytes(d, need)) return rc;
@@ -914,7 +940,7 @@ int run_backward(const msda_b200_desc* desc, KParams p, void* grad_value, void* 
                  bool have_tensors, cudaStream_t st) {
   if (desc->B == 0) return MSDA_B200_OK;  // validate() makes S >= 1, so only an empty batch has no grad_value
   size_t need = 0;
-  if (int rc = check_backward(desc, grad_value, workspace, workspace_bytes, have_tensors, &need)) return rc;
+  if (int rc = check_backward(desc, FUSED, grad_value, workspace, workspace_bytes, have_tensors, &need)) return rc;
   if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC) return run_backward_det<FUSED>(desc, p, grad_value, workspace, st);
 
   // Zero-fill the accumulator (and grad_value): the scatter only touches sampled pixels.
@@ -948,6 +974,7 @@ extern "C" {
 // declared in internal.h for the library's other files
 int msda_b200_internal_fail(int code, const char* msg) { return fail(code, "%s", msg); }
 int msda_b200_internal_validate(const msda_b200_desc* desc) { return validate(desc); }
+int msda_b200_internal_check_backward(const msda_b200_desc* desc) { return check_backward_smem(desc, false); }
 void msda_b200_internal_count_launch(void) { ++g_launches; }
 
 int msda_b200_abi_version(void) { return MSDA_B200_ABI_VERSION; }
@@ -984,9 +1011,11 @@ size_t msda_b200_backward_workspace_bytes(const msda_b200_desc* desc) {
   if (!desc) return 0;
   if (desc->flags & MSDA_B200_FLAG_DETERMINISTIC) {
     size_t bytes = 0;
-    if (validate(desc) || msda_b200_internal_det_workspace_bytes(desc, &bytes)) return 0;
+    if (validate(desc) || check_backward_smem(desc, false) || msda_b200_internal_det_workspace_bytes(desc, &bytes))
+      return 0;
     return bytes;
   }
+  if (validate(desc) == MSDA_B200_OK && check_backward_smem(desc, false)) return 0;
   if (desc->value_dtype == MSDA_B200_BF16)
     return (size_t)desc->B * desc->S * desc->H * desc->D * sizeof(float);
   return 0;

@@ -214,6 +214,10 @@ __global__ void __launch_bounds__(NT, 4) msda_bwd_mma_kernel(const __grid_consta
   // (In shared memory they cost 1.5 KB per block, which took the fused kernel from 4 to 3 blocks per SM.)
   static_assert(!FUSED || P == 4, "fused prologue: four lanes per (query, head) row");
   float f_lse[SPT], f_dsum[SPT];
+  // d(loss)/d(a) of the thread's samples, kept in fp32 until the softmax backward after the last level: parked in a
+  // bf16 grad_logits it would carry a 2^-9 rounding into ga - f_dsum, which cancels when the row's ga share a common
+  // part (value rows with a non-zero mean, one dominant logit). Local memory, indexed by the runtime level.
+  float ga_park[SPT][MSDA_B200_MAX_LEVELS];
 #pragma unroll
   for (int r = 0; r < SPT; ++r) { f_lse[r] = 0.f; f_dsum[r] = 0.f; }
   if (FUSED) {
@@ -592,10 +596,8 @@ __global__ void __launch_bounds__(NT, 4) msda_bwd_mma_kernel(const __grid_consta
           reinterpret_cast<float2*>(p.grad_loc)[gi] = make_float2((float)lv.W * a * g_px, (float)lv.H * a * g_py);
         }
       } else {
-        if (valid) {
-          store_pair<AT>(p.grad_offsets, gi, a * g_px, a * g_py);
-          reinterpret_cast<AT*>(p.grad_logits)[gi] = from_float<AT>(g_attn);  // parked; finished after the last level
-        }
+        if (valid) store_pair<AT>(p.grad_offsets, gi, a * g_px, a * g_py);
+        ga_park[r][l] = g_attn;  // finished after the last level
         float t = valid ? a * g_attn : 0.f;  // the P samples of one (query, level) sit in P adjacent lanes
 #pragma unroll
         for (int o = 1; o < P; o <<= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
@@ -606,8 +608,7 @@ __global__ void __launch_bounds__(NT, 4) msda_bwd_mma_kernel(const __grid_consta
 
   if (FUSED) {
     // softmax backward over the L*P logits of each (query, head): g_j = a_j * (ga_j - sum_k a_k ga_k).  Lane pt of the
-    // row's four lanes finishes the logits (l, pt) of every level l -- exactly the ones it parked itself in phase h, so
-    // no barrier is needed.
+    // row's four lanes finishes the logits (l, pt) of every level l -- exactly the ones it parked itself in phase h.
 #pragma unroll
     for (int r = 0; r < SPT; ++r) {
       const int ql = (r * NT + tid) >> LP2, pt = tid & (P - 1);
@@ -617,8 +618,7 @@ __global__ void __launch_bounds__(NT, 4) msda_bwd_mma_kernel(const __grid_consta
         for (int l = 0; l < p.L; ++l) {
           const long long gi = row + l * P + pt;
           const float a = expf(to_float<AT>(reinterpret_cast<const AT*>(p.logits)[gi]) - f_lse[r]);
-          const float ga = to_float<AT>(reinterpret_cast<const AT*>(p.grad_logits)[gi]);
-          reinterpret_cast<AT*>(p.grad_logits)[gi] = from_float<AT>(a * (ga - f_dsum[r]));
+          reinterpret_cast<AT*>(p.grad_logits)[gi] = from_float<AT>(a * (ga_park[r][l] - f_dsum[r]));
         }
       }
     }
